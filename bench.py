@@ -3,6 +3,13 @@
 
     python bench.py --gpus N --steps K --warmup W            (N > 1: launched by torch.distributed.run)
     python bench.py --impl reference --gpus N --steps K --warmup W
+    python bench.py --gpus N --steps K --warmup W --dump-outputs DIR
+
+--dump-outputs DIR writes what the last timed step computed -- final, filled and d8, in the dtypes a caller of
+ConditioningChain receives them (float64 final, float32 filled, d8 widened to float32) -- as DIR/<name>.npy: the whole
+rasters when they have at most DUMP_CELLS cells, else the cells at a fixed, seeded sample of positions (ascending
+row-major order, the same at every N).  The inputs are a pure function of the seed, so two builds run with the same
+arguments can be compared output for output.
 
 Workload (BASELINE.json configs[4], the one both north-star targets are quoted on): the full conditioning chain --
 Fourier stripe removal, groves correction x3, lagoon detection, recombination, 3x3 mean + round, sink-fill + D8 --
@@ -43,6 +50,7 @@ MOSAIC = 36000
 SEED = 1005
 METRIC = "Mcells/s, full conditioning chain"
 UNIT = "Mcells/s"
+DUMP_CELLS = 1 << 21            # cells per dumped output: 8 + 4 + 4 bytes each, 32 MB for the three outputs
 
 
 def algo_bytes_per_cell(odd):
@@ -173,18 +181,14 @@ def run_reference(args):
     if env_int("RANK", 0) != 0:
         return
     import multiprocessing as mp
-    from oracle import clib
-    clib.build()
     cores = len(os.sched_getaffinity(0)) or 1          # the cores this process may actually use
     size = args.cpu_sample
     ctx = mp.get_context("fork")
     with ctx.Pool(cores) as pool:
         pool.map(_cpu_worker, [(256, SEED + i) for i in range(cores)])          # warm-up (imports, page faults)
-        t_one = time.perf_counter()
-        pool.map(_cpu_worker, [(size, SEED + i) for i in range(cores)])
-        t_one = time.perf_counter() - t_one
-        # bounded: the whole run stays within a few minutes whatever --steps says
-        steps = max(1, min(args.steps, int(150.0 / max(t_one, 1e-3))))
+        for _ in range(args.warmup):
+            pool.map(_cpu_worker, [(size, SEED + i) for i in range(cores)])
+        steps = args.steps
         t0 = time.perf_counter()
         for _ in range(steps):
             pool.map(_cpu_worker, [(size, SEED + i) for i in range(cores)])     # one sample tile per core per step
@@ -268,6 +272,22 @@ def run_gpu(args):
             s1 += int((blk * wgt).sum().item())
         return s0, s1
 
+    def dumped_outputs(res, row0):
+        """final / filled / d8 of one step as --dump-outputs writes them (module docstring), gathered from all ranks."""
+        whole = cells <= DUMP_CELLS
+        idx = np.arange(cells) if whole else np.unique(np.random.default_rng(SEED).integers(0, cells, DUMP_CELLS))
+        out = {}
+        for name in ("final", "filled", "d8"):
+            t = res[name].tensor()
+            lo, hi = np.searchsorted(idx, [row0 * nx, (row0 + t.shape[0]) * nx])     # this rank's rows
+            mine = torch.from_numpy(idx[lo:hi] - row0 * nx).to(t.device)
+            vals = t[mine // nx, mine % nx].cpu().numpy()
+            if world > 1:
+                vals = np.concatenate(band.comm.gather_objects(vals))                 # bands in rank order
+            vals = vals.astype(np.float64 if res[name].ref_dtype == np.float64 else np.float32)
+            out[name] = vals.reshape(ny, nx) if whole else vals
+        return out
+
     # ---- the mosaic: generated on the device, straight into the rasters the chain reads ---------------------------
     mosaic = DeviceMosaic(ny, nx, SEED)
     chain = ConditioningChain()
@@ -322,6 +342,13 @@ def run_gpu(args):
     for name in ("final", "filled", "d8"):
         sums += list(checksums(res[name], r0))
     sums = sum_over_ranks(sums)
+    if args.dump_outputs:
+        dumped = dumped_outputs(res, r0)
+        if rank == 0:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, a in dumped.items():
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
+        del dumped
     fill_rounds = band.fill_rounds if band is not None else None
     fill_status = max_over_ranks(float(band.fill_status())) if band is not None else None
 
@@ -479,8 +506,6 @@ def run_gpu(args):
             "secondary": secondary,
         }
         if world == 1 and not args.no_cpu_baseline:
-            from oracle import clib
-            clib.build()
             dt = cpu_chain_sample(args.cpu_sample, SEED)
             line["cpu_baseline"] = {"value": args.cpu_sample ** 2 / dt / 1e6, "unit": UNIT, "cores": 1, "kind": "port",
                                     "seconds": dt,
@@ -503,7 +528,13 @@ def main():
     ap.add_argument("--e2e-steps", type=int, default=3)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-secondary", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write final / filled / d8 of the last timed step to DIR/<name>.npy (GPU path only)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU path; the reference arm times sample tiles")
     if args.impl == "reference":
         run_reference(args)
     else:
