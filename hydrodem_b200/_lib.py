@@ -66,6 +66,7 @@ SIGNATURES = {
     "hd_fft2_masked_inverse_abs": (_i, [_p, _p, _i64, _p, _i64, _p, _i, _i64, _p, _i64, _p]),
     "hd_fft2_c2c": (_i, [_p, _p, _i, _i64, _p, _i64, _i, _p, _i64, _p]),
     "hd_fft_rows": (_i, [_p, _p, _i, _i64, _p, _i64, _i64, _i, _i, _p, _i64, _p]),
+    "hd_fft_band_workspace_bytes": (_i64, [_i64, _i64]),
     "hd_fft_band_pass": (_i, [_p, _i, _i, _p, _i64, _i64, _p, _i64, _i, _i, _i, _p, _i64, _i64, _p, _i64, _p]),
     "hd_fft_band_pass_scatter": (_i, [_p, _i, _i, _p, _i64, _i64, _p, _i64, _i, _i, _i, _p, _i64, _p, _i64, _p]),
     "hd_ipc_export": (_i, [_p, _p, ctypes.POINTER(_i64)]),

@@ -31,10 +31,12 @@ void hd_count_launch(int n = 1);
 void hd_prof_begin(const char* name, cudaStream_t stream);
 
 // Host: encode a 2-D tiled tensor map over a pitched row-major raster.
-// elem: HD_F32 / HD_F64 / HD_U8 / HD_C64 (as 2xf32 -> encoded as f32 with doubled width is NOT done; c64 unsupported here)
+// dtype: HD_U8 / HD_F32 / HD_F64 / HD_I32, or HD_C64 (encoded as 64-bit integers: the bits are moved, no NaN fill).
+// swizzle128: CU_TENSOR_MAP_SWIZZLE_128B (box rows of at most 128 bytes; the shared-memory destination then wants
+// 1024-byte alignment).
 // Returns HD_OK or an error code (HD_ERR_ALIGN when base / pitch break the 16-byte TMA rules).
 int hd_make_tmap_2d(CUtensorMap* out, const void* base, int dtype, int64_t ny, int64_t nx, int64_t pitch_elems,
-                    int box_w, int box_h, bool nan_fill);
+                    int box_w, int box_h, bool nan_fill, bool swizzle128 = false);
 
 int hd_num_sms();          // SMs persistent grids are sized for (HD_SM_RESERVE leaves some to communication kernels)
 int hd_num_sms_total();

@@ -883,90 +883,145 @@ __device__ __forceinline__ int unpermute(int c, const RowPerm& pm)
     return k1 + pm.n1 * k2;
 }
 
-template <typename T, bool WITH_ABS>
-__global__ void __launch_bounds__(256) transpose_kernel(const T* __restrict__ in, int64_t in_pitch, T* __restrict__ out,
-                                                        int64_t out_pitch, float* __restrict__ out_abs, int64_t abs_pitch,
-                                                        int rows, int cols, int shift_r, int shift_c, RowPerm pm,
-                                                        int keep_max = -1, int mirror_rows = 0, int mirror_cols = 1)
+// One TMA-pipelined kernel serves every transpose of the 2-D transform.  A tile is 64 input rows x 256 bytes of input
+// columns (32 complex64 or 64 float), loaded as two 128-byte-wide boxes with the 128-byte swizzle: element (r, c) of a
+// box sits at r * 128 + ((16-byte chunk of c) ^ (r & 7)) * 16, so the 16-byte reads of eight consecutive rows in one
+// column group hit eight different chunks -- a tile column is read without bank conflicts.  A persistent grid walks
+// the tiles through a TR_STAGES-deep ring: the loads of the next TR_STAGES - 1 tiles are in flight while a tile is
+// stored.  What depends only on a tile column (un-permuting the row pass's storage order, the keep_max skip, the
+// shifted output row, the Hermitian mirror row) is computed once per tile into a shared table, so the store phase
+// does no division and no table load per element.  Stores: a warp writes 32 consecutive output columns of one
+// output row (256 bytes of complex64).
+//   in[r][c] lands at out[(kc + shift_c) % cols][(r + shift_r) % full_rows], kc = unpermute(c); out may be null.
+//   WITH_ABS: |in[r][c]| (hypotf) also lands at the same place of out_abs.
+//   keep_max >= 0: only input columns whose (unpermuted) index is <= keep_max are written (half spectrum of a real
+//                  transform).
+//   mirror_rows > 0: the input holds rows 0 .. rows-1 of a Hermitian spectrum whose full height is mirror_rows
+//                  (X[mirror_rows - r][cols - c] = conj X[r][c]); the missing rows are written from their mirror.
+//                  mirror_cols = 0: the symmetry is X[mirror_rows - r][c] = conj X[r][c] (second axis already real-space).
+//                  full_rows = mirror_rows, otherwise rows.
+//   OutT != T (float -> double only): the value is widened on the way out.
+constexpr int TR_ROWS = 64;              // input rows per tile = output columns per tile
+constexpr int TR_SWZ = 128;              // bytes per swizzled box row
+constexpr int TR_BOX_BYTES = TR_ROWS * TR_SWZ;
+constexpr int TR_STAGE_BYTES = 2 * TR_BOX_BYTES;
+constexpr int TR_STAGES = 4;
+constexpr int TR_THREADS = 256;
+constexpr int TR_SMEM = TR_STAGES * TR_STAGE_BYTES + 1024;     // + alignment slack: the swizzle wants 1024-byte stages
+
+struct TransArgs {
+    void* out;               // OutT, may be null (then only out_abs is written)
+    int64_t out_pitch;
+    float* out_abs;          // WITH_ABS only
+    int64_t abs_pitch;
+    int rows, cols;          // input extent
+    int tile_cols;           // input columns that can hold written values (cols, or keep_max + 1 when nothing is permuted)
+    int shift_r, shift_c;
+    RowPerm pm;
+    int keep_max, mirror_rows, mirror_cols;
+};
+
+template <typename T, typename OutT, bool WITH_ABS>
+__global__ void __launch_bounds__(TR_THREADS) transpose_tma_kernel(const __grid_constant__ CUtensorMap tm, TransArgs a)
 {
-    // keep_max >= 0: only input columns whose (unpermuted) index is <= keep_max are written (half spectrum of a real
-    //                transform).
-    // mirror_rows > 0: the input holds rows 0 .. rows-1 of a Hermitian spectrum whose full height is mirror_rows
-    //                (X[mirror_rows - r][cols - c] = conj X[r][c]); the missing rows are written from their mirror.
-    //                mirror_cols = 0: the symmetry is X[mirror_rows - r][c] = conj X[r][c] (second axis already real-space).
-    __shared__ T tile[32][33];
-    const int tiles_c = (cols + 31) / 32, tiles_r = (rows + 31) / 32;
-    const int ntiles = tiles_c * tiles_r;
-    const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;       // 32 x 8
-    for (int t = blockIdx.x; t < ntiles; t += gridDim.x) {
-        const int r0 = (t / tiles_c) * 32, c0 = (t % tiles_c) * 32;
+    constexpr int ES = (int)sizeof(T);
+    constexpr int BOXW = TR_SWZ / ES;            // elements per box row
+    constexpr int TC = 2 * BOXW;                 // tile columns
+    constexpr int V = 16 / ES;                   // elements per 16-byte shared-memory read
+    constexpr int PER_THREAD = TR_ROWS * TC / V / TR_THREADS;
+    static_assert(PER_THREAD * TR_THREADS * V == TR_ROWS * TC, "tile / thread mismatch");
+    constexpr bool CPLX = sizeof(T) == 8;
+    extern __shared__ unsigned char smem_raw[];
+    __shared__ uint64_t full[TR_STAGES];
+    __shared__ int orow_t[2][TC], mrow_t[2][TC];
+    unsigned char* ring = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
+    const int tiles_c = (a.tile_cols + TC - 1) / TC;
+    const int ntiles = tiles_c * ((a.rows + TR_ROWS - 1) / TR_ROWS);
+    const int full_rows = a.mirror_rows > 0 ? a.mirror_rows : a.rows;
+    if (threadIdx.x == 0) {
 #pragma unroll
-        for (int k = 0; k < 4; ++k) {
-            const int r = r0 + ty + 8 * k, c = c0 + tx;
-            if (r < rows && c < cols) tile[ty + 8 * k][tx] = in[(int64_t)r * in_pitch + c];
+        for (int s = 0; s < TR_STAGES; ++s) mbar_init(&full[s], 1);
+        mbar_fence_init();
+        tma_prefetch_desc(&tm);
+    }
+    __syncthreads();
+    auto issue = [&](int tile, int s) {
+        const int r0 = (tile / tiles_c) * TR_ROWS, c0 = (tile % tiles_c) * TC;
+        unsigned char* dst = ring + s * TR_STAGE_BYTES;
+        mbar_arrive_expect_tx(&full[s], TR_STAGE_BYTES);      // out-of-range box cells are zero-filled and counted
+        tma_load_2d(dst, &tm, c0, r0, &full[s]);
+        tma_load_2d(dst + TR_BOX_BYTES, &tm, c0 + BOXW, r0, &full[s]);
+    };
+    if (threadIdx.x == 0) {
+#pragma unroll
+        for (int k = 0; k < TR_STAGES - 1; ++k) {
+            const int t = (int)blockIdx.x + k * (int)gridDim.x;
+            if (t < ntiles) issue(t, k);
         }
-        __syncthreads();
-#pragma unroll
-        for (int k = 0; k < 4; ++k) {
-            const int c = c0 + ty + 8 * k, r = r0 + tx;            // out row = c, out col = r
-            if (r < rows && c < cols) {
-                const int kc = unpermute(c, pm);
-                if (keep_max >= 0 && kc > keep_max) continue;
-                const int full_rows = mirror_rows > 0 ? mirror_rows : rows;     // extent of the output's column axis
-                int orow = kc + shift_c; if (orow >= cols) orow -= cols;
-                int ocol = r + shift_r; if (ocol >= full_rows) ocol -= full_rows;
-                const T v = tile[tx][ty + 8 * k];
-                if (out) out[(int64_t)orow * out_pitch + ocol] = v;
-                float mag = 0.f;
-                if (WITH_ABS) {
-                    const float2 z = *reinterpret_cast<const float2*>(&v);
-                    mag = hypotf(z.x, z.y);                                     // np.abs(complex64) -> float32
-                    out_abs[(int64_t)orow * abs_pitch + ocol] = mag;
+    }
+    int k = 0;
+    for (int tile = blockIdx.x; tile < ntiles; tile += gridDim.x, ++k) {
+        const int s = k % TR_STAGES;
+        const int r0 = (tile / tiles_c) * TR_ROWS, c0 = (tile % tiles_c) * TC;
+        int* orow_tab = orow_t[k & 1];
+        int* mrow_tab = mrow_t[k & 1];
+        if (threadIdx.x < TC) {                                 // tile-column table (read two tiles ago: free again)
+            const int c = c0 + (int)threadIdx.x;
+            int orow = -1, mrow = -1;
+            if (c < a.cols) {
+                const int kc = unpermute(c, a.pm);
+                if (a.keep_max < 0 || kc <= a.keep_max) {
+                    orow = kc + a.shift_c; if (orow >= a.cols) orow -= a.cols;
+                    mrow = (a.mirror_cols ? (kc ? a.cols - kc : 0) : kc) + a.shift_c; if (mrow >= a.cols) mrow -= a.cols;
                 }
-                if (mirror_rows > 0 && r > 0 && 2 * r != mirror_rows) {
-                    // conjugate partner: (r, kc) -> (mirror_rows - r, (cols - kc) % cols)
-                    int mrow = (mirror_cols ? (kc ? cols - kc : 0) : kc) + shift_c; if (mrow >= cols) mrow -= cols;
-                    int mcol = (mirror_rows - r) + shift_r; if (mcol >= full_rows) mcol -= full_rows;
-                    if (out) {
-                        T cv = v;
-                        float2* pz = reinterpret_cast<float2*>(&cv);
-                        pz->y = -pz->y;
-                        out[(int64_t)mrow * out_pitch + mcol] = cv;
+            }
+            orow_tab[threadIdx.x] = orow;
+            mrow_tab[threadIdx.x] = mrow;
+        }
+        __syncthreads();                                        // table visible; every thread is done with tile k - 1
+        if (threadIdx.x == 0) {                                 // refill the stage tile k - 1 used
+            const int t = tile + (TR_STAGES - 1) * (int)gridDim.x;
+            if (t < ntiles) issue(t, (k + TR_STAGES - 1) % TR_STAGES);
+        }
+        mbar_wait(&full[s], (uint32_t)(k / TR_STAGES) & 1u);
+        const unsigned char* st = ring + s * TR_STAGE_BYTES;
+#pragma unroll
+        for (int j = 0; j < PER_THREAD; ++j) {
+            const int u = (int)threadIdx.x + j * TR_THREADS;
+            const int r = u & (TR_ROWS - 1), cg = u / TR_ROWS;  // a warp: 32 consecutive rows of one 16-byte column group
+            const int gr = r0 + r;
+            if (gr >= a.rows) continue;
+            const float4 raw = *reinterpret_cast<const float4*>(st + (cg >> 3) * TR_BOX_BYTES + r * TR_SWZ +
+                                                                (((cg & 7) ^ (r & 7)) << 4));
+            T vals[V];
+            memcpy(vals, &raw, sizeof raw);
+            int ocol = gr + a.shift_r; if (ocol >= full_rows) ocol -= full_rows;
+            const bool mirror = a.mirror_rows > 0 && gr > 0 && 2 * gr != a.mirror_rows;
+            int mcol = a.mirror_rows - gr + a.shift_r; if (mcol >= full_rows) mcol -= full_rows;
+#pragma unroll
+            for (int v = 0; v < V; ++v) {
+                const int orow = orow_tab[cg * V + v];
+                if (orow < 0) continue;
+                const T val = vals[v];
+                if (a.out) reinterpret_cast<OutT*>(a.out)[(int64_t)orow * a.out_pitch + ocol] = (OutT)val;
+                if constexpr (CPLX) {
+                    const float2 z = *reinterpret_cast<const float2*>(&val);
+                    float mag = 0.f;
+                    if constexpr (WITH_ABS) {
+                        mag = hypotf(z.x, z.y);                             // np.abs(complex64) -> float32
+                        a.out_abs[(int64_t)orow * a.abs_pitch + ocol] = mag;
                     }
-                    if (WITH_ABS) out_abs[(int64_t)mrow * abs_pitch + mcol] = mag;
+                    if (mirror) {                                           // conjugate partner
+                        const int mrow = mrow_tab[cg * V + v];
+                        if (a.out)
+                            reinterpret_cast<float2*>(a.out)[(int64_t)mrow * a.out_pitch + mcol] = make_float2(z.x, -z.y);
+                        if constexpr (WITH_ABS) a.out_abs[(int64_t)mrow * a.abs_pitch + mcol] = mag;
+                    }
                 }
             }
         }
-        __syncthreads();
     }
 }
-
-template <typename OutT>
-__global__ void __launch_bounds__(256) transpose_real_kernel(const float* __restrict__ in, int64_t in_pitch,
-                                                             OutT* __restrict__ out, int64_t out_pitch, int rows, int cols,
-                                                             RowPerm pm)
-{
-    __shared__ float tile[32][33];
-    const int tiles_c = (cols + 31) / 32, tiles_r = (rows + 31) / 32;
-    const int ntiles = tiles_c * tiles_r;
-    const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
-    for (int t = blockIdx.x; t < ntiles; t += gridDim.x) {
-        const int r0 = (t / tiles_c) * 32, c0 = (t % tiles_c) * 32;
-#pragma unroll
-        for (int k = 0; k < 4; ++k) {
-            const int r = r0 + ty + 8 * k, c = c0 + tx;
-            if (r < rows && c < cols) tile[ty + 8 * k][tx] = in[(int64_t)r * in_pitch + c];
-        }
-        __syncthreads();
-#pragma unroll
-        for (int k = 0; k < 4; ++k) {
-            const int c = c0 + ty + 8 * k, r = r0 + tx;
-            if (r < rows && c < cols) out[(int64_t)unpermute(c, pm) * out_pitch + r] = (OutT)tile[tx][ty + 8 * k];
-        }
-        __syncthreads();
-    }
-}
-
 
 // ---- transpose fused with the all-to-all: remote stores over NVLink --------------------------------------------------------
 // The sharded Fourier stage follows every row pass with "transpose, then send row range j of the result to rank j".
@@ -1177,6 +1232,44 @@ int transpose_grid(int rows, int cols)
     return (int)(nt < cap ? nt : cap);
 }
 
+// Row pitch (elements) of the scratch arrays the transposes read: TMA wants 16-byte-aligned rows.
+int64_t pitch_c64(int64_t n) { return (n + 1) & ~(int64_t)1; }
+int64_t pitch_f32(int64_t n) { return (n + 3) & ~(int64_t)3; }
+
+// in: (rows x cols) T with a 16-byte-aligned base and pitch (the scratch arrays of this file); name: profiler record
+template <typename T, typename OutT, bool WITH_ABS>
+int launch_transpose(const T* in, int64_t in_pitch, TransArgs a, cudaStream_t s, const char* name)
+{
+    constexpr int TC = 2 * TR_SWZ / (int)sizeof(T);
+    if (a.rows < 1 || a.cols < 1) return HD_OK;
+    // a half-spectrum consumer of rows in natural order only needs the columns up to keep_max
+    a.tile_cols = (a.keep_max >= 0 && a.pm.n1 == 1 && !a.pm.ipos) ? std::min(a.cols, a.keep_max + 1) : a.cols;
+    CUtensorMap tm;
+    if (int e = hd_make_tmap_2d(&tm, in, sizeof(T) == 8 ? HD_C64 : HD_F32, a.rows, a.cols, in_pitch, TR_SWZ / (int)sizeof(T),
+                                TR_ROWS, false, true))
+        return e;
+    auto kern = transpose_tma_kernel<T, OutT, WITH_ABS>;
+    HD_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, TR_SMEM));
+    int per_sm = 1;
+    HD_CUDA_OK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, TR_THREADS, TR_SMEM));
+    const int64_t ntiles = (int64_t)hd_cdiv(a.tile_cols, TC) * hd_cdiv(a.rows, TR_ROWS);
+    const int64_t cap = (int64_t)hd_num_sms() * (per_sm < 1 ? 1 : per_sm);
+    hd_prof_begin(name, s);
+    kern<<<(unsigned)(ntiles < cap ? ntiles : cap), TR_THREADS, TR_SMEM, s>>>(tm, a);
+    HD_LAUNCH_CHECK(); hd_count_launch();
+    return HD_OK;
+}
+
+TransArgs trans_args(void* out, int64_t out_pitch, int rows, int cols, RowPerm pm)
+{
+    TransArgs a{};
+    a.out = out; a.out_pitch = out_pitch;
+    a.rows = rows; a.cols = cols;
+    a.pm = pm;
+    a.keep_max = -1; a.mirror_rows = 0; a.mirror_cols = 1;
+    return a;
+}
+
 }  // namespace
 
 extern "C" {
@@ -1204,8 +1297,10 @@ int hd_fft2_plan_destroy(void* plan)
     return HD_OK;
 }
 
-// two complex64 scratch arrays of ny * nx
-int64_t hd_fft2_workspace_bytes(int64_t ny, int64_t nx) { return 2 * ny * nx * (int64_t)sizeof(float2); }
+// two complex64 scratch arrays of ny x nx, each with room for 16-byte-aligned row pitches in either orientation
+int64_t hd_fft2_workspace_bytes(int64_t ny, int64_t nx) { return 2 * pitch_c64(ny) * pitch_c64(nx) * (int64_t)sizeof(float2); }
+
+int64_t hd_fft_band_workspace_bytes(int64_t nrows, int64_t n) { return nrows * pitch_c64(n) * (int64_t)sizeof(float2); }
 
 int hd_fft2_forward_shift_abs(void* plan, const void* in, int64_t in_pitch, void* fshift, int64_t fshift_pitch, void* fabs_out,
                               int64_t fabs_pitch, void* workspace, int64_t workspace_bytes, void* stream)
@@ -1216,27 +1311,26 @@ int hd_fft2_forward_shift_abs(void* plan, const void* in, int64_t in_pitch, void
     if (workspace_bytes < hd_fft2_workspace_bytes(ny, nx)) return HD_ERR_WORKSPACE;
     if (in_pitch < nx || fabs_pitch < nx || (fshift && fshift_pitch < nx)) return HD_ERR_ARG;
     cudaStream_t s = (cudaStream_t)stream;
-    float2* A = (float2*)workspace;                 // [ny][nx]
-    float2* At = A + (int64_t)ny * nx;              // [nx][ny]
+    const int64_t pnx = pitch_c64(nx), pny = pitch_c64(ny);
+    float2* A = (float2*)workspace;                 // [ny][pnx]
+    float2* At = A + pny * pnx;                     // [nx][pny]
     // The input is real, so the spectrum is Hermitian: only columns kx = 0 .. nx/2 go through the second (column) pass,
     // the other half is written from its conjugate mirror by the last transpose.
     const int nh = nx / 2 + 1;
-    RowsArgs r1{in, in_pitch, A, nx, nullptr, 0, ny, 0, 0, 0, 0};
+    RowsArgs r1{in, in_pitch, A, pnx, nullptr, 0, ny, 0, 0, 0, 0};
     if (int e = launch_rows(p->px, r1, LOAD_REAL, s)) return e;
-    hd_prof_begin("transpose_kernel", s);
-    transpose_kernel<float2, false><<<transpose_grid(ny, nx), 256, 0, s>>>(A, nx, At, ny, nullptr, 0, ny, nx, 0, 0,
-                                                                          perm_of(p->px, LOAD_REAL), nh - 1, 0);
-    HD_LAUNCH_CHECK(); hd_count_launch();
-    RowsArgs r2{At, ny, A, ny, nullptr, 0, nh, 0, 0, 0, 0};              // out of place: long rows read the whole row
+    TransArgs t1 = trans_args(At, pny, ny, nx, perm_of(p->px, LOAD_REAL));
+    t1.keep_max = nh - 1;
+    if (int e = launch_transpose<float2, float2, false>(A, pnx, t1, s, "transpose_kernel")) return e;
+    RowsArgs r2{At, pny, A, pny, nullptr, 0, nh, 0, 0, 0, 0};            // out of place: long rows read the whole row
     if (int e = launch_rows(p->py, r2, LOAD_C64, s)) return e;
     // A[kx][ky] = F[ky][kx] for kx < nh; transpose back with fftshift folded in:
     // F[ky][kx] -> Fs[(ky + ny/2) % ny][(kx + nx/2) % nx], plus the mirrored half
-    hd_prof_begin("transpose_kernel", s);
-    transpose_kernel<float2, true><<<transpose_grid(nh, ny), 256, 0, s>>>(A, ny, (float2*)fshift, fshift_pitch,
-                                                                         (float*)fabs_out, fabs_pitch, nh, ny, nx / 2, ny / 2,
-                                                                         perm_of(p->py, LOAD_C64), -1, nx);
-    HD_LAUNCH_CHECK(); hd_count_launch();
-    return HD_OK;
+    TransArgs t2 = trans_args(fshift, fshift_pitch, nh, ny, perm_of(p->py, LOAD_C64));
+    t2.out_abs = (float*)fabs_out; t2.abs_pitch = fabs_pitch;
+    t2.shift_r = nx / 2; t2.shift_c = ny / 2;
+    t2.mirror_rows = nx;
+    return launch_transpose<float2, float2, true>(A, pny, t2, s, "transpose_kernel");
 }
 
 int hd_fft2_masked_inverse_abs(void* plan, const void* fshift, int64_t fshift_pitch, const void* mask, int64_t mask_pitch,
@@ -1250,10 +1344,11 @@ int hd_fft2_masked_inverse_abs(void* plan, const void* fshift, int64_t fshift_pi
     if (fshift_pitch < nx || mask_pitch < nx || out_pitch < nx) return HD_ERR_ARG;
     if (out_dtype != HD_F32 && out_dtype != HD_F64) return HD_ERR_UNSUPPORTED;
     cudaStream_t s = (cudaStream_t)stream;
-    float2* A = (float2*)workspace;
-    float2* At = A + (int64_t)ny * nx;
+    const int64_t pnx = pitch_c64(nx), pny = pitch_c64(ny), pny_f = pitch_f32(ny);
+    float2* A = (float2*)workspace;                 // [ny][pnx]
+    float2* At = A + pny * pnx;                     // [nx][pny]
     // ifftshift: unshifted index k reads shifted index (k + n/2) % n
-    float* absT = (float*)A;                        // [nx][ny] float, reuses A
+    float* absT = (float*)A;                        // [nx][pny_f] float, reuses A
     if ((ny & 1) && (nx & 1) && !getenv("HD_FFT_NO_HERMITIAN")) {
         // Odd x odd: the assembled mask is exactly point-symmetric about DC (custom_filters.py:1042-1049) and F is
         // the spectrum of a real raster, so (1 - mask) * F is Hermitian and the inverse is real.  Only rows
@@ -1261,32 +1356,25 @@ int hd_fft2_masked_inverse_abs(void* plan, const void* fshift, int64_t fshift_pi
         // (c[ny - ky][x] = conj c[ky][x]) written by the transpose; the second pass packs two real-output columns
         // into one complex transform.  abs() of a real number: |re| (the reference's imaginary part is rounding noise).
         const int nyh = ny / 2 + 1;
-        RowsArgs r1{fshift, fshift_pitch, A, nx, (const uint8_t*)mask, mask_pitch, nyh, ny / 2, nx / 2, 1, 0, ny};
+        RowsArgs r1{fshift, fshift_pitch, A, pnx, (const uint8_t*)mask, mask_pitch, nyh, ny / 2, nx / 2, 1, 0, ny};
         if (int e = launch_rows(p->px, r1, LOAD_MASKED_SHIFTED, s)) return e;
-        hd_prof_begin("transpose_kernel", s);
-        transpose_kernel<float2, false><<<transpose_grid(nyh, nx), 256, 0, s>>>(A, nx, At, ny, nullptr, 0, nyh, nx, 0, 0,
-                                                                               perm_of(p->px, LOAD_MASKED_SHIFTED), -1, ny, 0);
-        HD_LAUNCH_CHECK(); hd_count_launch();
-        RowsArgs r2{At, ny, (float2*)absT, ny, nullptr, 0, nx, 0, 0, 1, 1};
+        TransArgs t1 = trans_args(At, pny, nyh, nx, perm_of(p->px, LOAD_MASKED_SHIFTED));
+        t1.mirror_rows = ny; t1.mirror_cols = 0;
+        if (int e = launch_transpose<float2, float2, false>(A, pnx, t1, s, "transpose_kernel")) return e;
+        RowsArgs r2{At, pny, (float2*)absT, pny_f, nullptr, 0, nx, 0, 0, 1, 1};
         if (int e = launch_rows(p->py, r2, LOAD_C64_HPAIR, s)) return e;
     } else {
-        RowsArgs r1{fshift, fshift_pitch, A, nx, (const uint8_t*)mask, mask_pitch, ny, ny / 2, nx / 2, 1, 0};
+        RowsArgs r1{fshift, fshift_pitch, A, pnx, (const uint8_t*)mask, mask_pitch, ny, ny / 2, nx / 2, 1, 0};
         if (int e = launch_rows(p->px, r1, LOAD_MASKED_SHIFTED, s)) return e;
-        hd_prof_begin("transpose_kernel", s);
-        transpose_kernel<float2, false><<<transpose_grid(ny, nx), 256, 0, s>>>(A, nx, At, ny, nullptr, 0, ny, nx, 0, 0,
-                                                                              perm_of(p->px, LOAD_MASKED_SHIFTED));
-        HD_LAUNCH_CHECK(); hd_count_launch();
-        RowsArgs r2{At, ny, (float2*)absT, ny, nullptr, 0, nx, 0, 0, 1, 1};
+        const TransArgs t1 = trans_args(At, pny, ny, nx, perm_of(p->px, LOAD_MASKED_SHIFTED));
+        if (int e = launch_transpose<float2, float2, false>(A, pnx, t1, s, "transpose_kernel")) return e;
+        RowsArgs r2{At, pny, (float2*)absT, pny_f, nullptr, 0, nx, 0, 0, 1, 1};
         if (int e = launch_rows(p->py, r2, LOAD_C64, s)) return e;
     }
     const RowPerm pm2 = perm_of(p->py, ((ny & 1) && (nx & 1) && !getenv("HD_FFT_NO_HERMITIAN")) ? LOAD_C64_HPAIR : LOAD_C64);
-    hd_prof_begin("transpose_real_kernel", s);
-    if (out_dtype == HD_F32)
-        transpose_real_kernel<float><<<transpose_grid(nx, ny), 256, 0, s>>>(absT, ny, (float*)out, out_pitch, nx, ny, pm2);
-    else
-        transpose_real_kernel<double><<<transpose_grid(nx, ny), 256, 0, s>>>(absT, ny, (double*)out, out_pitch, nx, ny, pm2);
-    HD_LAUNCH_CHECK(); hd_count_launch();
-    return HD_OK;
+    const TransArgs t2 = trans_args(out, out_pitch, nx, ny, pm2);
+    if (out_dtype == HD_F32) return launch_transpose<float, float, false>(absT, pny_f, t2, s, "transpose_real_kernel");
+    return launch_transpose<float, double, false>(absT, pny_f, t2, s, "transpose_real_kernel");
 }
 
 int hd_fft2_c2c(void* plan, const void* in, int in_dtype, int64_t in_pitch, void* out, int64_t out_pitch, int inverse,
@@ -1299,22 +1387,18 @@ int hd_fft2_c2c(void* plan, const void* in, int in_dtype, int64_t in_pitch, void
     if (in_pitch < nx || out_pitch < nx) return HD_ERR_ARG;
     if (in_dtype != HD_F32 && in_dtype != HD_C64) return HD_ERR_UNSUPPORTED;
     cudaStream_t s = (cudaStream_t)stream;
-    float2* A = (float2*)workspace;
-    float2* At = A + (int64_t)ny * nx;
-    RowsArgs r1{in, in_pitch, A, nx, nullptr, 0, ny, 0, 0, inverse ? 1 : 0, 0};
+    const int64_t pnx = pitch_c64(nx), pny = pitch_c64(ny);
+    float2* A = (float2*)workspace;                 // [ny][pnx], then [nx][pny]
+    float2* At = A + pny * pnx;                     // [nx][pny]
+    RowsArgs r1{in, in_pitch, A, pnx, nullptr, 0, ny, 0, 0, inverse ? 1 : 0, 0};
     const int load1 = in_dtype == HD_F32 ? LOAD_REAL : LOAD_C64;
     if (int e = launch_rows(p->px, r1, load1, s)) return e;
-    hd_prof_begin("transpose_kernel", s);
-    transpose_kernel<float2, false><<<transpose_grid(ny, nx), 256, 0, s>>>(A, nx, At, ny, nullptr, 0, ny, nx, 0, 0,
-                                                                          perm_of(p->px, load1));
-    HD_LAUNCH_CHECK(); hd_count_launch();
-    RowsArgs r2{At, ny, A, ny, nullptr, 0, nx, 0, 0, inverse ? 1 : 0, 0};
+    const TransArgs t1 = trans_args(At, pny, ny, nx, perm_of(p->px, load1));
+    if (int e = launch_transpose<float2, float2, false>(A, pnx, t1, s, "transpose_kernel")) return e;
+    RowsArgs r2{At, pny, A, pny, nullptr, 0, nx, 0, 0, inverse ? 1 : 0, 0};
     if (int e = launch_rows(p->py, r2, LOAD_C64, s)) return e;
-    hd_prof_begin("transpose_kernel", s);
-    transpose_kernel<float2, false><<<transpose_grid(nx, ny), 256, 0, s>>>(A, ny, (float2*)out, out_pitch, nullptr, 0, nx, ny,
-                                                                          0, 0, perm_of(p->py, LOAD_C64));
-    HD_LAUNCH_CHECK(); hd_count_launch();
-    return HD_OK;
+    const TransArgs t2 = trans_args(out, out_pitch, nx, ny, perm_of(p->py, LOAD_C64));
+    return launch_transpose<float2, float2, false>(A, pny, t2, s, "transpose_kernel");
 }
 
 // Batched 1-D transforms along the rows of an (nrows x nx) array (nx = the plan's row length): the building block of
@@ -1332,27 +1416,23 @@ int hd_fft_rows(void* plan, const void* in, int in_dtype, int64_t in_pitch, void
     if (in_pitch < nx || out_pitch < (transpose_out ? nrows : nx)) return HD_ERR_ARG;
     if (in_dtype != HD_F32 && in_dtype != HD_C64) return HD_ERR_UNSUPPORTED;
     cudaStream_t s = (cudaStream_t)stream;
-    float2* A = (float2*)workspace;
-    float2* At = A + nrows * nx;
+    const int64_t pnx = pitch_c64(nx), pnr = pitch_c64(nrows);
+    float2* A = (float2*)workspace;                 // [nrows][pnx]
+    float2* At = A + pnr * pnx;                     // [nx][pnr]
     const bool direct = !transpose_out && p->px.n1 == 1;
     // LOAD_REAL would pack two real rows per transform and emit both spectra: fine here (full spectra are stored)
-    RowsArgs r1{in, in_pitch, direct ? (float2*)out : A, direct ? out_pitch : (int64_t)nx, nullptr, 0, (int)nrows, 0, 0,
+    RowsArgs r1{in, in_pitch, direct ? (float2*)out : A, direct ? out_pitch : pnx, nullptr, 0, (int)nrows, 0, 0,
                 inverse ? 1 : 0, 0};
     const int load1 = in_dtype == HD_F32 ? LOAD_REAL : LOAD_C64;
     if (int e = launch_rows(p->px, r1, load1, s, !direct)) return e;
     if (direct) return HD_OK;
-    float2* t_out = transpose_out ? (float2*)out : At;
-    const int64_t t_pitch = transpose_out ? out_pitch : nrows;
-    hd_prof_begin("transpose_kernel", s);
-    transpose_kernel<float2, false><<<transpose_grid((int)nrows, nx), 256, 0, s>>>(A, nx, t_out, t_pitch, nullptr, 0,
-                                                                                  (int)nrows, nx, 0, 0, perm_of(p->px, load1));
-    HD_LAUNCH_CHECK(); hd_count_launch();
+    const TransArgs t1 = trans_args(transpose_out ? out : (void*)At, transpose_out ? out_pitch : pnr, (int)nrows, nx,
+                                    perm_of(p->px, load1));
+    if (int e = launch_transpose<float2, float2, false>(A, pnx, t1, s, "transpose_kernel")) return e;
     if (transpose_out) return HD_OK;
-    hd_prof_begin("transpose_kernel", s);                         // long rows, row layout wanted: transpose back
-    transpose_kernel<float2, false><<<transpose_grid(nx, (int)nrows), 256, 0, s>>>(At, nrows, (float2*)out, out_pitch, nullptr,
-                                                                                  0, nx, (int)nrows, 0, 0, RowPerm{1, nx, nullptr});
-    HD_LAUNCH_CHECK(); hd_count_launch();
-    return HD_OK;
+    // long rows, row layout wanted: transpose back
+    const TransArgs t2 = trans_args(out, out_pitch, nx, (int)nrows, RowPerm{1, nx, nullptr});
+    return launch_transpose<float2, float2, false>(At, pnr, t2, s, "transpose_kernel");
 }
 
 
@@ -1372,25 +1452,18 @@ int hd_fft_band_pass(void* plan, int axis, int load, const void* in, int64_t in_
     if (nrows < 1 || nrows > 0x7fffffff || axis < 0 || axis > 1 || load < 0 || load > 3) return HD_ERR_ARG;
     if (load == LOAD_MASKED_SHIFTED && !mask) return HD_ERR_NULL;
     if (load == LOAD_C64_HPAIR && !real_out) return HD_ERR_ARG;
-    if (workspace_bytes < nrows * (int64_t)n * (int64_t)sizeof(float2)) return HD_ERR_WORKSPACE;
+    if (workspace_bytes < hd_fft_band_workspace_bytes(nrows, n)) return HD_ERR_WORKSPACE;
     if (in_pitch < n || out_t_pitch < nrows) return HD_ERR_ARG;
     cudaStream_t s = (cudaStream_t)stream;
-    float2* A = (float2*)workspace;
-    RowsArgs r{in, in_pitch, A, n, (const uint8_t*)mask, mask_pitch, (int)nrows, 0, shift_cols, inverse ? 1 : 0,
+    float2* A = (float2*)workspace;                 // [nrows][pitch] of complex64, or of float when real_out
+    const int64_t pitch = real_out ? pitch_f32(n) : pitch_c64(n);
+    RowsArgs r{in, in_pitch, A, pitch, (const uint8_t*)mask, mask_pitch, (int)nrows, 0, shift_cols, inverse ? 1 : 0,
                real_out ? 1 : 0, (int)nrows};
     if (int e = launch_rows(pl, r, load, s)) return e;
-    const RowPerm pm = perm_of(pl, load);
-    if (real_out) {
-        hd_prof_begin("transpose_real_kernel", s);
-        transpose_real_kernel<float><<<transpose_grid((int)nrows, n), 256, 0, s>>>((const float*)A, n, (float*)out_t, out_t_pitch,
-                                                                                  (int)nrows, n, pm);
-    } else {
-        hd_prof_begin("transpose_kernel", s);
-        transpose_kernel<float2, false><<<transpose_grid((int)nrows, n), 256, 0, s>>>(
-            A, n, (float2*)out_t, out_t_pitch, nullptr, 0, (int)nrows, n, 0, 0, pm, keep_cols > 0 ? (int)keep_cols - 1 : -1, 0);
-    }
-    HD_LAUNCH_CHECK(); hd_count_launch();
-    return HD_OK;
+    TransArgs t = trans_args(out_t, out_t_pitch, (int)nrows, n, perm_of(pl, load));
+    if (real_out) return launch_transpose<float, float, false>((const float*)A, pitch, t, s, "transpose_real_kernel");
+    t.keep_max = keep_cols > 0 ? (int)keep_cols - 1 : -1;
+    return launch_transpose<float2, float2, false>(A, pitch, t, s, "transpose_kernel");
 }
 
 

@@ -119,7 +119,7 @@ static PFN_encodeTiled get_encode()
 }
 
 int hd_make_tmap_2d(CUtensorMap* out, const void* base, int dtype, int64_t ny, int64_t nx, int64_t pitch_elems,
-                    int box_w, int box_h, bool nan_fill)
+                    int box_w, int box_h, bool nan_fill, bool swizzle128)
 {
     PFN_encodeTiled enc = get_encode();
     if (!enc) { hd_set_last_cuda_error((int)cudaErrorNotSupported); return HD_ERR_CUDA; }
@@ -129,17 +129,20 @@ int hd_make_tmap_2d(CUtensorMap* out, const void* base, int dtype, int64_t ny, i
         case HD_F32: dt = CU_TENSOR_MAP_DATA_TYPE_FLOAT32; break;
         case HD_F64: dt = CU_TENSOR_MAP_DATA_TYPE_FLOAT64; break;
         case HD_I32: dt = CU_TENSOR_MAP_DATA_TYPE_INT32; break;
+        case HD_C64: dt = CU_TENSOR_MAP_DATA_TYPE_INT64; break;      // moved as 8-byte words, bits untouched
         default: return HD_ERR_UNSUPPORTED;
     }
     const size_t es = hd_dtype_size(dtype);
     if (((uintptr_t)base & 15) || ((pitch_elems * es) & 15)) return HD_ERR_ALIGN;
     if (box_w > 256 || box_h > 256 || ((box_w * es) & 15)) return HD_ERR_UNSUPPORTED;
+    if (swizzle128 && box_w * es > 128) return HD_ERR_UNSUPPORTED;
+    if (nan_fill && dtype == HD_C64) return HD_ERR_UNSUPPORTED;
     cuuint64_t dims[2] = {(cuuint64_t)nx, (cuuint64_t)ny};
     cuuint64_t strides[1] = {(cuuint64_t)(pitch_elems * es)};
     cuuint32_t box[2] = {(cuuint32_t)box_w, (cuuint32_t)box_h};
     cuuint32_t estr[2] = {1, 1};
     CUresult r = enc(out, dt, 2, const_cast<void*>(base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                     CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
+                     swizzle128 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
                      nan_fill ? CU_TENSOR_MAP_FLOAT_OOB_FILL_NAN_REQUEST_ZERO_FMA : CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (r != CUDA_SUCCESS) { hd_set_last_cuda_error((int)cudaErrorInvalidValue); return HD_ERR_CUDA; }
     return HD_OK;

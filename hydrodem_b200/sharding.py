@@ -416,7 +416,7 @@ class Band:
     def _pass(self, plan, axis, load, src, nrows, out_t, keep_cols=0, mask=None, shift_cols=0, inverse=0, real_out=0):
         lib = _lib.load()
         n = self.nx if axis == 0 else self.ny
-        nbytes = int(nrows) * n * 8
+        nbytes = int(lib.hd_fft_band_workspace_bytes(int(nrows), n))
         work = dev.scratch(nbytes)
         mp, mpitch = (mask.ptr, mask.pitch) if mask is not None else (None, 0)
         _lib.check(lib.hd_fft_band_pass(plan, axis, load, src.ptr, src.pitch, int(nrows), mp, mpitch, int(shift_cols),

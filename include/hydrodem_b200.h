@@ -233,7 +233,9 @@ int hd_fft_rows(void* plan, const void* in, int in_dtype, int64_t in_pitch, void
  * n = plan ny), then the local transpose into out_t (kept_cols x nrows, natural frequency order).  load: 0 real rows
  * (two per transform), 1 complex, 2 (1 - mask) * column-shifted spectrum (mask U8), 3 Hermitian row pairs.  real_out:
  * the pass stores |z| (load 1) or |re| / |im| (load 3) as F32.  keep_cols > 0: only the first keep_cols frequencies
- * are written (half spectrum of real rows).  Workspace: nrows * n * 8 bytes. */
+ * are written (half spectrum of real rows).  Workspace: hd_fft_band_workspace_bytes(nrows, n) (nrows rows of n complex64
+ * with 16-byte-aligned rows). */
+int64_t hd_fft_band_workspace_bytes(int64_t nrows, int64_t n);
 int hd_fft_band_pass(void* plan, int axis, int load, const void* in, int64_t in_pitch, int64_t nrows, const void* mask,
                      int64_t mask_pitch, int shift_cols, int inverse, int real_out, void* out_t, int64_t out_t_pitch,
                      int64_t keep_cols, void* workspace, int64_t workspace_bytes, void* stream);
