@@ -61,6 +61,7 @@ SIGNATURES = {
     "hd_fourier_mask_assemble": (_i, [_p, _i64, _p, _i64, _p, _i, _i64, _i64, _i64, _i, _i, _p]),
     "hd_fft2_plan_create": (_i, [_i64, _i64, ctypes.POINTER(_p)]),
     "hd_fft2_plan_destroy": (_i, [_p]),
+    "hd_fft_plan_info": (_i, [_p, _i, ctypes.POINTER(_i64)]),
     "hd_fft2_workspace_bytes": (_i64, [_i64, _i64]),
     "hd_fft2_forward_shift_abs": (_i, [_p, _p, _i64, _p, _i64, _p, _i64, _p, _i64, _p]),
     "hd_fft2_masked_inverse_abs": (_i, [_p, _p, _i64, _p, _i64, _p, _i, _i64, _p, _i64, _p]),

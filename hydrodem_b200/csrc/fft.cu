@@ -1297,6 +1297,21 @@ int hd_fft2_plan_destroy(void* plan)
     return HD_OK;
 }
 
+int hd_fft_plan_info(const void* plan, int axis, int64_t* info)
+{
+    if (!plan || !info) return HD_ERR_NULL;
+    if (axis < 0 || axis > 1) return HD_ERR_ARG;
+    const Plan2D* p = (const Plan2D*)plan;
+    const Plan1D& pl = axis == 0 ? p->px : p->py;
+    info[0] = pl.n_total;
+    info[1] = pl.n1;
+    info[2] = pl.n;
+    info[3] = pl.m;
+    info[4] = pl.bluestein ? ALG_BLUESTEIN : pl.mixed ? ALG_MIXED : ALG_POW2;
+    info[5] = (!pl.mixed && pl.npass > 0) ? pl.k[pl.npass - 1] : 0;
+    return HD_OK;
+}
+
 // two complex64 scratch arrays of ny x nx, each with room for 16-byte-aligned row pitches in either orientation
 int64_t hd_fft2_workspace_bytes(int64_t ny, int64_t nx) { return 2 * pitch_c64(ny) * pitch_c64(nx) * (int64_t)sizeof(float2); }
 

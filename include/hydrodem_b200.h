@@ -203,6 +203,11 @@ int hd_fourier_mask_assemble(const void* q1, int64_t q1_pitch, const void* q2, i
  * a length with no such factor (a prime above 8192) -> HD_ERR_UNSUPPORTED. */
 int hd_fft2_plan_create(int64_t ny, int64_t nx, void** plan);
 int hd_fft2_plan_destroy(void* plan);
+/* Read-only description of the transform a plan runs along one axis (axis 0: rows of length nx, 1: columns of length
+ * ny).  info[6] = n_total, n1 (cluster size of a long row, 1 = one transform), n (inner length, n_total = n1 * n),
+ * m (shared-memory transform length), algorithm (0 radix-2^k, 1 Bluestein, 2 mixed radix), k of the last radix-2^k
+ * pass (0 when there is none).  No plan or no info -> HD_ERR_NULL; an axis other than 0 or 1 -> HD_ERR_ARG. */
+int hd_fft_plan_info(const void* plan, int axis, int64_t* info);
 int64_t hd_fft2_workspace_bytes(int64_t ny, int64_t nx);
 /* FourierInitial.apply, custom_filters.py:859-877: fft2 (complex64) -> fftshift -> abs.  in: F32 (ny x nx);
  * fshift: C64 out (may be NULL); fabs_out: F32 |F| in shifted layout. */

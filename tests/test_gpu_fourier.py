@@ -157,7 +157,8 @@ def test_fft_size_limit_fails_loudly():
         ef.FourierTransform().apply(np.zeros((16, 10007), dtype=np.float32))
 
 
-@pytest.mark.parametrize("shape", [(40, 9000), (10801, 48), (33, 16384), (18000, 20), (150, 36000)])
+@pytest.mark.parametrize("shape", [(40, 9000), (10801, 48), (33, 16384), (18000, 20), (150, 36000), (5, 32776), (28679, 3),
+                                   (4, 49152), (20000, 6), (9, 7201), (7201, 9)])
 def test_fft_long_rows_vs_scipy(shape):
     """Rows longer than one shared-memory transform: n = n1 * n2 split (9000 = 2 * 4500, 10801 = 7 * 1543,
     18000 = 3 * 6000, 36000 = 5 * 7200) and the 16384 power of two."""
@@ -200,7 +201,7 @@ def test_stripe_removal_long_rows():
     np.testing.assert_allclose(got, want, rtol=RTOL)
 
 
-@pytest.mark.parametrize("shape", [(301, 333), (259, 10801), (333, 300)])
+@pytest.mark.parametrize("shape", [(301, 333), (259, 10801), (333, 300), (131, 7201), (2025, 135), (10125, 131), (301, 256)])
 def test_stripe_removal_odd_sizes_hermitian_path(shape, monkeypatch):
     """Odd x odd rasters take the Hermitian (real-output) inverse: half of the rows in the first pass, two output
     columns per transform in the second.  Must agree with the oracle, and with the plain complex path."""
