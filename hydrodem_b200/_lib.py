@@ -18,6 +18,7 @@ HD_ERR_ALIGN, HD_ERR_CUDA, HD_ERR_UNSUPPORTED, HD_ERR_ARG, HD_ERR_WORKSPACE = -4
 U8, F32, F64, I64, C64, C128, I32, I16 = range(8)
 OP_COPY, OP_MUL, OP_ADD, OP_RSUB, OP_LT, OP_GT, OP_ABS, OP_RINT, OP_XOR, OP_TRUNC = range(10)
 MORPH_ERODE, MORPH_DILATE, MORPH_CLOSE, MORPH_OPEN = range(4)
+HD_SCATTER_MAX_SEGS = 16
 
 _p, _i, _i64, _d = ctypes.c_void_p, ctypes.c_int, ctypes.c_int64, ctypes.c_double
 
@@ -105,7 +106,7 @@ class ScatterSeg(ctypes.Structure):
 
 class Scatter(ctypes.Structure):
     """hd_scatter of include/hydrodem_b200.h."""
-    _fields_ = [("nseg", ctypes.c_int32), ("ncolseg", ctypes.c_int32), ("seg", ScatterSeg * 16),
+    _fields_ = [("nseg", ctypes.c_int32), ("ncolseg", ctypes.c_int32), ("seg", ScatterSeg * HD_SCATTER_MAX_SEGS),
                 ("col_local0", _i64 * 2), ("col_dst0", _i64 * 2), ("col_len", _i64 * 2)]
 
 

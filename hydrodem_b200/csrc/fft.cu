@@ -1270,6 +1270,28 @@ TransArgs trans_args(void* out, int64_t out_pitch, int rows, int cols, RowPerm p
     return a;
 }
 
+// The row pass of hd_fft_band_pass(_scatter): checks the arguments they share, then transforms the nrows local rows
+// into the workspace, [nrows][*pitch] of complex64 (float when real_out) with 16-byte-aligned rows.  *pl: the plan of
+// the transformed axis.
+int band_rows(void* plan, int axis, int load, const void* in, int64_t in_pitch, int64_t nrows, const void* mask,
+              int64_t mask_pitch, int shift_cols, int inverse, int real_out, void* workspace, int64_t workspace_bytes,
+              cudaStream_t s, const Plan1D** pl, int64_t* pitch)
+{
+    if (!plan || !in || !workspace) return HD_ERR_NULL;
+    Plan2D* p = (Plan2D*)plan;
+    *pl = axis == 0 ? &p->px : &p->py;
+    const int n = (*pl)->n_total;
+    if (nrows < 1 || nrows > 0x7fffffff || axis < 0 || axis > 1 || load < 0 || load > 3) return HD_ERR_ARG;
+    if (load == LOAD_MASKED_SHIFTED && !mask) return HD_ERR_NULL;
+    if (load == LOAD_C64_HPAIR && !real_out) return HD_ERR_ARG;
+    if (workspace_bytes < hd_fft_band_workspace_bytes(nrows, n)) return HD_ERR_WORKSPACE;
+    if (in_pitch < n) return HD_ERR_ARG;
+    *pitch = real_out ? pitch_f32(n) : pitch_c64(n);
+    RowsArgs r{in, in_pitch, (float2*)workspace, *pitch, (const uint8_t*)mask, mask_pitch, (int)nrows, 0, shift_cols,
+               inverse ? 1 : 0, real_out ? 1 : 0, (int)nrows};
+    return launch_rows(**pl, r, load, s);
+}
+
 }  // namespace
 
 extern "C" {
@@ -1460,25 +1482,18 @@ int hd_fft_band_pass(void* plan, int axis, int load, const void* in, int64_t in_
                      int64_t mask_pitch, int shift_cols, int inverse, int real_out, void* out_t, int64_t out_t_pitch,
                      int64_t keep_cols, void* workspace, int64_t workspace_bytes, void* stream)
 {
-    if (!plan || !in || !out_t || !workspace) return HD_ERR_NULL;
-    Plan2D* p = (Plan2D*)plan;
-    const Plan1D& pl = axis == 0 ? p->px : p->py;
-    const int n = pl.n_total;
-    if (nrows < 1 || nrows > 0x7fffffff || axis < 0 || axis > 1 || load < 0 || load > 3) return HD_ERR_ARG;
-    if (load == LOAD_MASKED_SHIFTED && !mask) return HD_ERR_NULL;
-    if (load == LOAD_C64_HPAIR && !real_out) return HD_ERR_ARG;
-    if (workspace_bytes < hd_fft_band_workspace_bytes(nrows, n)) return HD_ERR_WORKSPACE;
-    if (in_pitch < n || out_t_pitch < nrows) return HD_ERR_ARG;
+    if (!out_t) return HD_ERR_NULL;
+    if (out_t_pitch < nrows) return HD_ERR_ARG;
     cudaStream_t s = (cudaStream_t)stream;
-    float2* A = (float2*)workspace;                 // [nrows][pitch] of complex64, or of float when real_out
-    const int64_t pitch = real_out ? pitch_f32(n) : pitch_c64(n);
-    RowsArgs r{in, in_pitch, A, pitch, (const uint8_t*)mask, mask_pitch, (int)nrows, 0, shift_cols, inverse ? 1 : 0,
-               real_out ? 1 : 0, (int)nrows};
-    if (int e = launch_rows(pl, r, load, s)) return e;
-    TransArgs t = trans_args(out_t, out_t_pitch, (int)nrows, n, perm_of(pl, load));
-    if (real_out) return launch_transpose<float, float, false>((const float*)A, pitch, t, s, "transpose_real_kernel");
+    const Plan1D* pl;
+    int64_t pitch;
+    if (int e = band_rows(plan, axis, load, in, in_pitch, nrows, mask, mask_pitch, shift_cols, inverse, real_out, workspace,
+                          workspace_bytes, s, &pl, &pitch))
+        return e;
+    TransArgs t = trans_args(out_t, out_t_pitch, (int)nrows, pl->n_total, perm_of(*pl, load));
+    if (real_out) return launch_transpose<float, float, false>((const float*)workspace, pitch, t, s, "transpose_real_kernel");
     t.keep_max = keep_cols > 0 ? (int)keep_cols - 1 : -1;
-    return launch_transpose<float2, float2, false>(A, pitch, t, s, "transpose_kernel");
+    return launch_transpose<float2, float2, false>((const float2*)workspace, pitch, t, s, "transpose_kernel");
 }
 
 
@@ -1489,28 +1504,21 @@ int hd_fft_band_pass_scatter(void* plan, int axis, int load, const void* in, int
                              int64_t mask_pitch, int shift_cols, int inverse, int real_out, const hd_scatter* sc,
                              int64_t keep_cols, void* workspace, int64_t workspace_bytes, void* stream)
 {
-    if (!plan || !in || !sc || !workspace) return HD_ERR_NULL;
-    Plan2D* p = (Plan2D*)plan;
-    const Plan1D& pl = axis == 0 ? p->px : p->py;
-    const int n = pl.n_total;
-    if (nrows < 1 || nrows > 0x7fffffff || axis < 0 || axis > 1 || load < 0 || load > 3) return HD_ERR_ARG;
+    if (!sc) return HD_ERR_NULL;
     if (sc->nseg < 0 || sc->nseg > HD_SCATTER_MAX_SEGS || sc->ncolseg < 0 || sc->ncolseg > 2) return HD_ERR_ARG;
-    if (load == LOAD_MASKED_SHIFTED && !mask) return HD_ERR_NULL;
-    if (load == LOAD_C64_HPAIR && !real_out) return HD_ERR_ARG;
-    if (workspace_bytes < nrows * (int64_t)n * (int64_t)sizeof(float2)) return HD_ERR_WORKSPACE;
-    if (in_pitch < n) return HD_ERR_ARG;
     cudaStream_t s = (cudaStream_t)stream;
-    float2* A = (float2*)workspace;
-    RowsArgs r{in, in_pitch, A, n, (const uint8_t*)mask, mask_pitch, (int)nrows, 0, shift_cols, inverse ? 1 : 0,
-               real_out ? 1 : 0, (int)nrows};
-    if (int e = launch_rows(pl, r, load, s)) return e;
-    const RowPerm pm = perm_of(pl, load);
+    const Plan1D* pl;
+    int64_t pitch;
+    if (int e = band_rows(plan, axis, load, in, in_pitch, nrows, mask, mask_pitch, shift_cols, inverse, real_out, workspace,
+                          workspace_bytes, s, &pl, &pitch))
+        return e;
+    const int n = pl->n_total, grid = transpose_grid((int)nrows, n), keep_max = keep_cols > 0 ? (int)keep_cols - 1 : -1;
+    const RowPerm pm = perm_of(*pl, load);
     hd_prof_begin("transpose_scatter_kernel", s);
     if (real_out)
-        transpose_scatter_kernel<float><<<transpose_grid((int)nrows, n), 256, 0, s>>>((const float*)A, n, (int)nrows, n, pm, -1, *sc);
+        transpose_scatter_kernel<float><<<grid, 256, 0, s>>>((const float*)workspace, pitch, (int)nrows, n, pm, -1, *sc);
     else
-        transpose_scatter_kernel<float2><<<transpose_grid((int)nrows, n), 256, 0, s>>>(A, n, (int)nrows, n, pm,
-                                                                                     keep_cols > 0 ? (int)keep_cols - 1 : -1, *sc);
+        transpose_scatter_kernel<float2><<<grid, 256, 0, s>>>((const float2*)workspace, pitch, (int)nrows, n, pm, keep_max, *sc);
     HD_LAUNCH_CHECK(); hd_count_launch();
     return HD_OK;
 }

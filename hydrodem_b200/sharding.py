@@ -12,9 +12,11 @@ result equals the single-GPU result BIT FOR BIT -- exact-class and tolerance-cla
   (csrc/quadratic.cu accumulates in double for exactly this reason), so cut positions cannot change a bit.
 * **Fourier stage**: the row / column transforms of ``hd_fft2_forward_shift_abs`` / ``hd_fft2_masked_inverse_abs`` run
   on each rank's local rows through ``hd_fft_band_pass`` (the same row passes, same pairing), the four transposes
-  become all-to-all exchanges (grouped NCCL send / recv), the conjugate half of the spectrum is completed locally
-  because each rank owns a set of spectrum rows closed under ky -> -ky ("K layout"), and the window-55 peak detector
-  works on row slabs of the spectrum quarters with 61 rows of context (|F| stays banded: no all-gather).
+  become all-to-all exchanges (``fourier_exchanges``: the transposes store straight into the owning rank's memory,
+  mapped through CUDA IPC; where the ranks cannot map each other's memory the transposed blocks travel as NCCL send /
+  recv), the conjugate half of the spectrum is completed locally because each rank owns a set of spectrum rows closed
+  under ky -> -ky ("K layout"), and the window-55 peak detector works on row slabs of the spectrum quarters with 61
+  rows of context (|F| stays banded: no all-gather).
 * **Sink-fill**: every rank relaxes [halo row | band | halo row] to its local fixed point, edge rows are exchanged, a
   small kernel lowers the halo rows and raises a DEVICE flag, the flags are all-reduced and the host reads one word
   per round.  The fixed point is unique, so the banded surface equals the single-GPU one; NaN restoration and D8 are
@@ -25,6 +27,7 @@ The communicator is abstract: ``DistComm`` (torch.distributed: NCCL on the GPU b
 """
 import ctypes
 import threading
+import typing
 
 import numpy as np
 import torch
@@ -87,18 +90,10 @@ class DistComm:
         self.rank = dist.get_rank(group)
         self.world = dist.get_world_size(group)
 
-    class _Handle:
-        def __init__(self, works):
-            self.works = works
-
-        def wait(self):
-            for w in self.works:
-                w.wait()                        # NCCL: the current stream waits for the transfer, the host does not
-
-    def p2p_async(self, sends, recvs):
+    def p2p(self, sends, recvs):
         """sends: [(contiguous tensor, dst rank)], recvs: [(contiguous tensor, src rank)].  Messages between one pair of
         ranks are matched in posting order.  One grouped batch: NCCL fuses it into a single kernel over NVLink, on its
-        own stream -- kernels launched before ``wait()`` overlap the transfer."""
+        own stream."""
         dist = self.dist
         local = [t for t, d in sends if d == self.rank]
         ops = []
@@ -110,10 +105,8 @@ class DistComm:
         for t, d in sends:
             if d != self.rank:
                 ops.append(dist.P2POp(dist.isend, t, d, self.group))
-        return self._Handle(dist.batch_isend_irecv(ops) if ops else [])
-
-    def p2p(self, sends, recvs):
-        self.p2p_async(sends, recvs).wait()
+        for w in dist.batch_isend_irecv(ops) if ops else []:
+            w.wait()                            # NCCL: the current stream waits for the transfer, the host does not
 
     def allreduce_max_(self, t):
         self.dist.all_reduce(t, op=self.dist.ReduceOp.MAX, group=self.group)
@@ -163,10 +156,6 @@ class ThreadComm:
             torch.cuda.synchronize()
         sh.barrier.wait()
 
-    class _Done:
-        def wait(self):
-            pass
-
     same_process = True
 
     def gather_objects(self, obj):
@@ -181,10 +170,6 @@ class ThreadComm:
         if torch.cuda.is_available():
             torch.cuda.synchronize()
         self.shared.barrier.wait()
-
-    def p2p_async(self, sends, recvs):
-        self.p2p(sends, recvs)
-        return self._Done()
 
     def allreduce_max_(self, t):
         sh = self.shared
@@ -262,6 +247,60 @@ def redistribute_rows(comm, src, src_ids, dst_ids, dst, key=None):
 def _cview(t):
     """complex64 tensor -> float32 view with a trailing dimension of 2 (what the communicators move)."""
     return torch.view_as_real(t) if t.is_complex() else t
+
+
+# ---- geometry of the sharded Fourier stage (host only) --------------------------------------------------------------------
+def k_layouts(ny, world):
+    """Per rank: spectrum rows ky in [a, b) plus their mirrors ("K layout", hd_klayout_*): dict(a, b, rows, nlo, nhi, hlo,
+    ky = the ky of every local row)."""
+    lib = _lib.load()
+    out = []
+    for a, b in band_bounds(ny // 2 + 1, world, 1):
+        n = int(lib.hd_klayout_rows(a, b, ny))
+        nlo = b - a
+        nhi = n - nlo
+        hlo = int(lib.hd_klayout_ky(a, b, ny, nlo)) if nhi else 0
+        out.append(dict(a=a, b=b, rows=n, nlo=nlo, nhi=nhi, hlo=hlo,
+                        ky=np.concatenate([np.arange(a, b), np.arange(hlo, hlo + nhi)]).astype(np.int64)))
+    return out
+
+
+class Exchange(typing.NamedTuple):
+    """One pass of the sharded Fourier stage: every rank transforms its local rows and transposes the result T (one row
+    per frequency / pixel of the transformed axis, one column per local row); T then changes hands.
+      ranges[j]   row ranges of T that rank j holds, concatenated in this order in its buffer ``dest``
+      colsegs[i]  [(local row0, column0, length)]: where rank i's local rows land along the ``cols`` columns of ``dest``;
+                  they cover rank i's rows 0 .. n_i - 1 of the pass, so they also say how many rows it transforms"""
+    ranges: list
+    colsegs: list
+    dest: str
+    cols: int
+
+
+def fourier_exchanges(ny, nx, bounds):
+    """The K layouts and the four exchanges {"F1", "F2", "I1", "I2"} of DetectApplyFourier on row bands ``bounds``."""
+    W = len(bounds)
+    nh = nx // 2 + 1
+    odd = bool((ny & 1) and (nx & 1))
+    CB, XB = band_bounds(nh, W, 1), band_bounds(nx, W, 2)
+    KL = k_layouts(ny, W)
+
+    def spans(bb):                                       # rank i's rows land at the columns of its own band bb[i]
+        return [[(0, a, b - a)] for a, b in bb]
+
+    return KL, {
+        # forward along x (two real rows per transform, half spectrum kept): my columns of the half spectrum, all y
+        "F1": Exchange([[c] for c in CB], spans(bounds), "at", ny),
+        # forward along y into the K layout: rank j gets rows ky in [a_j, b_j) and their mirrors
+        "F2": Exchange([[(k["a"], k["b"]), (k["hlo"], k["hlo"] + k["nhi"])] for k in KL], spans(CB), "half", nh),
+        # inverse along x of (1 - mask) * F on my spectrum rows (the Hermitian, odd x odd, path needs only ky <= ny/2;
+        # hd_conj_mirror_fill writes the other columns): my x columns, all ky
+        "I1": Exchange([[x] for x in XB],
+                       [[(0, k["a"], k["nlo"])] + ([(k["nlo"], k["hlo"], k["nhi"])] if k["nhi"] and not odd else [])
+                        for k in KL], "bt", ny),
+        # inverse along y, real output (two columns per transform on the Hermitian path): my rows, all x
+        "I2": Exchange([[r] for r in bounds], spans(XB), "dem", nx),
+    }
 
 
 # ---- peer memory: persistent exchange buffers every rank can store into ---------------------------------------------------
@@ -360,9 +399,12 @@ class Band:
         self.narrow_final = os.environ.get("HD_NARROW_FINAL", "1") != "0"   # apply_to_host: final DEM down as int16
         if comm.world > 1 and min(b - a for a, b in self.bounds) < 2 * self.fill_overlap:
             self.fill_overlap = max(8, min(b - a for a, b in self.bounds) // 16 * 8)
-        self.up = self.halo if comm.rank > 0 else 0
-        self.down = self.halo if comm.rank < comm.world - 1 else 0
+        self.up, self.down = self._margins(comm.rank)
         self.fill_rounds = None
+
+    def _margins(self, rank):
+        """Halo rows above / below the band of ``rank`` (none at the ends of the mosaic)."""
+        return (self.halo if rank > 0 else 0), (self.halo if rank < self.comm.world - 1 else 0)
 
     @property
     def rows(self):
@@ -413,122 +455,114 @@ class Band:
         tdt = {_lib.C64: torch.complex64, _lib.F32: torch.float32, _lib.U8: torch.uint8}[dtype]
         return dev.DeviceRaster(torch.empty((max(int(rows), 1), int(cols)), dtype=tdt, device=dev.device()), rows, cols, dtype)
 
-    def _pass(self, plan, axis, load, src, nrows, out_t, keep_cols=0, mask=None, shift_cols=0, inverse=0, real_out=0):
-        lib = _lib.load()
-        n = self.nx if axis == 0 else self.ny
-        nbytes = int(lib.hd_fft_band_workspace_bytes(int(nrows), n))
-        work = dev.scratch(nbytes)
-        mp, mpitch = (mask.ptr, mask.pitch) if mask is not None else (None, 0)
-        _lib.check(lib.hd_fft_band_pass(plan, axis, load, src.ptr, src.pitch, int(nrows), mp, mpitch, int(shift_cols),
-                                        int(inverse), int(real_out), out_t.ptr, out_t.pitch, int(keep_cols),
-                                        ctypes.c_void_p(work.data_ptr()), nbytes, dev.stream_ptr()))
-
-    def _peer_setup(self, KL, CB, XB):
-        """Persistent exchange buffers of the Fourier stage in peer-mapped memory (once per Band).  None: the ranks could
-        not map each other's memory (or HD_BAND_DIRECT=0) -- the exchanges then go through NCCL send / recv."""
-        if not hasattr(self, "_peers"):
+    def _fourier_setup(self):
+        """The K layouts and exchanges of the Fourier stage, and its persistent exchange buffers in peer-mapped memory
+        (``self._peers``; once per Band).  No peers: the ranks could not map each other's memory (or HD_BAND_DIRECT=0)
+        -- the exchanges then go through NCCL send / recv."""
+        if not hasattr(self, "_fourier"):
             import os
+            self._fourier = fourier_exchanges(self.ny, self.nx, self.bounds)
             self._peers = None
             if self.comm.world > 1 and os.environ.get("HD_BAND_DIRECT", "1") != "0":
-                lib = _lib.load()
-                me = self.comm.rank
-                kl = KL[me]
-                pitch = int(lib.hd_pitch_elems(self.nx, _lib.F32))
-                sizes = {"at": (CB[me][1] - CB[me][0]) * self.ny * 8, "half": kl["rows"] * (self.nx // 2 + 1) * 8,
-                         "bt": (XB[me][1] - XB[me][0]) * self.ny * 8, "dem": (self.up + self.rows + self.down) * pitch * 4}
+                sizes = {}
+                for ex in self._fourier[1].values():
+                    rows, pitch, _, itemsize = self._buffer_shape(ex, self.comm.rank)
+                    sizes[ex.dest] = rows * pitch * itemsize
                 peers = PeerBuffers(self.comm, sizes)
                 if peers.ok:
-                    peers.dem_pitch = self.comm.gather_objects((pitch, self.up))
                     self._peers = peers
-        return self._peers
+        return self._fourier
 
-    def _pass_scatter(self, plan, axis, load, src, nrows, segs, colsegs, keep_cols=0, mask=None, shift_cols=0, inverse=0,
-                      real_out=0):
-        """Row pass + transpose whose stores go straight into the owning ranks' buffers (hd_fft_band_pass_scatter).
-        segs: [(row0, row1, device pointer, pitch in elements, dst_row0)]; colsegs: [(local row0, column0, length)]."""
+    def _buffer_shape(self, ex, rank):
+        """Buffer ``ex.dest`` of ``rank``: (rows, pitch in elements, first row the exchange writes, bytes per element).
+        "dem" is the stripe-free DEM with the band's halo margins (the layout of ``alloc_ext``); the others are dense."""
+        rows = sum(b - a for a, b in ex.ranges[rank])
+        if ex.dest != "dem":
+            return rows, ex.cols, 0, 8
+        up, down = self._margins(rank)
+        return up + rows + down, int(_lib.load().hd_pitch_elems(self.nx, _lib.F32)), up, 4
+
+    def _buffer(self, ex):
+        """This rank's buffer ``ex.dest`` (a view of the peer arena, else a new allocation; an ExtRaster for "dem") and,
+        when the ranks store into each other's memory, every rank's (address of the first written row, pitch)."""
+        rows, pitch, _, _ = self._buffer_shape(ex, self.comm.rank)
+        dtype = _lib.F32 if ex.dest == "dem" else _lib.C64
+        peers, targets = self._peers, None
+        if peers is None:
+            buf = self._dense(rows, pitch, dtype)
+        else:
+            buf = peers.view(ex.dest, rows, pitch, dtype)
+            targets = []
+            for j in range(self.comm.world):
+                _, pitch_j, first_j, itemsize = self._buffer_shape(ex, j)
+                targets.append((peers.ptr(j, ex.dest) + first_j * pitch_j * itemsize, pitch_j))
+        buf = buf.sub(0, rows, 0, ex.cols)
+        if ex.dest == "dem":
+            buf = ExtRaster(buf.with_ref(np.float64), self.up, self.rows, self.down)
+        return buf, targets
+
+    def _exchange(self, plan, axis, load, src, ex, keep_cols=0, mask=None, shift_cols=0, inverse=0, real_out=0):
+        """One pass of the sharded Fourier stage: the row transforms of this rank's rows of ``src`` (hd_fft_band_pass,
+        ``load`` and the keywords as there), then exchange ``ex`` of the transposed result.  Returns the buffer
+        ``ex.dest``.  With peer-mapped buffers the transpose stores every element straight into the memory of the rank
+        that owns it (hd_fft_band_pass_scatter) and a device barrier follows ("all stores landed"); otherwise the
+        transposed block goes out by send / recv and the blocks received are put in place.  Every rank takes part in
+        the barrier / the send / recv, with or without rows of its own."""
         lib = _lib.load()
-        n = self.nx if axis == 0 else self.ny
-        sc = _lib.Scatter()
-        segs = [g for g in segs if g[1] > g[0]]
-        sc.nseg, sc.ncolseg = len(segs), len(colsegs)
-        for k, (a, b, ptr, pitch, d0) in enumerate(segs):
-            sc.seg[k].row0, sc.seg[k].row1, sc.seg[k].base, sc.seg[k].pitch, sc.seg[k].dst_row0 = a, b, ptr, pitch, d0
-        for k, (l0, c0, ln) in enumerate(colsegs):
-            sc.col_local0[k], sc.col_dst0[k], sc.col_len[k] = l0, c0, ln
-        if nrows < 1:
-            return
-        nbytes = int(nrows) * n * 8
-        work = dev.scratch(nbytes)
-        mp, mpitch = (mask.ptr, mask.pitch) if mask is not None else (None, 0)
-        _lib.check(lib.hd_fft_band_pass_scatter(plan, axis, load, src.ptr, src.pitch, int(nrows), mp, mpitch, int(shift_cols),
-                                                int(inverse), int(real_out), ctypes.byref(sc), int(keep_cols),
-                                                ctypes.c_void_p(work.data_ptr()), nbytes, dev.stream_ptr()))
-
-    def _pass_exchange(self, plan, axis, load, src, counts, n_out, ranges, segs, out, dtype, mask=None, **kw):
-        """(Fallback when the ranks cannot map each other's memory.)  A row pass of the sharded Fourier stage followed by its all-to-all, software pipelined: the local rows are
-        transformed in a few chunks, the transposed block of chunk c (n_out x chunk rows) is on its way (NCCL's stream)
-        while chunk c + 1 is being transformed, and the blocks that arrive are put in place one chunk behind.
-          counts[i]  rows rank i transforms in this pass          ranges[j]  row ranges of the transposed block rank j gets
-          segs[i]    [(local row0, output column0, length)]: where rank i's local rows land along the columns of ``out``
-        ``out`` rows = the concatenation of ranges[me]."""
         comm, W, me = self.comm, self.comm.world, self.comm.rank
-        nch = 1          # (chunked pipelining did not overlap: NCCL's send / recv kernels wait behind the persistent grids)
-        chunks = [band_bounds(c, nch, 2) for c in counts]
-        tdt = {_lib.C64: torch.complex64, _lib.F32: torch.float32}[dtype]
-        pending = []
-        to = out.tensor()
+        n = self.nx if axis == 0 else self.ny
+        nrows = [max((l0 + ln for l0, _, ln in segs), default=0) for segs in ex.colsegs]
+        out, targets = self._buffer(ex)
+        mp, mpitch = (mask.ptr, mask.pitch) if mask is not None else (None, 0)
 
-        def place(item):
-            handle, places, _keep = item
-            handle.wait()
-            for buf, off, i, ia, ib in places:
-                for l0, c0, ln in segs[i]:
-                    lo, hi = max(ia, l0), min(ib, l0 + ln)
-                    if hi > lo:
-                        to[off:off + buf.shape[0], c0 + (lo - l0):c0 + (hi - l0)].copy_(buf[:, lo - ia:hi - ia])
+        def band_pass(fn, *out_args):                  # out_args: (out_t, out_t pitch) or (hd_scatter*,)
+            nbytes = int(lib.hd_fft_band_workspace_bytes(nrows[me], n))
+            work = dev.scratch(nbytes)
+            _lib.check(fn(plan, axis, load, src.ptr, src.pitch, nrows[me], mp, mpitch, int(shift_cols), int(inverse),
+                          int(real_out), *out_args, int(keep_cols), ctypes.c_void_p(work.data_ptr()), nbytes,
+                          dev.stream_ptr()))
 
-        for c in range(nch):
-            ra, rb = chunks[me][c]
-            t, sends = None, []
-            if rb > ra:
-                t = self._dense(n_out, rb - ra, dtype)
-                self._pass(plan, axis, load, src.sub(ra, rb, 0, src.nx), rb - ra, t,
-                           mask=mask.sub(ra, rb, 0, mask.nx) if mask is not None else None, **kw)
-                tt = t.tensor()
-                for j in range(W):
-                    sends += [(_cview(tt[a:b]), j) for a, b in ranges[j] if b > a]
-            recvs, places = [], []
-            for i in range(W):
-                ia, ib = chunks[i][c]
+        if targets is not None:
+            # segment = a row range of T in one rank's buffer, at its offset in that rank's concatenation
+            sc = _lib.Scatter()
+            for j, (ptr, pitch) in enumerate(targets):
                 off = 0
-                for a, b in ranges[me]:
-                    if b > a and ib > ia:
-                        buf = torch.empty((b - a, ib - ia), dtype=tdt, device=to.device)
-                        recvs.append((_cview(buf), i))
-                        places.append((buf, off, i, ia, ib))
+                for a, b in ex.ranges[j]:
+                    if b > a:
+                        sc.seg[sc.nseg] = _lib.ScatterSeg(a, b, ptr, pitch, off)
+                        sc.nseg += 1
                     off += b - a
-            pending.append((comm.p2p_async(sends, recvs), places, t))
-            if len(pending) > 1:
-                place(pending.pop(0))
-        while pending:
-            place(pending.pop(0))
+            for l0, c0, ln in ex.colsegs[me]:
+                sc.col_local0[sc.ncolseg], sc.col_dst0[sc.ncolseg], sc.col_len[sc.ncolseg] = l0, c0, ln
+                sc.ncolseg += 1
+            if nrows[me]:
+                band_pass(lib.hd_fft_band_pass_scatter, ctypes.byref(sc))
+            comm.device_barrier()
+            return out
+        region = out.owned() if isinstance(out, ExtRaster) else out
+        sends = []
+        if nrows[me]:
+            t = self._dense(keep_cols or n, nrows[me], region.dtype)
+            band_pass(lib.hd_fft_band_pass, t.ptr, t.pitch)
+            tt = t.tensor()
+            sends = [(_cview(tt[a:b]), j) for j in range(W) for a, b in ex.ranges[j] if b > a]
+        to = region.tensor()
+        recvs, places = [], []
+        for i in range(W):
+            off = 0
+            for a, b in ex.ranges[me]:
+                if b > a and nrows[i]:
+                    buf = torch.empty((b - a, nrows[i]), dtype=to.dtype, device=to.device)
+                    recvs.append((_cview(buf), i))
+                    places.append((buf, off, i))
+                off += b - a
+        comm.p2p(sends, recvs)
+        for buf, off, i in places:
+            for l0, c0, ln in ex.colsegs[i]:
+                to[off:off + buf.shape[0], c0:c0 + ln].copy_(buf[:, l0:l0 + ln])
         return out
 
-    def _k_layouts(self):
-        """Per rank: (a, b, rows, [ky of every local row]) -- spectrum rows ky in [a, b) plus their mirrors."""
-        lib = _lib.load()
-        nyh = self.ny // 2 + 1
-        out = []
-        for a, b in band_bounds(nyh, self.comm.world, 1):
-            n = int(lib.hd_klayout_rows(a, b, self.ny))
-            nlo = b - a
-            nhi = n - nlo
-            hlo = int(lib.hd_klayout_ky(a, b, self.ny, nlo)) if nhi else 0
-            out.append(dict(a=a, b=b, rows=n, nlo=nlo, nhi=nhi, hlo=hlo,
-                            ky=np.concatenate([np.arange(a, b), np.arange(hlo, hlo + nhi)]).astype(np.int64)))
-        return out
-
-    def detect_apply_fourier(self, srtm, out_ext=None):
+    def detect_apply_fourier(self, srtm):
         """DetectApplyFourier (custom_filters.py:1053-1101) on a banded mosaic.  ``srtm``: F32 device raster of this
         rank's rows.  Returns an ExtRaster (F32 storage, float64 reference dtype) whose owned rows hold the stripe-free
         DEM -- bit-identical to ``DetectApplyFourier().run_device`` on the whole mosaic; its halo rows are NOT filled."""
@@ -538,47 +572,17 @@ class Band:
         ny, nx = self.ny, self.nx
         nh = nx // 2 + 1
         odd = bool((ny & 1) and (nx & 1))
-        RB, CB, XB = self.bounds, band_bounds(nh, W, 1), band_bounds(nx, W, 2)
-        KL = self._k_layouts()
+        KL, ex = self._fourier_setup()
         kl = KL[me]
         plan = dev.fft_plan(ny, nx)
-        rows = self.rows
         src = dev.convert(srtm, _lib.F32)
 
         TRACE.mark("daf:start")
-        counts_rows = [b - a for a, b in RB]
-        counts_cb = [b - a for a, b in CB]
-        counts_xb = [b - a for a, b in XB]
-        c0, c1 = CB[me]
-        # forward along x (two real rows per transform, half spectrum kept) + all-to-all: my columns of the half
-        # spectrum, all y
-        peers = self._peer_setup(KL, CB, XB)
-        if peers is not None:
-            # the transposes store straight into the owning rank's buffers over NVLink (no NCCL, no unpack copies);
-            # device-side barriers say "destinations free" / "all stores landed"
-            comm.device_barrier()
-            at = peers.view("at", c1 - c0, ny, _lib.C64)
-            self._pass_scatter(plan, 0, LOAD_REAL, src, rows, [(CB[j][0], CB[j][1], peers.ptr(j, "at"), ny, 0) for j in range(W)],
-                               [(0, RB[me][0], rows)], keep_cols=nh)
-            comm.device_barrier()
-            TRACE.mark("F1 rows + T1")
-            half = peers.view("half", kl["rows"], nh, _lib.C64)
-            segs2 = []
-            for j, k in enumerate(KL):
-                segs2.append((k["a"], k["b"], peers.ptr(j, "half"), nh, 0))
-                segs2.append((k["hlo"], k["hlo"] + k["nhi"], peers.ptr(j, "half"), nh, k["nlo"]))
-            self._pass_scatter(plan, 1, LOAD_C64, at, c1 - c0, segs2, [(0, c0, c1 - c0)])
-            comm.device_barrier()
-        else:
-            at = self._dense(c1 - c0, ny, _lib.C64)
-            self._pass_exchange(plan, 0, LOAD_REAL, src, counts_rows, nh, [[cb] for cb in CB],
-                                [[(0, RB[i][0], counts_rows[i])] for i in range(W)], at, _lib.C64, keep_cols=nh)
-            TRACE.mark("F1 rows + T1")
-            # forward along y + exchange into the K layout: rank i gets rows ky in [a_i, b_i) and their mirrors
-            half = self._dense(kl["rows"], nh, _lib.C64)
-            self._pass_exchange(plan, 1, LOAD_C64, at, counts_cb, ny,
-                                [[(k["a"], k["b"]), (k["hlo"], k["hlo"] + k["nhi"])] for k in KL],
-                                [[(0, CB[i][0], counts_cb[i])] for i in range(W)], half, _lib.C64)
+        if self._peers is not None:
+            comm.device_barrier()          # destinations free: no rank still reads its buffers of the last call
+        at = self._exchange(plan, 0, LOAD_REAL, src, ex["F1"], keep_cols=nh)
+        TRACE.mark("F1 rows + T1")
+        half = self._exchange(plan, 1, LOAD_C64, at, ex["F2"])
         del at
         TRACE.mark("F2 cols + T2")
         # conjugate half, column shift, |F|  (FourierInitial, custom_filters.py:859-877)
@@ -649,42 +653,16 @@ class Band:
         self._last_mask = (mask, kl)
         TRACE.mark("mask back + assemble")
 
-        # ---- inverse along x: (1 - mask) * F on this rank's spectrum rows (the Hermitian, odd x odd, path needs only
-        # ky <= ny/2) + all-to-all: my x columns, all ky -------------------------------------------------------------
-        counts_i1 = [(k["nlo"] if odd else k["rows"]) for k in KL]
-        xa, xb = XB[me]
-        segs = [[(0, k["a"], k["nlo"])] + ([(k["nlo"], k["hlo"], k["nhi"])] if (not odd and k["nhi"]) else []) for k in KL]
-        if peers is not None:
-            bt = peers.view("bt", xb - xa, ny, _lib.C64)
-            self._pass_scatter(plan, 0, LOAD_MASKED, fshift, counts_i1[me],
-                               [(XB[j][0], XB[j][1], peers.ptr(j, "bt"), ny, 0) for j in range(W)], segs[me], mask=mask,
-                               shift_cols=nx // 2, inverse=1)
-            comm.device_barrier()
-        else:
-            bt = self._dense(xb - xa, ny, _lib.C64)
-            self._pass_exchange(plan, 0, LOAD_MASKED, fshift, counts_i1, nx, [[x] for x in XB], segs, bt, _lib.C64, mask=mask,
-                                shift_cols=nx // 2, inverse=1)
+        # ---- inverse: along x (1 - mask) * F, then along y with real output ----------------------------------------
+        bt = self._exchange(plan, 0, LOAD_MASKED, fshift, ex["I1"], mask=mask, shift_cols=nx // 2, inverse=1)
         del fshift
         TRACE.mark("I1 rows + T3")
         if odd:
-            _lib.check(lib.hd_conj_mirror_fill(bt.ptr, bt.pitch, xb - xa, ny, dev.stream_ptr()))
-        # inverse along y: real output (two columns per transform on the Hermitian path) + all-to-all: my rows, all x
-        if peers is not None:
-            pitch, _ = peers.dem_pitch[me]
-            dbuf = peers.arena[peers.offsets["dem"]:peers.offsets["dem"] + (self.up + rows + self.down) * pitch * 4]
-            out_ext = ExtRaster(dev.DeviceRaster(dbuf.view(torch.float32).view(self.up + rows + self.down, pitch),
-                                                 self.up + rows + self.down, nx, _lib.F32, np.float64), self.up, rows, self.down)
-            self._pass_scatter(plan, 1, LOAD_HPAIR if odd else LOAD_C64, bt, xb - xa,
-                               [(RB[j][0], RB[j][1], peers.ptr(j, "dem") + peers.dem_pitch[j][1] * peers.dem_pitch[j][0] * 4,
-                                 peers.dem_pitch[j][0], 0) for j in range(W)], [(0, xa, xb - xa)], inverse=1, real_out=1)
-            comm.device_barrier()
-        else:
-            out_ext = out_ext or self.alloc_ext(_lib.F32, np.float64)
-            self._pass_exchange(plan, 1, LOAD_HPAIR if odd else LOAD_C64, bt, counts_xb, ny, [[rb] for rb in RB],
-                                [[(0, XB[i][0], counts_xb[i])] for i in range(W)], out_ext.owned(), _lib.F32, inverse=1, real_out=1)
+            _lib.check(lib.hd_conj_mirror_fill(bt.ptr, bt.pitch, bt.ny, ny, dev.stream_ptr()))
+        dem = self._exchange(plan, 1, LOAD_HPAIR if odd else LOAD_C64, bt, ex["I2"], inverse=1, real_out=1)
         del bt
         TRACE.mark("I2 cols + T4")
-        return out_ext
+        return dem
 
     # -- the whole chain on row bands (BASELINE.json configs[4]: one mosaic over the GPUs of a box) --------------------
     def conditioning_chain(self, srtm, groves_class, hsheds, groves_iterations=3, with_hydrology=True, keep_complete=False,

@@ -248,7 +248,8 @@ int hd_fft_band_pass(void* plan, int axis, int load, const void* in, int64_t in_
  * into the memory of the rank that owns it (peer pointers from hd_ipc_import), 256-byte row segments per warp over NVLink --
  * no send buffer, no NCCL call, no unpack copy.  Output row `orow` (a frequency / pixel index of the transposed axis) in
  * [row0, row1) of a segment lives at base[(orow - row0 + dst_row0) * pitch + column]; this rank's local row r lands at
- * column col_dst0[q] + (r - col_local0[q]).  The caller synchronises the ranks before (destinations free) and after. */
+ * column col_dst0[q] + (r - col_local0[q]).  The caller synchronises the ranks before (destinations free) and after.
+ * Workspace: hd_fft_band_workspace_bytes(nrows, n), as for hd_fft_band_pass. */
 #define HD_SCATTER_MAX_SEGS 16
 typedef struct { int64_t row0, row1; void* base; int64_t pitch; int64_t dst_row0; } hd_scatter_seg;
 typedef struct {

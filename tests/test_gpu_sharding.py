@@ -55,11 +55,14 @@ def test_banded_sinkfill_matches_oracle(world, ny):
     assert res[0][2] >= 2 and all(r[3] == 0 for r in res)
 
 
+@pytest.mark.parametrize("direct", ["1", "0"])
 @pytest.mark.parametrize("world,shape", [(2, (301, 333)), (3, (301, 333)), (2, (300, 334)), (3, (421, 300)), (4, (1300, 262))])
-def test_banded_detect_apply_fourier_is_bit_identical(world, shape):
+def test_banded_detect_apply_fourier_is_bit_identical(world, shape, direct, monkeypatch):
     """The stripe-removal stage on row bands (the same row transforms as on one GPU, transposes as all-to-alls,
     Hermitian completion in the K layout, banded peak detector): odd x odd takes the Hermitian inverse, the others the
-    complex one; every output cell must carry the single-GPU bits."""
+    complex one; every output cell must carry the single-GPU bits -- with the exchanges as peer-memory stores from the
+    transposes (direct) and as send / recv messages."""
+    monkeypatch.setenv("HD_BAND_DIRECT", direct)
     sc = SynthScene(*shape, 71)
     srtm = sc.srtm()
     daf = cf.DetectApplyFourier()

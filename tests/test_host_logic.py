@@ -11,7 +11,7 @@ import torch
 import torch.multiprocessing as mp
 
 import hydrodem_b200
-from hydrodem_b200 import sharding
+from hydrodem_b200 import _lib, sharding
 from hydrodem_b200.exceptions import (CenterCloseBorderError, HydroDEMException, NumpyArrayExpectedError,
                                       WindowSizeEvenError, WindowSizeHighError)
 from hydrodem_b200.filters import ComposedFilter, ComposedFilterResults, Filter, custom_filters as cf
@@ -180,6 +180,62 @@ def test_band_rejects_thin_bands_on_every_rank():
             return "refused"
         return "ok"
     assert sharding.ThreadComm.run(3, fn) == ["refused"] * 3
+
+
+@pytest.fixture(scope="module")
+def lib():
+    if not os.path.exists(_lib.LIB_PATH):
+        from hydrodem_b200.build import build
+        build()
+    return _lib.load()
+
+
+@pytest.mark.parametrize("shape", [(36000, 36000), (18000, 18000), (3601, 3601), (301, 333), (420, 333)])
+def test_fourier_exchanges_cover_every_cell_once(shape, lib):
+    """The four exchanges of the sharded Fourier stage on 1 ... 8 ranks (host geometry only): every cell the next step
+    reads from a destination buffer is written by exactly one (rank, local row, row of the transposed result), it
+    holds the row / column the next step takes it for, and every pass fits the limits of hd_scatter."""
+    ny, nx = shape
+    nh = nx // 2 + 1
+    odd = ny % 2 == 1 and nx % 2 == 1
+    n_out = {"F1": nh, "F2": ny, "I1": nx, "I2": ny}              # rows of the transposed result T of each pass
+    read_cols = {"F1": ny, "F2": nh, "I1": ny // 2 + 1 if odd else ny, "I2": nx}   # odd x odd: conj mirror fills the rest
+    for world in range(1, 9):
+        bounds = sharding.band_bounds(ny, world, 8)
+        KL, ex = sharding.fourier_exchanges(ny, nx, bounds)
+        assert [(k, e.dest) for k, e in ex.items()] == [("F1", "at"), ("F2", "half"), ("I1", "bt"), ("I2", "dem")]
+        # what rank j's local row k is before each pass: a y row, a kx column, a ky row (K layout), an x column
+        held = {"F1": [np.arange(a, b) for a, b in bounds]}
+        for name, nxt in (("F1", "F2"), ("F2", "I1"), ("I1", "I2"), ("I2", None)):
+            e = ex[name]
+            assert sum(b > a for r in e.ranges for a, b in r) <= _lib.HD_SCATTER_MAX_SEGS, (world, name)
+            assert all(len(segs) <= 2 for segs in e.colsegs), (world, name)
+            # rows: every row of T goes to exactly one place, so every buffer row receives exactly one row of T
+            hits = np.zeros(n_out[name], dtype=np.int64)
+            for r in e.ranges:
+                for a, b in r:
+                    assert 0 <= a <= b <= n_out[name]
+                    hits[a:b] += 1
+            assert (hits == 1).all(), (world, name)
+            # columns: rank i's local rows land once each, at the column of the row / frequency they hold
+            cols = np.zeros(e.cols, dtype=np.int64)
+            for i, segs in enumerate(e.colsegs):
+                nrows = max((l0 + ln for l0, _, ln in segs), default=0)
+                assert nrows == len(held[name][i]) or (name == "I1" and nrows < len(held[name][i]))
+                where = np.full(nrows, -1, dtype=np.int64)
+                for l0, c0, ln in segs:
+                    assert 0 <= l0 and 0 <= c0 and c0 + ln <= e.cols and (where[l0:l0 + ln] == -1).all()
+                    where[l0:l0 + ln] = np.arange(c0, c0 + ln)
+                    cols[c0:c0 + ln] += 1
+                np.testing.assert_array_equal(where, held[name][i][:nrows])
+            assert (cols[:read_cols[name]] == 1).all() and (cols[read_cols[name]:] == 0).all(), (world, name)
+            held[nxt] = [np.concatenate([np.arange(a, b) for a, b in r]) for r in e.ranges]
+        # the spectrum rows arrive in the K layout; I1 transforms all of them (only ky <= ny/2 on odd x odd);
+        # the DEM rows land on the owned rows of each band
+        for j, k in enumerate(KL):
+            np.testing.assert_array_equal(held["I1"][j], k["ky"])
+            assert max(l0 + ln for l0, _, ln in ex["I1"].colsegs[j]) == (k["nlo"] if odd else k["rows"])
+            np.testing.assert_array_equal(held[None][j], np.arange(*bounds[j]))
 
 
 def test_device_mosaic_is_cut_independent():
