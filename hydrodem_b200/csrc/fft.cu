@@ -557,16 +557,32 @@ __device__ __forceinline__ void mix_twiddles(float2 (&w)[R], const float2* __res
     }
 }
 
+// Group g = blk * stride + j.  Threads step through the groups FNT at a time, which moves (blk, j) on by the per-pass
+// constants (FNT / stride, FNT % stride): no division per group.  The padded slot of element q of a group is
+// padv(base, sh) + q * pst whenever that is exact, which holds for every pass of the planner's usual choices:
+//   stride a multiple of 2^sh:  (base + q stride) >> sh = (base >> sh) + q (stride >> sh),  pst = padv(stride, sh);
+//   stride 1, L a multiple of 2^sh and R <= 2^sh:  base = blk L, and base + q stays inside one padding period,  pst = 1.
+// Other passes (pst = 0) pad each index on its own.
 template <int R>
 __device__ __forceinline__ void mix_dif_pass(float2* s, int n, int L, const float2* __restrict__ tw, int sh)
 {
     const int stride = L / R, ngroups = n / R, tstep = n / L;
+    const int dblk = FNT / stride, dj = FNT - dblk * stride;
+    const int pmask = sh < 31 ? (1 << sh) - 1 : 0;
+    const int pst = (stride & pmask) == 0 ? padv(stride, sh)
+                  : (stride == 1 && (L & pmask) == 0 && R - 1 <= pmask) ? 1 : 0;
+    int blk = (int)threadIdx.x / stride, j = (int)threadIdx.x - blk * stride;
     for (int g = threadIdx.x; g < ngroups; g += FNT) {
-        const int blk = g / stride, j = g - blk * stride;
         const int base = blk * L + j;
         float2 x[R];
+        if (pst) {
+            const float2* p = s + padv(base, sh);
 #pragma unroll
-        for (int q = 0; q < R; ++q) x[q] = s[padv(base + q * stride, sh)];
+            for (int q = 0; q < R; ++q) x[q] = p[q * pst];
+        } else {
+#pragma unroll
+            for (int q = 0; q < R; ++q) x[q] = s[padv(base + q * stride, sh)];
+        }
         dft_fwd<R>(x);
         if (stride > 1) {
             float2 w[R];
@@ -574,8 +590,17 @@ __device__ __forceinline__ void mix_dif_pass(float2* s, int n, int L, const floa
 #pragma unroll
             for (int q = 1; q < R; ++q) x[q] = cmul(x[q], w[q]);
         }
+        if (pst) {
+            float2* p = s + padv(base, sh);
 #pragma unroll
-        for (int q = 0; q < R; ++q) s[padv(base + q * stride, sh)] = x[q];
+            for (int q = 0; q < R; ++q) p[q * pst] = x[q];
+        } else {
+#pragma unroll
+            for (int q = 0; q < R; ++q) s[padv(base + q * stride, sh)] = x[q];
+        }
+        blk += dblk;
+        j += dj;
+        if (j >= stride) { j -= stride; ++blk; }
     }
     __syncthreads();
 }
@@ -661,6 +686,17 @@ __device__ __forceinline__ float2 load_elem(const RowsArgs& a, int row, int col)
 //   transform CTA k1 transforms y_k1 (length n) on its own and stores X[k1 + n1 k2] at position k1 * n + k2.
 // Two cluster barriers per row: "all y have landed" and "my shared memory is free again" -- the second one is split
 // (arrive after the store phase, wait under the next row's first global loads).
+// Memory ordering of the two barriers:
+//   1. "All y have landed" (cluster_sync_all after the load stage) orders the DSMEM stores of every CTA before the
+//      shared-memory reads of the transform in the CTA that owns the memory: a writer-to-reader edge, so it is a
+//      release arrive and an acquire wait.
+//   2. "My shared memory is free" (cluster_arrive_relaxed after the store phase, waited for in long_row_load) only has
+//      to keep the peers' DSMEM stores of the next row from landing before this CTA's reads of the current row.  Every
+//      one of those reads has delivered its value into a register that the global store of the same iteration consumed
+//      before the __syncthreads() that precedes the arrive, so a later write cannot change what was read; and nothing
+//      in the cluster reads the global stores of the store phase (the next kernel does, ordered by the kernel
+//      boundary).  A release arrive would add nothing here but a MEMBAR.ALL.GPU that makes every thread wait for its
+//      global stores of the row to complete, so this arrive is relaxed.
 __device__ __forceinline__ uint32_t cluster_rank()
 {
     uint32_t r;
@@ -670,6 +706,10 @@ __device__ __forceinline__ uint32_t cluster_rank()
 __device__ __forceinline__ void cluster_arrive()
 {
     asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
+}
+__device__ __forceinline__ void cluster_arrive_relaxed()
+{
+    asm volatile("barrier.cluster.arrive.relaxed.aligned;" ::: "memory");
 }
 __device__ __forceinline__ void cluster_wait()
 {
@@ -692,10 +732,10 @@ __device__ __forceinline__ void dsmem_st(uint32_t addr, float2 v)
 // (and the Bluestein chirp), then y_k1[j] is stored into CTA k1's shared memory at slot(j) -- remote stores only, no
 // remote loads.  The cluster barrier that says "everybody is done with the previous row's shared memory" is waited for
 // after the first batch of global loads has been issued, i.e. under their latency.
-// (not inlined: with the seven n1 cases inlined side by side ptxas spills hundreds of bytes in every one of them)
+// Inlined: the kernel is instantiated per n1 (fft_rows_kernel's N1), so each instantiation holds one case.
 template <int N1, int LOAD, int ALG>
-__device__ __noinline__ void long_row_load(float2* s, int n, uint32_t rank, int row, const RowsArgs& a,
-                                           const float2* __restrict__ chirp, int padsh)
+__device__ __forceinline__ void long_row_load(float2* s, int n, uint32_t rank, int row, const RowsArgs& a,
+                                              const float2* __restrict__ chirp, int padsh)
 {
     constexpr bool BLUE = ALG == ALG_BLUESTEIN;
     const float2* __restrict__ wn2 = a.wn;
@@ -703,7 +743,11 @@ __device__ __noinline__ void long_row_load(float2* s, int n, uint32_t rank, int 
     auto slot = [&](int k) { return ALG == ALG_MIXED ? padv(k, padsh) : pad(k); };
     const int chunk = (n + N1 - 1) / N1;
     const int j_end = min(n, (int)(rank + 1) * chunk);
-    const uint32_t local = smem_u32(s);
+    // the shared::cluster address of this CTA's s in CTA k1; slot offsets are added to it (the window of one CTA is
+    // contiguous, so mapa(s + o, k1) = mapa(s, k1) + o)
+    uint32_t dst[N1];
+#pragma unroll
+    for (int k1 = 0; k1 < N1; ++k1) dst[k1] = dsmem_addr(smem_u32(s), (uint32_t)k1);
     // software pipelined: the global loads of the next j are issued right after the remote stores of this one
     int j = (int)rank * chunk + (int)threadIdx.x;
     bool live = j < j_end;
@@ -716,15 +760,15 @@ __device__ __noinline__ void long_row_load(float2* s, int n, uint32_t rank, int 
     while (live) {
         dft_fwd<N1>(x);
 #pragma unroll
-        for (int k1 = 1; k1 < N1; ++k1) x[k1] = cmul(x[k1], __ldg(&wn2[(size_t)k1 * n + j]));     // W_N^(j k1)
+        for (int k1 = 1; k1 < N1; ++k1) x[k1] = cmul(x[k1], __ldg(&wn2[k1 * n + j]));     // W_N^(j k1)
         if (BLUE) {
             const float2 c = __ldg(&chirp[j]);
 #pragma unroll
             for (int k1 = 0; k1 < N1; ++k1) x[k1] = cmul(x[k1], c);
         }
-        const uint32_t addr = local + (uint32_t)slot(j) * (uint32_t)sizeof(float2);
+        const uint32_t off = (uint32_t)slot(j) * (uint32_t)sizeof(float2);
 #pragma unroll
-        for (int k1 = 0; k1 < N1; ++k1) dsmem_st(dsmem_addr(addr, (uint32_t)k1), x[k1]);
+        for (int k1 = 0; k1 < N1; ++k1) dsmem_st(dst[k1] + off, x[k1]);
         j += FNT;
         live = j < j_end;
         if (live) {
@@ -734,11 +778,13 @@ __device__ __noinline__ void long_row_load(float2* s, int n, uint32_t rank, int 
     }
 }
 
-template <int LOAD, int ALG, bool LONG>
+// N1 = the row's outer factor a.n1 (1: the whole row is one transform; 2..8: long rows on a cluster of N1 CTAs)
+template <int LOAD, int ALG, int N1>
 __global__ void __launch_bounds__(FNT, 3) fft_rows_kernel(RowsArgs a, int n, int m, int log2m, PassPlan plan,
                                                        const float2* __restrict__ tw, const float2* __restrict__ chirp,
                                                        const float2* __restrict__ bhat, MixPlan mix)
 {
+    constexpr bool LONG = N1 > 1;
     constexpr bool BLUE = ALG == ALG_BLUESTEIN;
     constexpr bool MIXED = ALG == ALG_MIXED;
     extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -752,7 +798,7 @@ __global__ void __launch_bounds__(FNT, 3) fft_rows_kernel(RowsArgs a, int n, int
         return pad(log2m ? (int)(__brev((unsigned)k) >> (32 - log2m)) : 0);
     };
     const float scale = a.inverse ? 1.0f / (float)a.n_total : 1.0f;
-    const int n1 = LONG ? a.n1 : 1;
+    const int n1 = N1;
     const uint32_t crank = LONG ? cluster_rank() : 0u;
     const int nworkers = LONG ? (int)gridDim.x / n1 : (int)gridDim.x;          // clusters (LONG) or CTAs
     const int worker = LONG ? (int)blockIdx.x / n1 : (int)blockIdx.x;
@@ -762,24 +808,16 @@ __global__ void __launch_bounds__(FNT, 3) fft_rows_kernel(RowsArgs a, int n, int
     const bool hpair = (LOAD == LOAD_C64_HPAIR);
     const int nwork = (pair || hpair) ? (a.nrows + 1) / 2 : a.nrows;
     auto elem = [&](int row, int col) -> float2 { return load_elem<LOAD>(a, row, col); };
-    if (LONG) cluster_arrive();                         // "my shared memory is free" (matched by the wait in long_row_load)
+    if (LONG) cluster_arrive_relaxed();                 // "my shared memory is free" (matched by the wait in long_row_load)
     for (int item = worker; item < nwork; item += nworkers) {
         const int row = (pair || hpair) ? 2 * item : item;
         const int k1 = (int)crank;
         const bool has_b = pair && (row + 1 < a.nrows);
         // ---- load (+ chirp for Bluestein) ------------------------------------------------------------------------
-        if (LONG) {
+        if constexpr (LONG) {
             if (BLUE)                                   // zero tail of the Bluestein buffer (own shared memory)
                 for (int k = n + (int)threadIdx.x; k < m; k += FNT) s[in_slot(k)] = make_float2(0.f, 0.f);
-            switch (n1) {
-                case 2: long_row_load<2, LOAD, ALG>(s, n, crank, row, a, chirp, mix.padsh); break;
-                case 3: long_row_load<3, LOAD, ALG>(s, n, crank, row, a, chirp, mix.padsh); break;
-                case 4: long_row_load<4, LOAD, ALG>(s, n, crank, row, a, chirp, mix.padsh); break;
-                case 5: long_row_load<5, LOAD, ALG>(s, n, crank, row, a, chirp, mix.padsh); break;
-                case 6: long_row_load<6, LOAD, ALG>(s, n, crank, row, a, chirp, mix.padsh); break;
-                case 7: long_row_load<7, LOAD, ALG>(s, n, crank, row, a, chirp, mix.padsh); break;
-                default: long_row_load<8, LOAD, ALG>(s, n, crank, row, a, chirp, mix.padsh); break;
-            }
+            long_row_load<N1, LOAD, ALG>(s, n, crank, row, a, chirp, mix.padsh);
             cluster_sync_all();                         // every y_k1[j] of this row has landed
         } else {
             // batches of LB elements per thread: all global loads of a batch are issued before the first is used
@@ -864,7 +902,7 @@ __global__ void __launch_bounds__(FNT, 3) fft_rows_kernel(RowsArgs a, int n, int
             }
         }
         __syncthreads();
-        if (LONG) cluster_arrive();                     // this row is stored: my shared memory is free again
+        if (LONG) cluster_arrive_relaxed();             // this row is stored: my shared memory is free again
     }
     if (LONG) cluster_wait();                           // closes the last arrive; nobody writes to a CTA that has left
 }
@@ -1164,18 +1202,18 @@ int launch_rows(const Plan1D& p, const RowsArgs& a_in, int load, cudaStream_t s,
     for (int i = 0; i < p.nrad; ++i) rad8 |= (unsigned long long)p.rad[i] << (8 * i);
     MixPlan mix{p.nrad, rad8, p.padsh, p.d_pos};
     if (a.nrows < 1) return HD_OK;
-#define HD_ROWS_L(LOADV, ALGV, LONGV)                                                                     \
+#define HD_ROWS_L(LOADV, ALGV, N1V)                                                                     \
     {                                                                                                    \
-        auto kern = fft_rows_kernel<LOADV, ALGV, LONGV>;                                                 \
+        auto kern = fft_rows_kernel<LOADV, ALGV, N1V>;                                                   \
         HD_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));   \
-        const int nwork = ((LOADV == LOAD_REAL && !LONGV) || LOADV == LOAD_C64_HPAIR) ? (a.nrows + 1) / 2 : a.nrows; \
+        const int nwork = ((LOADV == LOAD_REAL && N1V == 1) || LOADV == LOAD_C64_HPAIR) ? (a.nrows + 1) / 2 : a.nrows; \
         cudaLaunchConfig_t cfg = {};                                                                     \
         cfg.blockDim = dim3(FNT);                                                                        \
         cfg.dynamicSmemBytes = smem;                                                                     \
         cfg.stream = s;                                                                                  \
         cudaLaunchAttribute attr[1];                                                                     \
         int workers = 1;                                                                                 \
-        if (LONGV) {                                                                                     \
+        if (N1V > 1) {                                                                                   \
             attr[0].id = cudaLaunchAttributeClusterDimension;                                            \
             attr[0].val.clusterDim.x = (unsigned)p.n1;                                                   \
             attr[0].val.clusterDim.y = 1;                                                                \
@@ -1192,15 +1230,23 @@ int launch_rows(const Plan1D& p, const RowsArgs& a_in, int load, cudaStream_t s,
         }                                                                                                \
         if (workers < 1) workers = 1;                                                                    \
         if (workers > nwork) workers = nwork;                                                            \
-        cfg.gridDim = dim3((unsigned)(workers * (LONGV ? p.n1 : 1)));                                    \
+        cfg.gridDim = dim3((unsigned)(workers * (N1V > 1 ? p.n1 : 1)));                                    \
         hd_prof_begin("fft_rows_kernel", s);                                                             \
         HD_CUDA_OK(cudaLaunchKernelEx(&cfg, kern, a, p.n, p.m, p.log2m, plan, (const float2*)p.d_tw,     \
                                       (const float2*)p.d_w, (const float2*)p.d_bhat, mix));              \
     }
 #define HD_ROWS(LOADV, ALGV)                                        \
     {                                                               \
-        if (p.n1 > 1) HD_ROWS_L(LOADV, ALGV, true)                  \
-        else HD_ROWS_L(LOADV, ALGV, false)                          \
+        switch (p.n1) {                                             \
+            case 1: HD_ROWS_L(LOADV, ALGV, 1) break;                \
+            case 2: HD_ROWS_L(LOADV, ALGV, 2) break;                \
+            case 3: HD_ROWS_L(LOADV, ALGV, 3) break;                \
+            case 4: HD_ROWS_L(LOADV, ALGV, 4) break;                \
+            case 5: HD_ROWS_L(LOADV, ALGV, 5) break;                \
+            case 6: HD_ROWS_L(LOADV, ALGV, 6) break;                \
+            case 7: HD_ROWS_L(LOADV, ALGV, 7) break;                \
+            default: HD_ROWS_L(LOADV, ALGV, 8) break;               \
+        }                                                           \
     }
     if (p.bluestein) {
         if (load == LOAD_REAL) HD_ROWS(LOAD_REAL, ALG_BLUESTEIN)
