@@ -96,6 +96,11 @@ SIGNATURES = {
     "hd_max_filter": (_i, [_p, _i64, _p, _i64, _i, _i64, _i64, _i, _p]),
     "hd_tidy_lagoons": (_i, [_p, _i64, _p, _i64, _i64, _i64, _p]),
     "hd_convolve3": (_i, [_p, _i64, _p, _i64, _i, _i64, _i64, ctypes.POINTER(_d), _d, _i, _p, _i64, _p]),
+    "hd_correlate": (_i, [_p, _i64, _p, _i64, _i, _i64, _i64, _i, ctypes.POINTER(_i), ctypes.POINTER(_i),
+                          ctypes.POINTER(_d), _d, _p]),
+    "hd_binary_morph_struct": (_i, [_p, _i, _i64, _p, _i64, _i64, _i64, _i, _i, ctypes.POINTER(_i), ctypes.POINTER(_i),
+                                    _i, _p, _p]),
+    "hd_max_filter_rect": (_i, [_p, _i64, _p, _i64, _i, _i64, _i64, _i, _i, _p, _i64, _p]),
 }
 
 

@@ -3,6 +3,8 @@
 //   hd_expand      ExpandFilter.apply                 custom_filters.py:102-125
 //   hd_binary_morph BinaryErosion / BinaryClosing     extension_filters.py:218-235, :276-293 (scipy.ndimage)
 //   hd_max_filter  GreyDilation(size=(s,s))           extension_filters.py:328-345 (scipy.ndimage.grey_dilation)
+//   hd_binary_morph_struct  the same with any structure up to 31x31, several steps per launch, changed flag
+//   hd_max_filter_rect      GreyDilation(size=(a, b)), any size 1 ... 255 per axis (van Herk / Gil-Werman)
 //
 // All three are HBM-bound: a 32x128 tile (+halo) is staged by TMA, thresholded to one bit per cell with
 // warp ballots, and the window logic runs on 32-cell words (funnel shifts / ORs), a few hundred word
@@ -414,6 +416,172 @@ __global__ void __launch_bounds__(TL_NT) tidy_lagoons_kernel(const __grid_consta
     });
 }
 
+// ------------------------------------------------------------------------------------------------ any structure
+// scipy.ndimage.binary_erosion / binary_dilation with a structure up to 31 x 31, border_value = 0.  The host passes the
+// structure's True cells as offsets (dy, dx) from the output cell, reflected and origin-shifted for a dilation.  Erosion
+// is the AND, dilation the OR of the bit rows shifted by each offset; cells outside the raster are False before and after
+// every step.  `nsteps` repetitions run in the tile (halo = nsteps x reach); `changed` (may be NULL) is set when the
+// result differs from the input anywhere.
+constexpr int MS_MAX_REACH = 15;
+constexpr int MS_MAX_TAPS = (2 * MS_MAX_REACH + 1) * (2 * MS_MAX_REACH + 1);
+constexpr int MS_MAX_IN_H = TH + 2 * MS_MAX_REACH;                    // 62
+constexpr uint32_t MS_STAGE = MS_MAX_IN_H * MAX_IN_W * 4;              // f32 box of 62 x 160
+
+struct MorphTaps {
+    int ntaps;
+    signed char dy[MS_MAX_TAPS], dx[MS_MAX_TAPS];
+};
+
+// bits of columns 32k + dx ... 32k + 31 + dx of a bit row (columns outside the row's NWORD words read as 0)
+__device__ __forceinline__ uint32_t shifted_word(const uint32_t* row, int k, int dx)
+{
+    if (dx >= 0) return __funnelshift_rc(row[k], k + 1 < NWORD ? row[k + 1] : 0u, (uint32_t)dx);
+    return __funnelshift_lc(k > 0 ? row[k - 1] : 0u, row[k], (uint32_t)-dx);
+}
+
+template <typename InT>
+__global__ void __launch_bounds__(NT) morph_struct_kernel(const __grid_constant__ CUtensorMap tm_in, uint8_t* __restrict__ out,
+                                                          int64_t out_pitch, int64_t ny, int64_t nx,
+                                                          const __grid_constant__ MorphTaps p, int dilate, int nsteps, int hy,
+                                                          int hx, int in_w, int in_h, int tiles_x, int ntiles,
+                                                          int* __restrict__ changed)
+{
+    extern __shared__ __align__(128) unsigned char smem[];
+    __shared__ uint64_t bars[2];
+    __shared__ uint32_t src[MS_MAX_IN_H * NWORD], bufA[MS_MAX_IN_H * NWORD], bufB[MS_MAX_IN_H * NWORD];
+    __shared__ uint32_t res[TH * 4];
+    const TilePlane planes[1] = {{&tm_in, 0u, (uint32_t)(in_w * in_h * sizeof(InT)), hx, hy}};
+    tile_loop<1>(smem, MS_STAGE, bars, planes, TW, TH, tiles_x, ntiles, [&](unsigned char* st, int ty0, int tx0) {
+        // scipy: non-zero elements are True (NaN != 0 is true); cells outside the raster arrive as 0 = border_value
+        tile_to_bits<InT>(reinterpret_cast<const InT*>(st), in_w, in_h, src, [](InT v) { return v != (InT)0; });
+        __syncthreads();
+        const uint32_t* cur = src;
+        for (int s = 0; s < nsteps; ++s) {
+            uint32_t* nxt = (s & 1) ? bufB : bufA;
+            for (int t = threadIdx.x; t < in_h * NWORD; t += NT) {
+                const int r = t / NWORD, k = t - r * NWORD;
+                uint32_t v = dilate ? 0u : 0xffffffffu;
+                for (int j = 0; j < p.ntaps; ++j) {
+                    const int rr = r + p.dy[j];
+                    const uint32_t w = (rr >= 0 && rr < in_h) ? shifted_word(cur + rr * NWORD, k, p.dx[j]) : 0u;
+                    v = dilate ? (v | w) : (v & w);
+                }
+                // the result only exists on the raster: outside stays border_value = 0
+                const int64_t gy = (int64_t)ty0 - hy + r;
+                uint32_t m = 0u;
+                if (gy >= 0 && gy < ny) {
+                    const int64_t gx0 = (int64_t)tx0 - hx + 32 * k;      // global x of bit 0
+                    const int64_t lo = gx0 < 0 ? -gx0 : 0;
+                    const int64_t hi = (nx - gx0) < 32 ? (nx - gx0) : 32;   // exclusive
+                    if (hi > lo) m = (hi - lo >= 32 ? 0xffffffffu : ((1u << (hi - lo)) - 1u)) << lo;
+                }
+                nxt[t] = v & m;
+            }
+            __syncthreads();
+            cur = nxt;
+        }
+        if (threadIdx.x < TH * 4) {
+            const int ro = threadIdx.x >> 2, k = threadIdx.x & 3;
+            const uint32_t w = (uint32_t)(win64(cur + (ro + hy) * NWORD, k) >> hx);
+            res[threadIdx.x] = w;
+            // both words are 0 on cells outside the raster
+            if (changed && w != (uint32_t)(win64(src + (ro + hy) * NWORD, k) >> hx)) atomicOr(changed, 1);
+        }
+        __syncthreads();
+        write_bits<uint8_t>(res, out, out_pitch, ty0, tx0, ny, nx, 0);
+    });
+}
+
+// ------------------------------------------------------------------------------------------------ rectangular max
+// One axis of scipy.ndimage.grey_dilation(size=(a, b)), mode='reflect' (any distance: periodic), as van Herk / Gil-Werman:
+// the extended segment is cut into blocks of k cells; h = running max from each cell to the end of its block (backward),
+// g = running max from the block start (forward); window [j, j + k - 1] = max(h[j], g[j + k - 1]).  Three maxima per cell
+// for any k.  A CTA takes 32 lines x SG outputs; shared memory holds [position][line] with a 33-line pitch, so loads
+// along either axis and the per-line scans (one lane per line) are conflict free.  NaN cells are skipped (fmax).
+constexpr int ML_LINES = 32, ML_LP = ML_LINES + 1;
+template <typename T> constexpr int ml_seg() { return sizeof(T) == 4 ? 256 : 128; }
+
+template <typename T, int AXIS>   // AXIS 0: along columns (window rows), 1: along rows
+__global__ void __launch_bounds__(NT) maxline_kernel(const T* __restrict__ in, int64_t in_pitch, T* __restrict__ out,
+                                                     int64_t out_pitch, int64_t ny, int64_t nx, int k, int lo)
+{
+    constexpr int SG = ml_seg<T>();
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    const int E = SG + k - 1;
+    T* e = reinterpret_cast<T*>(smem_raw);                    // [E][ML_LP] the extended segment
+    T* h = e + (size_t)E * ML_LP;                             // [E][ML_LP] backward maxima, then the result
+    const int64_t n_along = AXIS == 0 ? ny : nx, n_lines = AXIS == 0 ? nx : ny;
+    const int64_t segs = (n_along + SG - 1) / SG, lgroups = (n_lines + ML_LINES - 1) / ML_LINES;
+    const int64_t ntiles = segs * lgroups;
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    for (int64_t tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
+        const int64_t a0 = (tile % segs) * SG, l0 = (tile / segs) * ML_LINES;
+        for (int idx = threadIdx.x; idx < E * ML_LINES; idx += NT) {
+            const int p = AXIS == 0 ? idx / ML_LINES : idx % E, l = AXIS == 0 ? idx % ML_LINES : idx / E;
+            const int64_t gl = l0 + l, raw = a0 - lo + p;
+            const int64_t ga = (raw >= 0 && raw < n_along) ? raw : reflect_periodic_idx(raw, n_along);
+            if (gl < n_lines) e[p * ML_LP + l] = AXIS == 0 ? in[ga * in_pitch + gl] : in[gl * in_pitch + ga];
+        }
+        __syncthreads();
+        const int nb = (E + k - 1) / k;
+        for (int b = warp; b * k < SG; b += NT / 32) {       // h over the blocks that hold outputs
+            const int j0 = b * k, j1 = min(E, j0 + k) - 1;
+            T m = e[j1 * ML_LP + lane];
+            h[j1 * ML_LP + lane] = m;
+            for (int j = j1 - 1; j >= j0; --j) {
+                m = tmax<T>(m, e[j * ML_LP + lane]);
+                h[j * ML_LP + lane] = m;
+            }
+        }
+        __syncthreads();
+        for (int b = warp; b < nb; b += NT / 32) {            // g, combined into h at the window's first cell
+            const int i0 = b * k, i1 = min(E, i0 + k);
+            T m = e[i0 * ML_LP + lane];
+            for (int i = i0; i < i1; ++i) {
+                m = tmax<T>(m, e[i * ML_LP + lane]);
+                const int j = i - k + 1;
+                if (j >= 0 && j < SG) h[j * ML_LP + lane] = tmax<T>(h[j * ML_LP + lane], m);
+            }
+        }
+        __syncthreads();
+        const int n_out = (int)min((int64_t)SG, n_along - a0);
+        for (int idx = threadIdx.x; idx < SG * ML_LINES; idx += NT) {
+            const int p = AXIS == 0 ? idx / ML_LINES : idx % SG, l = AXIS == 0 ? idx % ML_LINES : idx / SG;
+            const int64_t gl = l0 + l;
+            if (p >= n_out || gl >= n_lines) continue;
+            const T v = h[p * ML_LP + l];
+            if (AXIS == 0) out[(a0 + p) * out_pitch + gl] = v; else out[gl * out_pitch + a0 + p] = v;
+        }
+        __syncthreads();
+    }
+}
+
+template <typename T>
+int launch_max_rect(const void* in, int64_t in_pitch, void* out, int64_t out_pitch, int64_t ny, int64_t nx, int size_y,
+                    int size_x, void* workspace, cudaStream_t s)
+{
+    constexpr int SG = ml_seg<T>();
+    // grey_dilation: origin -1 on an even axis, so the window of output i is [i - (k/2 - 1), i + k/2]
+    auto lo_of = [](int k) { return k / 2 - (k % 2 == 0 ? 1 : 0); };
+    const size_t smem_y = 2 * (size_t)(SG + size_y - 1) * ML_LP * sizeof(T), smem_x = 2 * (size_t)(SG + size_x - 1) * ML_LP * sizeof(T);
+    const int tiles_y = hd_cdiv(ny, SG) * hd_cdiv(nx, ML_LINES), tiles_x = hd_cdiv(nx, SG) * hd_cdiv(ny, ML_LINES);
+    const int per_sm = sizeof(T) == 4 ? 2 : 1;
+    T* ws = (T*)workspace;                                    // dense ny x nx
+    HD_CUDA_OK(cudaFuncSetAttribute(maxline_kernel<T, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_y));
+    HD_CUDA_OK(cudaFuncSetAttribute(maxline_kernel<T, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_x));
+    hd_prof_begin("maxline_kernel", s);
+    maxline_kernel<T, 0><<<grid_for(tiles_y, per_sm), NT, smem_y, s>>>((const T*)in, in_pitch, ws, nx, ny, nx, size_y,
+                                                                       lo_of(size_y));
+    HD_LAUNCH_CHECK();
+    hd_count_launch();
+    hd_prof_begin("maxline_kernel", s);
+    maxline_kernel<T, 1><<<grid_for(tiles_x, per_sm), NT, smem_x, s>>>(ws, nx, (T*)out, out_pitch, ny, nx, size_x,
+                                                                       lo_of(size_x));
+    HD_LAUNCH_CHECK();
+    hd_count_launch();
+    return HD_OK;
+}
+
 template <typename InT, typename OutT>
 int launch_expand(const CUtensorMap& tm, void* out, int64_t out_pitch, int64_t ny, int64_t nx, int h, int in_w, int in_h,
                   cudaStream_t stream, const float* select = nullptr, int64_t sel_pitch = 0)
@@ -560,6 +728,64 @@ extern "C" int hd_max_filter(const void* in, int64_t in_pitch, void* out, int64_
     HD_LAUNCH_CHECK();
     hd_count_launch();
     return HD_OK;
+}
+
+extern "C" int hd_binary_morph_struct(const void* in, int in_dtype, int64_t in_pitch, void* out, int64_t out_pitch,
+                                      int64_t ny, int64_t nx, int dilate, int ntaps, const int* tap_dy, const int* tap_dx,
+                                      int iterations, int* changed, void* stream)
+{
+    if (!in || !out || (ntaps > 0 && (!tap_dy || !tap_dx))) return HD_ERR_NULL;
+    if (ny < 1 || nx < 1 || in_pitch < nx || out_pitch < nx || ntaps < 0 || iterations < 1) return HD_ERR_ARG;
+    if (in_dtype != HD_U8 && in_dtype != HD_F32) return HD_ERR_UNSUPPORTED;
+    if (ntaps > MS_MAX_TAPS) return HD_ERR_UNSUPPORTED;
+    MorphTaps p;
+    p.ntaps = ntaps;
+    int ry = 0, rx = 0;
+    for (int t = 0; t < ntaps; ++t) {
+        const int ay = tap_dy[t] < 0 ? -tap_dy[t] : tap_dy[t], ax = tap_dx[t] < 0 ? -tap_dx[t] : tap_dx[t];
+        if (ay > MS_MAX_REACH || ax > MS_MAX_REACH) return HD_ERR_UNSUPPORTED;
+        ry = ay > ry ? ay : ry;
+        rx = ax > rx ? ax : rx;
+        p.dy[t] = (signed char)tap_dy[t];
+        p.dx[t] = (signed char)tap_dx[t];
+    }
+    if (iterations * ry > MS_MAX_REACH || iterations * rx > MS_MAX_REACH) return HD_ERR_UNSUPPORTED;
+    const int hy = iterations * ry, hx = hd_halo_x(iterations * rx, (int)hd_dtype_size(in_dtype));
+    const int in_w = TW + 2 * hx, in_h = TH + 2 * hy;
+    CUtensorMap tm;
+    if (int e = hd_make_tmap_2d(&tm, in, in_dtype, ny, nx, in_pitch, in_w, in_h, false)) return e;
+    const int tiles_x = hd_cdiv(nx, TW), tiles_y = hd_cdiv(ny, TH), ntiles = tiles_x * tiles_y;
+    const size_t smem = 2 * (size_t)MS_STAGE;
+    cudaStream_t s = (cudaStream_t)stream;
+    if (changed) HD_CUDA_OK(cudaMemsetAsync(changed, 0, sizeof(int), s));
+    if (in_dtype == HD_F32) {
+        HD_CUDA_OK(cudaFuncSetAttribute(morph_struct_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        hd_prof_begin("morph_struct_kernel", s);
+        morph_struct_kernel<float><<<grid_for(ntiles, 2), NT, smem, s>>>(tm, (uint8_t*)out, out_pitch, ny, nx, p, dilate != 0,
+                                                                        iterations, hy, hx, in_w, in_h, tiles_x, ntiles, changed);
+    } else {
+        HD_CUDA_OK(cudaFuncSetAttribute(morph_struct_kernel<uint8_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        hd_prof_begin("morph_struct_kernel", s);
+        morph_struct_kernel<uint8_t><<<grid_for(ntiles, 2), NT, smem, s>>>(tm, (uint8_t*)out, out_pitch, ny, nx, p, dilate != 0,
+                                                                          iterations, hy, hx, in_w, in_h, tiles_x, ntiles,
+                                                                          changed);
+    }
+    HD_LAUNCH_CHECK();
+    hd_count_launch();
+    return HD_OK;
+}
+
+extern "C" int hd_max_filter_rect(const void* in, int64_t in_pitch, void* out, int64_t out_pitch, int dtype, int64_t ny,
+                                  int64_t nx, int size_y, int size_x, void* workspace, int64_t workspace_bytes, void* stream)
+{
+    if (!in || !out || !workspace) return HD_ERR_NULL;
+    if (ny < 1 || nx < 1 || in_pitch < nx || out_pitch < nx || size_y < 1 || size_x < 1) return HD_ERR_ARG;
+    if (dtype != HD_F32 && dtype != HD_F64) return HD_ERR_UNSUPPORTED;
+    if (size_y > 255 || size_x > 255) return HD_ERR_UNSUPPORTED;
+    if (workspace_bytes < ny * nx * (int64_t)hd_dtype_size(dtype)) return HD_ERR_WORKSPACE;
+    cudaStream_t s = (cudaStream_t)stream;
+    if (dtype == HD_F32) return launch_max_rect<float>(in, in_pitch, out, out_pitch, ny, nx, size_y, size_x, workspace, s);
+    return launch_max_rect<double>(in, in_pitch, out, out_pitch, ny, nx, size_y, size_x, workspace, s);
 }
 
 // TidyingLagoons.apply (custom_filters.py:587-610) in one kernel: majority (F32) -> lagoon values (F32).

@@ -3,6 +3,7 @@
 //   hd_nanfix     CorrectNANValues.apply   custom_filters.py:286-317   (bit-exact float32 mean, numpy order)
 //   hd_isolated   IsolatedPoints.apply     custom_filters.py:345-366
 //   hd_convolve3  Convolve.apply + Around  extension_filters.py:166-184, :113-130 (PostProcessingFinal)
+//   hd_correlate  Convolve.apply          extension_filters.py:166-184, any weights up to 31x31
 //
 // HBM-bound: 4 B read + 4 B written per cell (8 + 8 for float64 rasters).  A 32x128 tile with a one-cell
 // halo is staged by TMA; each thread produces 4 consecutive cells of 4 rows and stores them as one
@@ -184,6 +185,57 @@ __global__ void __launch_bounds__(NT) conv3_kernel(const __grid_constant__ CUten
     });
 }
 
+// ---- Convolve with any weights up to 31 x 31 (reflect) ----------------------------------------------------------------
+// The host hands over NI_Correlate's footprint as a tap list: offsets (dy, dx) from the output cell, already flipped and
+// origin-shifted for a convolution, with the weights |w| <= DBL_EPSILON left out, in the order the sum runs.  The list
+// lives in kernel-parameter (constant) memory: every thread reads the same tap at the same time.
+constexpr int CORR_MAX_REACH = 15;                       // 31 x 31 weights
+constexpr int CORR_MAX_TAPS = (2 * CORR_MAX_REACH + 1) * (2 * CORR_MAX_REACH + 1);
+constexpr int CORR_ROWS = TH * TW / NT;                  // output cells per thread, one column, every other row
+
+struct CorrTaps {
+    int ntaps;
+    int off[CORR_MAX_TAPS];       // (hy + dy) * in_w + hx + dx: staged-box offset of the tap from the output cell's (ro, co)
+    double w[CORR_MAX_TAPS];
+};
+
+template <typename T>
+__global__ void __launch_bounds__(NT) correlate_kernel(const __grid_constant__ CUtensorMap tm_in, T* __restrict__ out,
+                                                       int64_t out_pitch, int64_t ny, int64_t nx,
+                                                       const __grid_constant__ CorrTaps p, double divisor, int hy, int hx,
+                                                       int in_w, int in_h, int tiles_x, int ntiles)
+{
+    extern __shared__ __align__(128) unsigned char smem[];
+    __shared__ uint64_t bars[2];
+    const uint32_t stage_bytes = (uint32_t)((in_w * in_h * sizeof(T) + 127) / 128 * 128);
+    const TilePlane planes[1] = {{&tm_in, 0u, (uint32_t)(in_w * in_h * sizeof(T)), hx, hy}};
+    // lanes take consecutive columns (conflict-free shared-memory reads); rows rg, rg + 2, ... give each thread
+    // CORR_ROWS independent accumulators for one weight read
+    const int co = threadIdx.x % TW, rg = threadIdx.x / TW;
+    constexpr int RSTEP = NT / TW;
+    tile_loop<1>(smem, stage_bytes, bars, planes, TW, TH, tiles_x, ntiles, [&](unsigned char* st, int ty0, int tx0) {
+        T* tile = reinterpret_cast<T*>(st);
+        patch_reflect<T, true>(tile, in_w, in_h, ty0 - hy, tx0 - hx, ny, nx);
+        const T* base = tile + rg * in_w + co;
+        double acc[CORR_ROWS];
+#pragma unroll
+        for (int i = 0; i < CORR_ROWS; ++i) acc[i] = 0.0;     // NI_Correlate: tmp = 0.0; tmp += in * w, footprint order
+        for (int t = 0; t < p.ntaps; ++t) {
+            const double w = p.w[t];
+            const T* q = base + p.off[t];
+#pragma unroll
+            for (int i = 0; i < CORR_ROWS; ++i) acc[i] = __dadd_rn(acc[i], __dmul_rn((double)q[i * RSTEP * in_w], w));
+        }
+        const int64_t x = tx0 + co;
+        if (x < nx) {
+#pragma unroll
+            for (int i = 0; i < CORR_ROWS; ++i) {
+                const int64_t y = ty0 + rg + i * RSTEP;
+                if (y < ny) out[y * out_pitch + x] = div_round<T>((T)acc[i], divisor, 0);   // cast, then / weights.size
+            }
+        }
+    });
+}
 
 // ---- _prepare_final_terms + the three-term sum + PostProcessingFinal in ONE pass (no rivers) ----------------------------
 // hydro_dem_process.py:60-91, :148-149 with rivers = 0:  complete = srtm * (1 - mask) + lagoon_values + hsheds * 0,
@@ -328,6 +380,51 @@ extern "C" int hd_convolve3(const void* in, int64_t in_pitch, void* out, int64_t
         hd_prof_begin("conv3_kernel", s);
         conv3_kernel<double><<<grid_for(ntiles, 3), NT, smem, s>>>(tm, (double*)out, out_pitch, (float*)out32, out32_pitch, ny, nx,
                                                                   p, in_w, tiles_x, ntiles);
+    }
+    HD_LAUNCH_CHECK();
+    hd_count_launch();
+    return HD_OK;
+}
+
+extern "C" int hd_correlate(const void* in, int64_t in_pitch, void* out, int64_t out_pitch, int dtype, int64_t ny,
+                            int64_t nx, int ntaps, const int* tap_dy, const int* tap_dx, const double* tap_w, double divisor,
+                            void* stream)
+{
+    if (!in || !out || (ntaps > 0 && (!tap_dy || !tap_dx || !tap_w))) return HD_ERR_NULL;
+    if (ny < 1 || nx < 1 || in_pitch < nx || out_pitch < nx || ntaps < 0) return HD_ERR_ARG;
+    if (dtype != HD_F32 && dtype != HD_F64) return HD_ERR_UNSUPPORTED;
+    if (ntaps > CORR_MAX_TAPS) return HD_ERR_UNSUPPORTED;
+    int ry = 0, rx = 0;
+    for (int t = 0; t < ntaps; ++t) {
+        const int ay = tap_dy[t] < 0 ? -tap_dy[t] : tap_dy[t], ax = tap_dx[t] < 0 ? -tap_dx[t] : tap_dx[t];
+        if (ay > CORR_MAX_REACH || ax > CORR_MAX_REACH) return HD_ERR_UNSUPPORTED;
+        ry = ay > ry ? ay : ry;
+        rx = ax > rx ? ax : rx;
+    }
+    const size_t es = hd_dtype_size(dtype);
+    const int hx = hd_halo_x(rx, (int)es), in_w = TW + 2 * hx, in_h = TH + 2 * ry;
+    static thread_local CorrTaps q;                           // 11.5 KB: kept off the caller's stack
+    static_assert(sizeof(CorrTaps) <= 32000, "kernel parameters are limited to 32 KB");
+    q.ntaps = ntaps;
+    for (int t = 0; t < ntaps; ++t) {
+        q.off[t] = (ry + tap_dy[t]) * in_w + hx + tap_dx[t];
+        q.w[t] = tap_w[t];
+    }
+    CUtensorMap tm;
+    if (int e = hd_make_tmap_2d(&tm, in, dtype, ny, nx, in_pitch, in_w, in_h, false)) return e;
+    const int tiles_x = hd_cdiv(nx, TW), tiles_y = hd_cdiv(ny, TH), ntiles = tiles_x * tiles_y;
+    const size_t smem = 2 * ((in_w * in_h * es + 127) / 128 * 128);
+    cudaStream_t s = (cudaStream_t)stream;
+    if (dtype == HD_F32) {
+        HD_CUDA_OK(cudaFuncSetAttribute(correlate_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        hd_prof_begin("correlate_kernel", s);
+        correlate_kernel<float><<<grid_for(ntiles, 2), NT, smem, s>>>(tm, (float*)out, out_pitch, ny, nx, q, divisor, ry, hx,
+                                                                     in_w, in_h, tiles_x, ntiles);
+    } else {
+        HD_CUDA_OK(cudaFuncSetAttribute(correlate_kernel<double>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        hd_prof_begin("correlate_kernel", s);
+        correlate_kernel<double><<<grid_for(ntiles, 1), NT, smem, s>>>(tm, (double*)out, out_pitch, ny, nx, q, divisor, ry, hx,
+                                                                      in_w, in_h, tiles_x, ntiles);
     }
     HD_LAUNCH_CHECK();
     hd_count_launch();

@@ -105,7 +105,18 @@ __device__ __forceinline__ int reflect_idx(int64_t i, int64_t n)
     return (int)i;
 }
 
-template <typename T>
+// mode='reflect' for any distance from the raster (d c b a | a b c d | d c b a | a b ...): the extension repeats with
+// period 2n, so windows wider than the raster wrap as often as they need.  reflect_idx is its first period only.
+__device__ __forceinline__ int reflect_periodic_idx(int64_t i, int64_t n)
+{
+    int64_t m = i % (2 * n);
+    if (m < 0) m += 2 * n;
+    return (int)(m < n ? m : 2 * n - 1 - m);
+}
+
+// PERIODIC = false: one reflection (halo <= raster size); true: reflect_periodic_idx.  Every cell outside the raster is
+// copied from a cell inside it, and that cell lies in the staged box whenever an output of the tile needs it.
+template <typename T, bool PERIODIC = false>
 __device__ __forceinline__ void patch_reflect(T* tile, int in_w, int in_h, int gy0, int gx0, int64_t ny, int64_t nx)
 {
     const bool touches = gy0 < 0 || gx0 < 0 || gy0 + in_h > ny || gx0 + in_w > nx;
@@ -114,7 +125,8 @@ __device__ __forceinline__ void patch_reflect(T* tile, int in_w, int in_h, int g
         const int r = t / in_w, c = t - r * in_w;
         const int64_t gy = gy0 + r, gx = gx0 + c;
         if (gy >= 0 && gy < ny && gx >= 0 && gx < nx) continue;
-        const int sy = reflect_idx(gy, ny) - gy0, sx = reflect_idx(gx, nx) - gx0;
+        const int sy = (PERIODIC ? reflect_periodic_idx(gy, ny) : reflect_idx(gy, ny)) - gy0;
+        const int sx = (PERIODIC ? reflect_periodic_idx(gx, nx) : reflect_idx(gx, nx)) - gx0;
         if (sy >= 0 && sy < in_h && sx >= 0 && sx < in_w) tile[t] = tile[sy * in_w + sx];
     }
     __syncthreads();

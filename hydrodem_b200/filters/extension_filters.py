@@ -7,10 +7,11 @@ include/hydrodem_b200.h for the contract of each entry point).
 """
 import copy
 import ctypes
+import operator
 
 import numpy as np
 
-from . import DeviceFilter
+from . import DeviceFilter, Filter
 from .. import _lib, device as dev
 from ..exceptions import DeviceError
 from .simple_filters import _operand
@@ -53,23 +54,127 @@ class Around(DeviceFilter):
         return dev.elementwise(_lib.OP_RINT, raster, None, 0.0, out)
 
 
-class Convolve(DeviceFilter):
+# ---- general footprints: host-side plans --------------------------------------------------------------------------
+# scipy.ndimage puts the centre of an axis of length k at k // 2 + origin, so footprint index j sits at offset
+# j - (k // 2 + origin) from the output cell.  A convolution, a binary dilation and grey_dilation reverse the footprint
+# and turn origin 0 into -1 on an axis of even length (scipy's _correlate_or_convolve, binary_dilation, grey_dilation).
+MAX_FOOTPRINT = 31          # Convolve weights and BinaryClosing structures, per axis
+MAX_GREY_SIZE = 255         # GreyDilation size, per axis
+DBL_EPSILON = np.finfo(np.float64).eps
+MORPH_STEPS_PER_LAUNCH = 8  # hd_binary_morph's cap for erosions with the cross
+STABLE_STEPS_PER_LAUNCH = 15  # cross erosions per hd_binary_morph_struct launch when iterating until stable
+STABLE_LAUNCHES_PER_READ = 8  # launches between two host reads of their changed flags
+_CROSS = np.array([[0, 1, 0], [1, 1, 1], [0, 1, 0]], dtype=bool)
+
+
+def _centre(k, reversed_):
+    return k // 2 + (-1 if reversed_ and k % 2 == 0 else 0)
+
+
+def _offsets(mask, reversed_):
+    """(dy, dx) of the True cells of a 2-D footprint, row-major; `reversed_` flips it with the even-axis origin shift."""
+    if reversed_:
+        mask = mask[::-1, ::-1]
+    cy, cx = _centre(mask.shape[0], reversed_), _centre(mask.shape[1], reversed_)
+    iy, ix = np.nonzero(mask)                                           # row-major
+    return (iy - cy).astype(np.int32), (ix - cx).astype(np.int32)
+
+
+def _footprint_2d(a, what):
+    if a.ndim != 2:
+        raise DeviceError(f"{what} must be 2-D like the raster (got shape {a.shape})")
+    if a.size == 0:
+        raise DeviceError(f"{what} must not be empty (got shape {a.shape})")
+    if max(a.shape) > MAX_FOOTPRINT:
+        raise DeviceError(f"{what}: at most {MAX_FOOTPRINT}x{MAX_FOOTPRINT} on the device (got {a.shape})")
+
+
+def convolve_taps(weights):
+    """NI_Correlate's footprint of scipy.ndimage.convolve(image, weights) as (dy, dx, w) in summation order: the flipped
+    weights, origin -1 on even axes, entries with |w| <= DBL_EPSILON left out (a NaN weight too: its |w| > eps is false)."""
+    w = np.asarray(weights, dtype=np.float64)
+    _footprint_2d(w, "Convolve weights")
+    with np.errstate(invalid="ignore"):
+        keep = np.abs(w) > DBL_EPSILON
+    dy, dx = _offsets(keep, reversed_=True)
+    return dy, dx, w[::-1, ::-1][keep[::-1, ::-1]]
+
+
+def closing_taps(structure):
+    """binary_closing(structure): (dilation taps, erosion taps), each (dy, dx).  None = the cross."""
+    s = _CROSS if structure is None else np.asarray(structure)
+    _footprint_2d(s, "BinaryClosing structure")
+    s = s.astype(bool)                                                  # non-zero (NaN included) is True
+    return _offsets(s, reversed_=True), _offsets(s, reversed_=False)
+
+
+def grey_sizes(size):
+    """(a, b) of grey_dilation(size=...): an int for both axes or a pair, each 1 ... MAX_GREY_SIZE."""
+    pair = (size, size) if np.ndim(size) == 0 else tuple(np.asarray(size).ravel())
+    if np.ndim(size) > 1 or len(pair) != 2:
+        raise DeviceError(f"GreyDilation: size must be an int or a pair (got {size!r})")
+    try:
+        pair = tuple(operator.index(s) for s in pair)
+    except TypeError:
+        raise DeviceError(f"GreyDilation: sizes must be integers (got {size!r})") from None
+    for s in pair:
+        if s < 1:
+            raise DeviceError(f"GreyDilation: sizes must be >= 1 (got {size!r})")
+        if s > MAX_GREY_SIZE:
+            raise DeviceError(f"GreyDilation: sizes up to {MAX_GREY_SIZE} on the device (got {size!r})")
+    return pair
+
+
+def _int_array(v):
+    v = np.ascontiguousarray(v, dtype=np.int32)
+    return v, v.ctypes.data_as(ctypes.POINTER(ctypes.c_int))
+
+
+class _CheckedFilter(DeviceFilter):
+    """A filter whose arguments are validated on the host (``plan``) before the raster goes to the device."""
+
+    def plan(self, shape):
+        raise NotImplementedError
+
+    def apply(self, image_to_filter):
+        Filter.apply(self, image_to_filter)
+        self.plan(np.shape(image_to_filter))
+        return DeviceFilter.apply(self, image_to_filter)
+
+
+class Convolve(_CheckedFilter):
     """``scipy.ndimage.convolve(image, weights) / weights.size`` with the default
-    mode='reflect' (extension_filters.py:133-184).  3x3 weights only (the
-    pipeline uses ones((3, 3)))."""
+    mode='reflect' (extension_filters.py:133-184).  3x3 weights (the pipeline's ones((3, 3))) run on
+    hd_convolve3; any other 2-D weights up to 31x31 on hd_correlate."""
 
     def __init__(self, weights=np.ones((3, 3))):
         self.weights = weights
 
+    def plan(self, shape):
+        """("conv3", None) or ("correlate", (dy, dx, w))."""
+        w = np.asarray(self.weights, dtype=np.float64)
+        if w.shape == (3, 3):
+            return "conv3", None
+        return "correlate", convolve_taps(w)
+
     def run_device(self, raster, do_round=False, copy32=None):
         """``copy32``: optional F32 device raster that receives a float32 copy of the result (chain plumbing)."""
+        path, taps = self.plan(raster.shape)
         w = np.asarray(self.weights, dtype=np.float64)
-        if w.shape != (3, 3):
-            raise DeviceError(f"Convolve: only 3x3 weights are implemented on the device (got {w.shape})")
         ref = np.dtype(raster.ref_dtype)
         work = np.float32 if ref == np.float32 else np.float64       # ndimage keeps float dtypes, else float64
+        if path == "correlate" and (do_round or copy32 is not None):
+            raise DeviceError("Convolve: rounding and the float32 copy are only fused into the 3x3 path")
         src = dev.convert(raster, dev.hd_dtype_of(work))
         out = dev.empty(raster.ny, raster.nx, src.dtype, work)
+        if path == "correlate":
+            dy, dx, tw = taps
+            (dy, pdy), (dx, pdx) = _int_array(dy), _int_array(dx)
+            tw = np.ascontiguousarray(tw, dtype=np.float64)
+            _lib.check(_lib.load().hd_correlate(src.ptr, src.pitch, out.ptr, out.pitch, src.dtype, src.ny, src.nx, len(tw),
+                                                pdy, pdx, tw.ctypes.data_as(ctypes.POINTER(ctypes.c_double)),
+                                                float(w.size), dev.stream_ptr()))
+            return out
         corr = np.ascontiguousarray(w[::-1, ::-1])                    # convolution = correlation with the flipped kernel
         cw = (ctypes.c_double * 9)(*corr.ravel())
         _lib.check(_lib.load().hd_convolve3(src.ptr, src.pitch, out.ptr, out.pitch, src.dtype, src.ny, src.nx, cw,
@@ -78,25 +183,81 @@ class Convolve(DeviceFilter):
         return out
 
 
-class BinaryErosion(DeviceFilter):
+class BinaryErosion(_CheckedFilter):
     """``scipy.ndimage.binary_erosion(image, iterations=n)`` (extension_filters.py:187-235):
-    cross structuring element, border_value 0, bool result."""
+    cross structuring element, border_value 0, bool result.  n >= 1 is n erosions (hd_binary_morph, up to 8 per
+    launch); n < 1 repeats until the result stops changing, as scipy does."""
 
     def __init__(self, *, iterations):
         self.iterations = iterations
 
+    def plan(self, shape):
+        """("erode", [steps per launch]) or ("stable", None)."""
+        n = int(self.iterations)
+        if n < 1:
+            return "stable", None
+        k = MORPH_STEPS_PER_LAUNCH
+        return "erode", [k] * (n // k) + ([n % k] if n % k else [])
+
     def run_device(self, raster):
-        return _morph(raster, _lib.MORPH_ERODE, None, self.iterations)
+        path, launches = self.plan(raster.shape)
+        if path == "erode":
+            out = raster
+            for n in launches:
+                out = _morph(out, _lib.MORPH_ERODE, None, n)
+            return out
+        return _erode_until_stable(raster)
 
 
-class BinaryClosing(DeviceFilter):
-    """``scipy.ndimage.binary_closing(image, structure=...)`` (extension_filters.py:238-293)."""
+class BinaryClosing(_CheckedFilter):
+    """``scipy.ndimage.binary_closing(image, structure=...)`` (extension_filters.py:238-293).  None, the 3x3 cross and
+    the 3x3 square run on hd_binary_morph; any other 2-D structure up to 31x31 is a dilation and an erosion on
+    hd_binary_morph_struct."""
 
     def __init__(self, *, structure=None):
         self.structure = structure
 
+    def plan(self, shape):
+        """("morph3", None) or ("struct", (dilation taps, erosion taps))."""
+        if self.structure is None:
+            return "morph3", None
+        s = np.asarray(self.structure)
+        if s.shape == (3, 3) and ((s != 0).all() or ((s != 0) == _CROSS).all()):
+            return "morph3", None
+        return "struct", closing_taps(s)
+
     def run_device(self, raster):
-        return _morph(raster, _lib.MORPH_CLOSE, self.structure, 1)
+        path, taps = self.plan(raster.shape)
+        if path == "morph3":
+            return _morph(raster, _lib.MORPH_CLOSE, self.structure, 1)
+        dil, ero = taps
+        src = raster if raster.dtype in (_lib.U8, _lib.F32) else _nonzero_u8(raster)
+        return _morph_struct(_morph_struct(src, 1, dil, 1), 0, ero, 1)
+
+
+def _morph_struct(src, dilate, taps, iterations, changed=None):
+    dy, dx = taps
+    (dy, pdy), (dx, pdx) = _int_array(dy), _int_array(dx)
+    out = dev.empty(src.ny, src.nx, _lib.U8, np.bool_)
+    _lib.check(_lib.load().hd_binary_morph_struct(src.ptr, src.dtype, src.pitch, out.ptr, out.pitch, src.ny, src.nx, dilate,
+                                                  len(dy), pdy, pdx, iterations, changed, dev.stream_ptr()))
+    return out
+
+
+def _erode_until_stable(raster):
+    """Cross erosions until the result stops changing: launches of STABLE_STEPS_PER_LAUNCH erosions, each with its own
+    device flag "output != input", read once per STABLE_LAUNCHES_PER_READ launches.  Erosion with a structure that holds
+    its centre only removes cells, so a launch that changes nothing has reached the fixed point, and launches after it
+    return the same raster."""
+    import torch
+    taps = _offsets(_CROSS, reversed_=False)
+    flags = torch.zeros(STABLE_LAUNCHES_PER_READ, dtype=torch.int32, device=dev.device())
+    cur = raster if raster.dtype in (_lib.U8, _lib.F32) else _nonzero_u8(raster)
+    while True:
+        for i in range(STABLE_LAUNCHES_PER_READ):
+            cur = _morph_struct(cur, 0, taps, STABLE_STEPS_PER_LAUNCH, ctypes.c_void_p(flags.data_ptr() + 4 * i))
+        if bool((flags == 0).any().item()):                             # the one host read of these launches
+            return cur
 
 
 def _morph(raster, op, structure, iterations):
@@ -127,25 +288,37 @@ def _nonzero_u8(raster):
     return dev.elementwise(_lib.OP_ADD, lt, gt, 0.0, dev.empty(raster.ny, raster.nx, _lib.U8, np.bool_))
 
 
-class GreyDilation(DeviceFilter):
-    """``scipy.ndimage.grey_dilation(image, size=(s, s))`` (extension_filters.py:296-345):
-    flat square maximum filter, mode='reflect'."""
+class GreyDilation(_CheckedFilter):
+    """``scipy.ndimage.grey_dilation(image, size=(a, b))`` (extension_filters.py:296-345):
+    flat rectangular maximum filter, mode='reflect'.  Odd square sizes up to 17 that fit the raster run on
+    hd_max_filter; any other size 1 ... 255 per axis on hd_max_filter_rect."""
 
     def __init__(self, *, size):
         self.size = size
 
+    def plan(self, shape):
+        """("square", (s, s)) or ("rect", (a, b))."""
+        a, b = grey_sizes(self.size)
+        if a == b and a % 2 == 1 and a <= 17 and a <= min(shape):
+            return "square", (a, b)
+        return "rect", (a, b)
+
     def run_device(self, raster):
-        size = self.size if np.ndim(self.size) else (self.size, self.size)
-        if len(size) != 2 or size[0] != size[1] or size[0] % 2 != 1:
-            raise DeviceError(f"GreyDilation: only odd square sizes are implemented on the device (got {self.size})")
+        path, (a, b) = self.plan(raster.shape)
         ref = np.dtype(raster.ref_dtype)
         if ref == np.float64 and raster.dtype == _lib.F32:
             src = raster                                              # narrow-exact storage (e.g. majority values)
         else:
             src = dev.convert(raster, _lib.F32 if ref == np.float32 else _lib.F64)
         out = dev.empty(raster.ny, raster.nx, src.dtype, ref)
-        _lib.check(_lib.load().hd_max_filter(src.ptr, src.pitch, out.ptr, out.pitch, src.dtype, src.ny, src.nx,
-                                             int(size[0]), dev.stream_ptr()))
+        if path == "square":
+            _lib.check(_lib.load().hd_max_filter(src.ptr, src.pitch, out.ptr, out.pitch, src.dtype, src.ny, src.nx, a,
+                                                 dev.stream_ptr()))
+            return out
+        nbytes = src.ny * src.nx * src.itemsize
+        work = dev.scratch(nbytes)
+        _lib.check(_lib.load().hd_max_filter_rect(src.ptr, src.pitch, out.ptr, out.pitch, src.dtype, src.ny, src.nx, a, b,
+                                                  ctypes.c_void_p(work.data_ptr()), nbytes, dev.stream_ptr()))
         return out
 
 

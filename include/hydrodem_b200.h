@@ -308,6 +308,32 @@ int hd_tidy_lagoons(const void* majority, int64_t in_pitch, void* out, int64_t o
 int hd_convolve3(const void* in, int64_t in_pitch, void* out, int64_t out_pitch, int dtype, int64_t ny, int64_t nx,
                  const double* weights, double divisor, int do_round, void* out32, int64_t out32_pitch, void* stream);
 
+/* ---- general scipy.ndimage footprints (the drop-in wrappers with any argument the reference accepts) ---------------- */
+/* Convolve.apply, extension_filters.py:166-184, with any weights up to 31x31: out = (dtype) sum_t in[y + dy_t][x + dx_t] *
+ * w_t / (dtype) divisor, mode='reflect' at any distance (the extension repeats with period 2n, so rasters smaller than the
+ * weights work).  The taps (HOST arrays) are NI_Correlate's footprint: the flipped weights with scipy's origin shift on
+ * even axes, entries with |w| <= DBL_EPSILON left out, in row-major order, which is the order of the double sum (from
+ * +0.0, multiply then add, each rounded).  ntaps <= 961 (0: every cell 0), |dy|, |dx| <= 15, else HD_ERR_UNSUPPORTED.
+ * dtype: F32 or F64 (in and out alike). */
+int hd_correlate(const void* in, int64_t in_pitch, void* out, int64_t out_pitch, int dtype, int64_t ny, int64_t nx,
+                 int ntaps, const int* tap_dy, const int* tap_dx, const double* tap_w, double divisor, void* stream);
+/* BinaryErosion / BinaryClosing.apply, extension_filters.py:218-235, :276-293, with any structure up to 31x31:
+ * `iterations` erosions (dilate = 0: AND over the taps) or dilations (dilate = 1: OR) with border_value = 0.  The taps
+ * (HOST arrays) are the structure's True cells as offsets from the output cell: as given for scipy.ndimage.binary_erosion,
+ * reflected with the origin shift of even axes for binary_dilation.  ntaps = 0 gives all True (erosion) / all False
+ * (dilation), as scipy does.  iterations x |dy| and iterations x |dx| <= 15, else HD_ERR_UNSUPPORTED.  in: F32 or U8,
+ * non-zero = True (NaN is True); out: U8 0/1.  changed (DEVICE int, may be NULL): set to 1 if out differs from the input
+ * anywhere, else 0 -- "until stable" reads it once per launch of several iterations. */
+int hd_binary_morph_struct(const void* in, int in_dtype, int64_t in_pitch, void* out, int64_t out_pitch, int64_t ny,
+                           int64_t nx, int dilate, int ntaps, const int* tap_dy, const int* tap_dx, int iterations,
+                           int* changed, void* stream);
+/* GreyDilation.apply, extension_filters.py:328-345, with size=(size_y, size_x), each 1 ... 255 (even sizes with scipy's
+ * origin shift: the window of output i is [i - size/2 + 1, i + size/2]), mode='reflect' at any distance.  Two separable
+ * passes with a van Herk / Gil-Werman running maximum (three maxima per cell for any size); NaN cells are skipped.
+ * dtype: F32 or F64 (in and out alike).  workspace: DEVICE, at least ny * nx elements of dtype. */
+int hd_max_filter_rect(const void* in, int64_t in_pitch, void* out, int64_t out_pitch, int dtype, int64_t ny, int64_t nx,
+                       int size_y, int size_x, void* workspace, int64_t workspace_bytes, void* stream);
+
 /* ---- NEW hydrology stages (not in the reference, SURVEY.md 8a N2 / N3) ----------------------------------- */
 /* Sink-fill: Planchon-Darboux fixed point with eps = 0, 8-connectivity; frame cells and NaN cells are outlets.
  * z, w: F32.  Default (max_sweeps <= 0): persistent worklist kernels with a multigrid start (coarse DEMs of 8x8 block
