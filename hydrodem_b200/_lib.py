@@ -81,7 +81,7 @@ SIGNATURES = {
     "hd_fourier_mask_assemble_rows": (_i, [_p, _i64, _p, _i64, _i64, _i64, _p, _i64, _i64, _i64, _i64, _i64, _i64, _i, _p]),
     "hd_fftshift2": (_i, [_p, _i64, _p, _i64, _i, _i64, _i64, _i, _p]),
     "hd_pdfill_workspace_bytes": (_i64, [_i64, _i64]),
-    "hd_pdfill": (_i, [_p, _i64, _p, _i64, _i64, _i64, _p, _i64, _i, ctypes.POINTER(_i), _p]),
+    "hd_pdfill": (_i, [_p, _i64, _p, _i64, _i64, _i64, _p, _i64, ctypes.POINTER(_i), _p]),
     "hd_pdfill_band": (_i, [_p, _i64, _p, _i64, _i64, _i64, _p, _i64, _i, ctypes.POINTER(_i), _p]),
     "hd_pdfill_d8": (_i, [_p, _i64, _p, _i64, _p, _i64, _i64, _i64, _p, _i64, ctypes.POINTER(_i), _p]),
     "hd_pdfill_finish_d8": (_i, [_p, _i64, _p, _i64, _i64, _i64, _p, _p]),
@@ -90,7 +90,6 @@ SIGNATURES = {
     "hd_fill_pool_band": (_i, [_p, _i64, _i64, _i64, _p, _p, _i64, _i, _p, _p]),
     "hd_pdfill_coarse": (_i, [_p, _p, _i64, _i64, _i64, _p, _i64, _p]),
     "hd_pdfill_band_start": (_i, [_p, _i64, _p, _i64, _i64, _i64, _p, _i64, _i, _p, _i64, _i64, _p]),
-    "hd_pdfill_finish": (_i, [_p, _i64, _p, _i64, _i64, _i64, _p]),
     "hd_d8": (_i, [_p, _i64, _p, _i64, _i64, _i64, _p]),
     "hd_binary_morph": (_i, [_p, _i, _i64, _p, _i64, _i64, _i64, _i, _i, _i, _p]),
     "hd_max_filter": (_i, [_p, _i64, _p, _i64, _i, _i64, _i64, _i, _p]),

@@ -14,9 +14,8 @@
 //                       exactly the neighbours whose cells can still be lowered;
 //   fill_pool_kernel /  multigrid start: block maxima give coarse DEMs whose fill is an upper bound of the fine fill, so
 //   fill_refine_kernel  every level starts from the level above instead of +inf (same result, no raster-crossing wave);
-//   fill_sweep_kernel   the simple variant (HD_FILL_MODE=sweep): one launch per global sweep over the active tiles, z and
-//                       W staged by TMA; kept as an independent cross-check of the worklist kernel;
-//   d8_kernel           flow directions of the filled surface.
+//   d8_kernel           flow directions of the filled surface (fill_finish_d8_kernel: the same decision, d8_code, fused
+//                       with the fill's last pass).
 //
 // Algorithmic HBM traffic: 4 B (z) + 4 B (W) read + 4 B (W) written per cell of a visited tile.
 #include <cstdio>
@@ -30,14 +29,7 @@ namespace {
 constexpr int FT = 64;                    // tile edge
 constexpr int CB = 8;                     // block edge between two levels of the multigrid start of the fill (4: no fewer fine visits, one more level of latency)
 constexpr int FNT = 256;
-constexpr int WHX = 4;                    // x halo of the W box (16-byte TMA rule), 1 needed
-constexpr int WBOX_W = FT + 2 * WHX;      // 72
-constexpr int WBOX_H = FT + 2;            // 66
 constexpr int WS_STRIDE = FT + 3;         // 67: odd stride -> row marches are bank-conflict free
-constexpr uint32_t Z_BYTES = FT * FT * 4;
-constexpr uint32_t W_BYTES = WBOX_W * WBOX_H * 4;
-
-struct FillCounters { int changed_tiles; int pad[3]; };
 
 __global__ void __launch_bounds__(256) fill_init_kernel(const float* __restrict__ z, int64_t z_pitch, float* __restrict__ w,
                                                         int64_t w_pitch, int64_t ny, int64_t nx, int top_is_halo = 0,
@@ -96,80 +88,9 @@ __global__ void __launch_bounds__(256) fill_finish_kernel(const float* __restric
     }
 }
 
-template <int ZSTRIDE = FT>
-__device__ __forceinline__ float relax(const float* ws, const float* zs, int r, int c)
-{
-    // ws is the padded (FT+2) x WS_STRIDE array, cell (r, c) of the tile lives at ws[(r+1)*WS_STRIDE + c+1]
-    const float* p = ws + (r + 1) * WS_STRIDE + (c + 1);
-    float m = fminf(fminf(p[-WS_STRIDE - 1], p[-WS_STRIDE]), fminf(p[-WS_STRIDE + 1], p[-1]));
-    m = fminf(m, fminf(fminf(p[1], p[WS_STRIDE - 1]), fminf(p[WS_STRIDE], p[WS_STRIDE + 1])));
-    return fmaxf(zs[r * ZSTRIDE + c], m);       // fminf / fmaxf skip NaN operands
-}
-
-__global__ void __launch_bounds__(FNT) fill_sweep_kernel(const __grid_constant__ CUtensorMap tm_z,
-                                                         const __grid_constant__ CUtensorMap tm_w, float* __restrict__ w,
-                                                         int64_t w_pitch, int64_t ny, int64_t nx, int tiles_x, int tiles_y,
-                                                         const int* __restrict__ active_in, int* __restrict__ active_out,
-                                                         FillCounters* counters)
-{
-    extern __shared__ __align__(128) unsigned char smem[];
-    __shared__ uint64_t bar;
-    const int tile = blockIdx.x;
-    if (!active_in[tile]) return;
-    float* zs = reinterpret_cast<float*>(smem);                           // [FT][FT]
-    float* wbox = reinterpret_cast<float*>(smem + Z_BYTES);               // [WBOX_H][WBOX_W] as loaded
-    float* ws = reinterpret_cast<float*>(smem + Z_BYTES + W_BYTES);       // [(FT+2)][WS_STRIDE] padded copy
-    const int ty0 = (tile / tiles_x) * FT, tx0 = (tile % tiles_x) * FT;
-    if (threadIdx.x == 0) {
-        mbar_init(&bar, 1);
-        mbar_fence_init();
-        mbar_arrive_expect_tx(&bar, Z_BYTES + W_BYTES);
-        tma_load_2d(zs, &tm_z, tx0, ty0, &bar);
-        tma_load_2d(wbox, &tm_w, tx0 - WHX, ty0 - 1, &bar);
-    }
-    __syncthreads();
-    mbar_wait(&bar, 0);
-    for (int t = threadIdx.x; t < WBOX_H * (FT + 2); t += FNT) {
-        const int r = t / (FT + 2), c = t - r * (FT + 2);
-        ws[r * WS_STRIDE + c] = wbox[r * WBOX_W + c + WHX - 1];
-    }
-    __syncthreads();
-
-    const int group = threadIdx.x >> 6, lane64 = threadIdx.x & 63;
-    bool tile_changed = false;
-    for (int iter = 0; iter < 4096; ++iter) {
-        bool changed = false;
-        for (int step = 0; step < FT; ++step) {
-            int r, c;
-            if (group == 0) { r = step; c = lane64; }                     // marching down
-            else if (group == 1) { r = FT - 1 - step; c = lane64; }       // up
-            else if (group == 2) { r = lane64; c = step; }                // right
-            else { r = lane64; c = FT - 1 - step; }                       // left
-            float* cell = ws + (r + 1) * WS_STRIDE + (c + 1);
-            const float cand = relax(ws, zs, r, c);
-            if (cand < *cell) { *cell = cand; changed = true; }           // only ever lowers W
-        }
-        if (!__syncthreads_or(changed)) break;
-        tile_changed = true;
-    }
-    if (tile_changed) {
-        for (int t = threadIdx.x; t < FT * FT; t += FNT) {
-            const int r = t >> 6, c = t & 63;
-            const int64_t y = ty0 + r, x = tx0 + c;
-            if (y < ny && x < nx) w[y * w_pitch + x] = ws[(r + 1) * WS_STRIDE + c + 1];
-        }
-        if (threadIdx.x < 9) {
-            const int dy = (int)threadIdx.x / 3 - 1, dx = (int)threadIdx.x % 3 - 1;
-            const int tyy = tile / tiles_x + dy, txx = tile % tiles_x + dx;
-            if (tyy >= 0 && tyy < tiles_y && txx >= 0 && txx < tiles_x) active_out[tyy * tiles_x + txx] = 1;
-        }
-        if (threadIdx.x == 0) atomicAdd(&counters->changed_tiles, 1);
-    }
-}
-
-// ---- asynchronous worklist variant (default on one GPU) --------------------------------------------------------------
-// The sweep kernel above needs one launch per "ring" of tiles the fill wave crosses (39 sweeps on a 3601^2 tile) and
-// visits every active tile once per sweep.  Here a persistent grid of co-resident CTAs pulls tiles from a device-side
+// ---- asynchronous worklist ----------------------------------------------------------------------------------------------
+// A level-synchronous schedule needs one launch per "ring" of tiles the fill wave crosses (39 sweeps on a 3601^2 tile)
+// and visits every active tile once per sweep.  Here a persistent grid of co-resident CTAs pulls tiles from a device-side
 // FIFO: a tile that changed pushes exactly the neighbours whose halo it changed, so the wave advances as fast as single
 // tiles finish and nothing waits for a grid-wide barrier.  Because the fixed point is unique, the (racy) order in which
 // tiles are processed cannot change the result.
@@ -215,10 +136,11 @@ struct FillCtl {
 constexpr int SLOT_EMPTY = -1;
 constexpr int SPIN_LIMIT = 1 << 22;
 // Sticky status word of a fill, at byte STATUS_OFF of the workspace (inside the 256 bytes reserved for the finest level's
-// control block, cleared once per hd_pdfill / first hd_pdfill_band call): set by ANY level whose worklist stalled
-// (a waiting CTA ran out of patience: preemption, MPS, a debugger) or whose in-tile iteration hit its cap.  The finish
-// kernels poison W[0][0] with NaN when it is set, and hd_pdfill_status reads it back: a fill that did not reach the
-// fixed point can never pass silently, with or without statistics, inside or outside a CUDA graph.
+// control block, cleared once per fill: hd_pdfill, hd_pdfill_d8, hd_pdfill_coarse, hd_pdfill_band_start): set by ANY
+// level whose worklist stalled (a waiting CTA ran out of patience: preemption, MPS, a debugger) or whose in-tile
+// iteration hit its cap.  The finish kernels poison W[0][0] with NaN when it is set, and hd_pdfill_status reads it
+// back: a fill that did not reach the fixed point can never pass silently, with or without statistics, inside or
+// outside a CUDA graph.
 constexpr int STATUS_OFF = 192;
 enum { FILL_STALLED = 1, FILL_ITER_CAP = 2, FILL_PENDING = 4 };
 // per-tile state: a tile is never processed by two CTAs at once (a second writer could overwrite a lower W with a
@@ -611,6 +533,30 @@ __global__ void __launch_bounds__(FNT, 4) fill_async_kernel(const float* __restr
 // ---- D8 ------------------------------------------------------------------------------------------------------
 // ESRI codes E=1 SE=2 S=4 SW=8 W=16 NW=32 N=64 NE=128; steepest positive drop, diagonal drops scaled by
 // 0.70710678f in float32; ties keep the first in that order; frame cells, NaN centres, no drop -> 0.
+// The code of cell j of a quad from its window: three rows of (left neighbour, aligned quad, right neighbour).
+__device__ __forceinline__ uint8_t d8_code(const float (&win)[3][6], int j)
+{
+    const float c = win[1][j + 1];
+    // E, SE, S, SW, W, NW, N, NE; diagonal drops scaled in float32
+    const float d0 = __fsub_rn(c, win[1][j + 2]), d1 = __fmul_rn(__fsub_rn(c, win[2][j + 2]), 0.70710678f);
+    const float d2 = __fsub_rn(c, win[2][j + 1]), d3 = __fmul_rn(__fsub_rn(c, win[2][j]), 0.70710678f);
+    const float d4 = __fsub_rn(c, win[1][j]), d5 = __fmul_rn(__fsub_rn(c, win[0][j]), 0.70710678f);
+    const float d6 = __fsub_rn(c, win[0][j + 1]), d7 = __fmul_rn(__fsub_rn(c, win[0][j + 2]), 0.70710678f);
+    // "first strictly larger drop wins" == the FIRST direction that attains the maximum, if it is positive
+    // (three-input max: 4 instructions; NaN drops are skipped by max and never compare equal)
+    const float best = fmax3(fmax3(d0, d1, d2), fmax3(d3, d4, d5), fmax3(d6, d7, 0.f));
+    unsigned code = 0u;
+    code = d7 == best ? 128u : code;
+    code = d6 == best ? 64u : code;
+    code = d5 == best ? 32u : code;
+    code = d4 == best ? 16u : code;
+    code = d3 == best ? 8u : code;
+    code = d2 == best ? 4u : code;
+    code = d1 == best ? 2u : code;
+    code = d0 == best ? 1u : code;
+    return best > 0.f ? (uint8_t)code : (uint8_t)0;
+}
+
 __global__ void __launch_bounds__(256) d8_kernel(const float* __restrict__ w, int64_t w_pitch, uint8_t* __restrict__ out,
                                                  int64_t out_pitch, int64_t ny, int64_t nx)
 {
@@ -634,19 +580,7 @@ __global__ void __launch_bounds__(256) d8_kernel(const float* __restrict__ w, in
             for (int j = 0; j < 4; ++j) {
                 const int64_t x = x0 + j;
                 if (x == 0 || x >= nx - 1) continue;
-                const float c = win[1][j + 1];
-                // E, SE, S, SW, W, NW, N, NE
-                const float nb[8] = {win[1][j + 2], win[2][j + 2], win[2][j + 1], win[2][j], win[1][j], win[0][j],
-                                     win[0][j + 1], win[0][j + 2]};
-                float best = 0.f;
-                uint8_t code = 0;
-#pragma unroll
-                for (int k = 0; k < 8; ++k) {
-                    float drop = __fsub_rn(c, nb[k]);
-                    if (k & 1) drop = __fmul_rn(drop, 0.70710678f);
-                    if (drop > best) { best = drop; code = (uint8_t)(1u << k); }
-                }
-                codes[j] = code;
+                codes[j] = d8_code(win, j);
             }
         }
         store4v<uint8_t>(out, out_pitch, y, x0, nx, codes);
@@ -710,24 +644,7 @@ __global__ void __launch_bounds__(256) fill_finish_d8_kernel(float* __restrict__
             const float c = win[1][j + 1];
             restore |= has_nodata && (c != c) && x < nx;
             if (y == 0 || y >= ny - 1 || x == 0 || x >= nx - 1) continue;
-            // E, SE, S, SW, W, NW, N, NE; diagonal drops scaled in float32
-            const float d0 = __fsub_rn(c, win[1][j + 2]), d1 = __fmul_rn(__fsub_rn(c, win[2][j + 2]), 0.70710678f);
-            const float d2 = __fsub_rn(c, win[2][j + 1]), d3 = __fmul_rn(__fsub_rn(c, win[2][j]), 0.70710678f);
-            const float d4 = __fsub_rn(c, win[1][j]), d5 = __fmul_rn(__fsub_rn(c, win[0][j]), 0.70710678f);
-            const float d6 = __fsub_rn(c, win[0][j + 1]), d7 = __fmul_rn(__fsub_rn(c, win[0][j + 2]), 0.70710678f);
-            // "first strictly larger drop wins" == the FIRST direction that attains the maximum, if it is positive
-            // (three-input max: 4 instructions; NaN drops are skipped by max and never compare equal)
-            const float best = fmax3(fmax3(d0, d1, d2), fmax3(d3, d4, d5), fmax3(d6, d7, 0.f));
-            unsigned code = 0u;
-            code = d7 == best ? 128u : code;
-            code = d6 == best ? 64u : code;
-            code = d5 == best ? 32u : code;
-            code = d4 == best ? 16u : code;
-            code = d3 == best ? 8u : code;
-            code = d2 == best ? 4u : code;
-            code = d1 == best ? 2u : code;
-            code = d0 == best ? 1u : code;
-            codes[j] = best > 0.f ? (uint8_t)code : (uint8_t)0;
+            codes[j] = d8_code(win, j);
         }
         if (restore) {                                                    // rare: rewrite the quad with NaN at the nodata cells
 #pragma unroll
@@ -852,8 +769,8 @@ static int pdfill_async(const void* z, int64_t z_pitch, void* w, int64_t w_pitch
 static int64_t fill_level_bytes(int64_t ny, int64_t nx)
 {
     const int64_t ntiles = (int64_t)hd_cdiv(ny, FT) * hd_cdiv(nx, FT);
-    // control block + FIFO ring (ntiles + slack) + per-tile flags; the sweep variant uses two flag arrays
-    const int64_t b = 256 + (2 * ntiles + 8192) * (int64_t)sizeof(int) + 2 * ntiles * (int64_t)sizeof(int);
+    // what pdfill_async lays out: control block, FIFO ring (ntiles + slack slots), per-tile states
+    const int64_t b = 256 + (2 * ntiles + 8192) * (int64_t)sizeof(int);
     return (b + 255) / 256 * 256;
 }
 static int64_t coarse_pitch(int64_t nxc) { return (nxc + 31) / 32 * 32; }
@@ -874,48 +791,41 @@ extern "C" int64_t hd_pdfill_workspace_bytes(int64_t ny, int64_t nx)
     return total;
 }
 
-// Multigrid start (see fill_pool_kernel): DEM -> coarser DEMs by block maxima; the coarsest level is filled from
-// scratch, every finer level starts from the fill of the level above it.
-static int pdfill_multilevel(const void* z, int64_t z_pitch, void* w, int64_t w_pitch, int64_t ny, int64_t nx, void* workspace,
-                             int* visits_out, cudaStream_t s, int flags = 0, bool finish = true)
+// Multigrid start (see fill_pool_kernel): the coarse levels below a raster, by block maxima, laid out in its workspace
+// after its own control block; the coarsest level is filled from scratch, every finer one from the level above it.
+// The first level pools z: its outlet marks come from the frame and the NaN cells, plus those of `marks` when given
+// (a coarse raster whose W carries its own outlet marks, same pitch as z).  *first = the finest coarse level, whose w
+// is nullptr when the raster is too small for one.
+struct FillLevel { int64_t ny, nx, pitch; float* z; float* w; char* ctl; };
+
+static int fill_coarse_levels(const float* z, const float* marks, int64_t pitch, int64_t ny, int64_t nx, void* workspace,
+                              cudaStream_t s, FillLevel* first)
 {
-    struct Level { int64_t ny, nx, pitch; float* z; float* w; char* ctl; };
-    Level lv[MAX_LEVELS];
+    FillLevel lv[MAX_LEVELS];
     int nlev = 0;
-    const char* off = getenv("HD_FILL_MULTILEVEL");
     char* cur = (char*)workspace + fill_level_bytes(ny, nx);
-    int64_t lny = ny, lnx = nx;
-    if (!(off && off[0] == '0')) {
-        for (int l = 1; l < MAX_LEVELS; ++l) {
-            const int64_t nyc = hd_cdiv(lny, CB), nxc = hd_cdiv(lnx, CB);
-            if (!level_worth_it(nyc, nxc)) break;
-            Level& L = lv[nlev++];
-            L.ny = nyc; L.nx = nxc; L.pitch = coarse_pitch(nxc);
-            L.ctl = cur;
-            L.z = (float*)(cur + fill_level_bytes(nyc, nxc));
-            L.w = L.z + nyc * L.pitch;
-            cur = (char*)(L.w + nyc * L.pitch);
-            lny = nyc; lnx = nxc;
-        }
-    }
-    if (nlev == 0) return pdfill_async(z, z_pitch, w, w_pitch, ny, nx, workspace, visits_out, s, flags, finish);
     // downward: block maxima + outlet marks of every level
-    for (int l = 0; l < nlev; ++l) {
-        const Level& L = lv[l];
-        const float* zin = l == 0 ? (const float*)z : lv[l - 1].z;
-        const float* win = l == 0 ? nullptr : lv[l - 1].w;
-        const int64_t pin = l == 0 ? z_pitch : lv[l - 1].pitch, iny = l == 0 ? ny : lv[l - 1].ny, inx = l == 0 ? nx : lv[l - 1].nx;
-        const int tiles_x_c = hd_cdiv(L.nx, FT), ntiles_c = tiles_x_c * hd_cdiv(L.ny, FT);
+    for (int l = 1; l < MAX_LEVELS; ++l) {
+        const int64_t nyc = hd_cdiv(ny, CB), nxc = hd_cdiv(nx, CB);
+        if (!level_worth_it(nyc, nxc)) break;
+        FillLevel& L = lv[nlev++];
+        L.ny = nyc; L.nx = nxc; L.pitch = coarse_pitch(nxc);
+        L.ctl = cur;
+        L.z = (float*)(cur + fill_level_bytes(nyc, nxc));
+        L.w = L.z + nyc * L.pitch;
+        cur = (char*)(L.w + nyc * L.pitch);
+        const int tiles_x_c = hd_cdiv(nxc, FT), ntiles_c = tiles_x_c * hd_cdiv(nyc, FT);
         int* queued_c = (int*)(L.ctl + 256) + (ntiles_c + 8192);
         HD_CUDA_OK(cudaMemsetAsync(queued_c, 0, (size_t)ntiles_c * sizeof(int), s));
         hd_prof_begin("fill_pool_kernel", s);
-        fill_pool_kernel<<<stream_grid(L.ny * L.nx), 256, 0, s>>>(zin, pin, iny, inx, L.z, L.w, L.pitch, L.ny, L.nx, queued_c,
-                                                                  tiles_x_c, win, flags & 2, flags & 4);
+        fill_pool_kernel<<<stream_grid(nyc * nxc), 256, 0, s>>>(z, pitch, ny, nx, L.z, L.w, L.pitch, nyc, nxc, queued_c,
+                                                                tiles_x_c, marks, 0, 0);
         HD_LAUNCH_CHECK(); hd_count_launch();
+        z = L.z; marks = L.w; pitch = L.pitch; ny = nyc; nx = nxc;
     }
     // upward: coarsest level from scratch, every finer one from the level above
     for (int l = nlev - 1; l >= 0; --l) {
-        const Level& L = lv[l];
+        const FillLevel& L = lv[l];
         FillOpts o;
         o.preinit = true;
         o.status = (int*)((char*)workspace + STATUS_OFF);
@@ -925,100 +835,47 @@ static int pdfill_multilevel(const void* z, int64_t z_pitch, void* w, int64_t w_
             HD_LAUNCH_CHECK(); hd_count_launch();
             o.seed_all = true;
         }
-        if (int e = pdfill_async(L.z, L.pitch, L.w, L.pitch, L.ny, L.nx, L.ctl, nullptr, s, flags & 6, false, o)) return e;
+        if (int e = pdfill_async(L.z, L.pitch, L.w, L.pitch, L.ny, L.nx, L.ctl, nullptr, s, 0, false, o)) return e;
     }
+    *first = nlev ? lv[0] : FillLevel{};
+    return HD_OK;
+}
+
+// Fill of one whole raster: the fine level starts from the fill of the coarse levels.
+static int pdfill_multilevel(const void* z, int64_t z_pitch, void* w, int64_t w_pitch, int64_t ny, int64_t nx, void* workspace,
+                             int* visits_out, cudaStream_t s, bool finish)
+{
+    FillLevel first;
+    if (int e = fill_coarse_levels((const float*)z, nullptr, z_pitch, ny, nx, workspace, s, &first)) return e;
     FillOpts fine;
-    fine.status = (int*)((char*)workspace + STATUS_OFF);
-    fine.seed_all = true;
-    fine.wc = lv[0].w;
-    fine.c_pitch = lv[0].pitch;
-    return pdfill_async(z, z_pitch, w, w_pitch, ny, nx, workspace, visits_out, s, flags, finish, fine);
+    if (first.w) {
+        fine.seed_all = true;
+        fine.wc = first.w;
+        fine.c_pitch = first.pitch;
+    }
+    return pdfill_async(z, z_pitch, w, w_pitch, ny, nx, workspace, visits_out, s, 0, finish, fine);
 }
 
 extern "C" int hd_pdfill(const void* z, int64_t z_pitch, void* w, int64_t w_pitch, int64_t ny, int64_t nx, void* workspace,
-                         int64_t workspace_bytes, int max_sweeps, int* sweeps_out, void* stream)
+                         int64_t workspace_bytes, int* visits_out, void* stream)
 {
     if (!z || !w || !workspace) return HD_ERR_NULL;
     if (ny < 1 || nx < 1 || z_pitch < nx || w_pitch < nx) return HD_ERR_ARG;
     if (workspace_bytes < hd_pdfill_workspace_bytes(ny, nx)) return HD_ERR_WORKSPACE;
     cudaStream_t s = (cudaStream_t)stream;
     HD_CUDA_OK(cudaMemsetAsync((char*)workspace + STATUS_OFF, 0, sizeof(int), s));
-    const int tiles_x = hd_cdiv(nx, FT), tiles_y = hd_cdiv(ny, FT), ntiles = tiles_x * tiles_y;
-    const char* mode = getenv("HD_FILL_MODE");
-    if (!(mode && mode[0] == 's') && max_sweeps <= 0)
-        return pdfill_multilevel(z, z_pitch, w, w_pitch, ny, nx, workspace, sweeps_out, s);
-    FillCounters* counters = (FillCounters*)workspace;
-    int* flags_a = (int*)((char*)workspace + 256);
-    int* flags_b = flags_a + ntiles;
-    CUtensorMap tm_z, tm_w;
-    if (int e = hd_make_tmap_2d(&tm_z, z, HD_F32, ny, nx, z_pitch, FT, FT, false)) return e;
-    if (int e = hd_make_tmap_2d(&tm_w, w, HD_F32, ny, nx, w_pitch, WBOX_W, WBOX_H, true)) return e;
-    const size_t smem = Z_BYTES + W_BYTES + (size_t)(FT + 2) * WS_STRIDE * 4;
-    HD_CUDA_OK(cudaFuncSetAttribute(fill_sweep_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-
-    hd_prof_begin("fill_init_kernel", s);
-    fill_init_kernel<<<stream_grid(ny * ((nx + 3) / 4)), 256, 0, s>>>((const float*)z, z_pitch, (float*)w, w_pitch, ny, nx);
-    HD_LAUNCH_CHECK(); hd_count_launch();
-    // every tile starts active
-    HD_CUDA_OK(cudaMemsetAsync(flags_a, 1, (size_t)ntiles * sizeof(int), s));   // any non-zero byte pattern = active
-    static thread_local int* h_changed = nullptr;
-    if (!h_changed) HD_CUDA_OK(cudaHostAlloc((void**)&h_changed, sizeof(int), cudaHostAllocDefault));
-    int sweeps = 0, rc = HD_OK;
-    int* fin = flags_a;
-    int* fout = flags_b;
-    if (max_sweeps <= 0) max_sweeps = 1 << 30;
-    const bool trace = getenv("HD_FILL_TRACE") != nullptr;
-    const int batch = trace ? 1 : 4;          // sweeps between host convergence checks
-    for (;;) {
-        int last_changed_ptr_valid = 0;
-        for (int b = 0; b < batch && sweeps < max_sweeps; ++b) {
-            HD_CUDA_OK(cudaMemsetAsync(fout, 0, (size_t)ntiles * sizeof(int), s));
-            HD_CUDA_OK(cudaMemsetAsync(counters, 0, sizeof(FillCounters), s));
-            hd_prof_begin("fill_sweep_kernel", s);
-            fill_sweep_kernel<<<ntiles, FNT, smem, s>>>(tm_z, tm_w, (float*)w, w_pitch, ny, nx, tiles_x, tiles_y, fin, fout,
-                                                       counters);
-            HD_LAUNCH_CHECK(); hd_count_launch();
-            int* tmp = fin; fin = fout; fout = tmp;
-            ++sweeps;
-            last_changed_ptr_valid = 1;
-        }
-        if (!last_changed_ptr_valid) { rc = HD_OK; break; }
-        // the counter of the LAST sweep of the batch: zero means that sweep found a global fixed point
-        HD_CUDA_OK(cudaMemcpyAsync(h_changed, &counters->changed_tiles, sizeof(int), cudaMemcpyDeviceToHost, s));
-        HD_CUDA_OK(cudaStreamSynchronize(s));
-        if (trace) fprintf(stderr, "pdfill sweep %d: %d of %d tiles changed\n", sweeps, *h_changed, ntiles);
-        if (*h_changed == 0) break;
-        if (sweeps >= max_sweeps) { rc = HD_ERR_UNSUPPORTED; break; }        // did not converge within max_sweeps
-    }
-    hd_prof_begin("fill_finish_kernel", s);
-    fill_finish_kernel<<<stream_grid(ny * nx), 256, 0, s>>>((const float*)z, z_pitch, (float*)w, w_pitch, ny, nx);
-    HD_LAUNCH_CHECK(); hd_count_launch();
-    if (sweeps_out) *sweeps_out = sweeps;
-    return rc;
+    return pdfill_multilevel(z, z_pitch, w, w_pitch, ny, nx, workspace, visits_out, s, true);
 }
 
+// Next round of a banded fill, after a halo exchange: W holds the previous round's result (the first round is
+// hd_pdfill_band_start), only the tile rows next to the halo rows are re-seeded.
 extern "C" int hd_pdfill_band(const void* z, int64_t z_pitch, void* w, int64_t w_pitch, int64_t ny, int64_t nx,
                               void* workspace, int64_t workspace_bytes, int flags, int* visits_out, void* stream)
 {
     if (!z || !w || !workspace) return HD_ERR_NULL;
-    if (ny < 1 || nx < 1 || z_pitch < nx || w_pitch < nx || (flags & ~7)) return HD_ERR_ARG;
+    if (ny < 1 || nx < 1 || z_pitch < nx || w_pitch < nx || (flags & ~6)) return HD_ERR_ARG;
     if (workspace_bytes < hd_pdfill_workspace_bytes(ny, nx)) return HD_ERR_WORKSPACE;
-    if (!(flags & 1)) HD_CUDA_OK(cudaMemsetAsync((char*)workspace + STATUS_OFF, 0, sizeof(int), (cudaStream_t)stream));
-    if (!(flags & 1))       // first round of a band: multigrid start (halo rows are not outlets); later rounds continue
-        return pdfill_multilevel(z, z_pitch, w, w_pitch, ny, nx, workspace, visits_out, (cudaStream_t)stream, flags, false);
-    return pdfill_async(z, z_pitch, w, w_pitch, ny, nx, workspace, visits_out, (cudaStream_t)stream, flags, false);
-}
-
-extern "C" int hd_pdfill_finish(const void* z, int64_t z_pitch, void* w, int64_t w_pitch, int64_t ny, int64_t nx,
-                                void* stream)
-{
-    if (!z || !w) return HD_ERR_NULL;
-    if (ny < 1 || nx < 1 || z_pitch < nx || w_pitch < nx) return HD_ERR_ARG;
-    cudaStream_t s = (cudaStream_t)stream;
-    hd_prof_begin("fill_finish_kernel", s);
-    fill_finish_kernel<<<stream_grid(ny * nx), 256, 0, s>>>((const float*)z, z_pitch, (float*)w, w_pitch, ny, nx);
-    HD_LAUNCH_CHECK(); hd_count_launch();
-    return HD_OK;
+    return pdfill_async(z, z_pitch, w, w_pitch, ny, nx, workspace, visits_out, (cudaStream_t)stream, flags | 1, false);
 }
 
 extern "C" int hd_d8(const void* w, int64_t w_pitch, void* out, int64_t out_pitch, int64_t ny, int64_t nx, void* stream)
@@ -1042,7 +899,7 @@ extern "C" int hd_pdfill_d8(const void* z, int64_t z_pitch, void* w, int64_t w_p
     if (workspace_bytes < hd_pdfill_workspace_bytes(ny, nx)) return HD_ERR_WORKSPACE;
     cudaStream_t s = (cudaStream_t)stream;
     HD_CUDA_OK(cudaMemsetAsync((char*)workspace + STATUS_OFF, 0, sizeof(int), s));
-    if (int e = pdfill_multilevel(z, z_pitch, w, w_pitch, ny, nx, workspace, visits_out, s, 0, false)) return e;
+    if (int e = pdfill_multilevel(z, z_pitch, w, w_pitch, ny, nx, workspace, visits_out, s, false)) return e;
     return launch_finish_d8(w, w_pitch, d8, d8_pitch, ny, nx, workspace, s);
 }
 
@@ -1117,58 +974,16 @@ extern "C" int hd_pdfill_coarse(const void* zc, void* wc, int64_t c_pitch, int64
     if (workspace_bytes < hd_pdfill_workspace_bytes(nyc, nxc)) return HD_ERR_WORKSPACE;
     cudaStream_t s = (cudaStream_t)stream;
     HD_CUDA_OK(cudaMemsetAsync((char*)workspace + STATUS_OFF, 0, sizeof(int), s));
-    int* status = (int*)((char*)workspace + STATUS_OFF);
-    struct Level { int64_t ny, nx, pitch; float* z; float* w; char* ctl; };
-    Level lv[MAX_LEVELS];
-    int nlev = 0;
-    char* cur = (char*)workspace + fill_level_bytes(nyc, nxc);
-    int64_t lny = nyc, lnx = nxc;
-    for (int l = 1; l < MAX_LEVELS; ++l) {
-        const int64_t ny2 = hd_cdiv(lny, CB), nx2 = hd_cdiv(lnx, CB);
-        if (!level_worth_it(ny2, nx2)) break;
-        Level& L = lv[nlev++];
-        L.ny = ny2; L.nx = nx2; L.pitch = coarse_pitch(nx2);
-        L.ctl = cur;
-        L.z = (float*)(cur + fill_level_bytes(ny2, nx2));
-        L.w = L.z + ny2 * L.pitch;
-        cur = (char*)(L.w + ny2 * L.pitch);
-        lny = ny2; lnx = nx2;
-    }
-    for (int l = 0; l < nlev; ++l) {                                  // downward: block maxima + outlet marks
-        const Level& L = lv[l];
-        const float* zin = l == 0 ? (const float*)zc : lv[l - 1].z;
-        const float* win = l == 0 ? (const float*)wc : lv[l - 1].w;
-        const int64_t pin = l == 0 ? c_pitch : lv[l - 1].pitch, iny = l == 0 ? nyc : lv[l - 1].ny, inx = l == 0 ? nxc : lv[l - 1].nx;
-        const int tiles_x_c = hd_cdiv(L.nx, FT), ntiles_c = tiles_x_c * hd_cdiv(L.ny, FT);
-        int* queued_c = (int*)(L.ctl + 256) + (ntiles_c + 8192);
-        HD_CUDA_OK(cudaMemsetAsync(queued_c, 0, (size_t)ntiles_c * sizeof(int), s));
-        hd_prof_begin("fill_pool_kernel", s);
-        fill_pool_kernel<<<stream_grid(L.ny * L.nx), 256, 0, s>>>(zin, pin, iny, inx, L.z, L.w, L.pitch, L.ny, L.nx, queued_c,
-                                                                  tiles_x_c, win, 0, 0);
+    FillLevel first;
+    if (int e = fill_coarse_levels((const float*)zc, (const float*)wc, c_pitch, nyc, nxc, workspace, s, &first)) return e;
+    if (first.w) {
+        hd_prof_begin("fill_refine_kernel", s);
+        fill_refine_kernel<<<stream_grid(nyc * nxc), 256, 0, s>>>((float*)wc, c_pitch, nyc, nxc, first.w, first.pitch);
         HD_LAUNCH_CHECK(); hd_count_launch();
-    }
-    for (int l = nlev - 1; l >= 0; --l) {                              // upward
-        const Level& L = lv[l];
-        FillOpts o;
-        o.preinit = true;
-        o.status = status;
-        if (l < nlev - 1) {
-            hd_prof_begin("fill_refine_kernel", s);
-            fill_refine_kernel<<<stream_grid(L.ny * L.nx), 256, 0, s>>>(L.w, L.pitch, L.ny, L.nx, lv[l + 1].w, lv[l + 1].pitch);
-            HD_LAUNCH_CHECK(); hd_count_launch();
-            o.seed_all = true;
-        }
-        if (int e = pdfill_async(L.z, L.pitch, L.w, L.pitch, L.ny, L.nx, L.ctl, nullptr, s, 0, false, o)) return e;
     }
     FillOpts top;
     top.preinit = true;
     top.seed_all = true;
-    top.status = status;
-    if (nlev > 0) {
-        hd_prof_begin("fill_refine_kernel", s);
-        fill_refine_kernel<<<stream_grid(nyc * nxc), 256, 0, s>>>((float*)wc, c_pitch, nyc, nxc, lv[0].w, lv[0].pitch);
-        HD_LAUNCH_CHECK(); hd_count_launch();
-    }
     return pdfill_async(zc, c_pitch, wc, c_pitch, nyc, nxc, workspace, nullptr, s, 0, false, top);
 }
 

@@ -45,10 +45,9 @@ class MedianFilter(WindowFilter):
 class SinkFill(DeviceFilter):
     """Depression filling: the Planchon-Darboux fixed point with eps = 0 and
     8-connectivity; frame cells and NaN cells are outlets.  float32 result.
-    ``sweeps`` holds the number of global tile sweeps of the last call."""
+    ``sweeps`` holds the number of tile visits of the finest level in the last call."""
 
-    def __init__(self, *, max_sweeps=0, want_stats=True):
-        self.max_sweeps = max_sweeps
+    def __init__(self, *, want_stats=True):
         self.want_stats = want_stats      # False: no host synchronisation inside the call
         self.sweeps = None
 
@@ -61,12 +60,11 @@ class SinkFill(DeviceFilter):
         import torch
         # statistics need a host synchronisation inside the call: impossible while a CUDA graph is being captured
         stats = self.want_stats and not torch.cuda.is_current_stream_capturing()
-        sweeps = ctypes.c_int(-1)
+        visits = ctypes.c_int(-1)
         self._work = work
         _lib.check(lib.hd_pdfill(src.ptr, src.pitch, out.ptr, out.pitch, src.ny, src.nx, ctypes.c_void_p(work.data_ptr()),
-                                 nbytes, int(self.max_sweeps), ctypes.byref(sweeps) if stats else None,
-                                 dev.stream_ptr()))
-        self.sweeps = sweeps.value if stats else None
+                                 nbytes, ctypes.byref(visits) if stats else None, dev.stream_ptr()))
+        self.sweeps = visits.value if stats else None
         return out
 
 

@@ -748,36 +748,34 @@ class Band:
         recv_up = torch.empty(nx, dtype=torch.float32, device=dev.device()) if n_up else None
         recv_down = torch.empty(nx, dtype=torch.float32, device=dev.device()) if n_down else None
         rounds = 0
-        wc_g = None
         TRACE.mark("fill: overlap exchange")
-        if comm.world > 1:
-            # global multigrid start: pool my band, all-gather the coarse DEM, fill the whole coarse mosaic on every rank
-            nyc, nxc = -(-self.ny // 8), -(-nx // 8)
-            cp = (nxc + 31) // 32 * 32
-            zc_g = torch.empty((nyc, cp), dtype=torch.float32, device=dev.device())
-            wc_g = torch.empty((nyc, cp), dtype=torch.float32, device=dev.device())
-            cb = [(a // 8, -(-b // 8)) for a, b in self.bounds]
-            c0, c1 = cb[comm.rank]
-            scratch = torch.zeros(((c1 - c0) // 64 + 2) * (nxc // 64 + 2), dtype=torch.int32, device=dev.device())
-            own = z.owned()
-            _lib.check(lib.hd_fill_pool_band(own.ptr, own.pitch, rows, nx, ctypes.c_void_p(zc_g[c0].data_ptr()),
-                                             ctypes.c_void_p(wc_g[c0].data_ptr()), cp, flags,
-                                             ctypes.c_void_p(scratch.data_ptr()), dev.stream_ptr()))
-            for g in (zc_g, wc_g):
-                comm.p2p([(g[c0:c1], j) for j in range(comm.world) if j != comm.rank],
-                         [(g[a:b], i) for i, (a, b) in enumerate(cb) if i != comm.rank])
-            cbytes = lib.hd_pdfill_workspace_bytes(nyc, nxc)
-            cwork = dev.scratch(cbytes)
-            _lib.check(lib.hd_pdfill_coarse(ctypes.c_void_p(zc_g.data_ptr()), ctypes.c_void_p(wc_g.data_ptr()), cp, nyc, nxc,
-                                            ctypes.c_void_p(cwork.data_ptr()), cbytes, dev.stream_ptr()))
+        # global multigrid start: pool my band, all-gather the coarse DEM, fill the whole coarse mosaic on every rank
+        nyc, nxc = -(-self.ny // 8), -(-nx // 8)
+        cp = (nxc + 31) // 32 * 32
+        zc_g = torch.empty((nyc, cp), dtype=torch.float32, device=dev.device())
+        wc_g = torch.empty((nyc, cp), dtype=torch.float32, device=dev.device())
+        cb = [(a // 8, -(-b // 8)) for a, b in self.bounds]
+        c0, c1 = cb[comm.rank]
+        scratch = torch.zeros(((c1 - c0) // 64 + 2) * (nxc // 64 + 2), dtype=torch.int32, device=dev.device())
+        own = z.owned()
+        _lib.check(lib.hd_fill_pool_band(own.ptr, own.pitch, rows, nx, ctypes.c_void_p(zc_g[c0].data_ptr()),
+                                         ctypes.c_void_p(wc_g[c0].data_ptr()), cp, flags,
+                                         ctypes.c_void_p(scratch.data_ptr()), dev.stream_ptr()))
+        for g in (zc_g, wc_g):
+            comm.p2p([(g[c0:c1], j) for j in range(comm.world) if j != comm.rank],
+                     [(g[a:b], i) for i, (a, b) in enumerate(cb) if i != comm.rank])
+        cbytes = lib.hd_pdfill_workspace_bytes(nyc, nxc)
+        cwork = dev.scratch(cbytes)
+        _lib.check(lib.hd_pdfill_coarse(ctypes.c_void_p(zc_g.data_ptr()), ctypes.c_void_p(wc_g.data_ptr()), cp, nyc, nxc,
+                                        ctypes.c_void_p(cwork.data_ptr()), cbytes, dev.stream_ptr()))
         TRACE.mark("fill: global coarse level")
         while True:
-            if rounds == 0 and wc_g is not None:
+            if rounds == 0:
                 _lib.check(lib.hd_pdfill_band_start(zv.ptr, zv.pitch, w.ptr, w.pitch, zv.ny, nx, wp, nbytes, flags,
                                                     ctypes.c_void_p(wc_g.data_ptr()), cp, self.r0 - n_up, dev.stream_ptr()))
             else:
-                _lib.check(lib.hd_pdfill_band(zv.ptr, zv.pitch, w.ptr, w.pitch, zv.ny, nx, wp, nbytes,
-                                              flags | (1 if rounds else 0), None, dev.stream_ptr()))
+                _lib.check(lib.hd_pdfill_band(zv.ptr, zv.pitch, w.ptr, w.pitch, zv.ny, nx, wp, nbytes, flags, None,
+                                              dev.stream_ptr()))
             rounds += 1
             if comm.world == 1:
                 break

@@ -336,18 +336,18 @@ int hd_max_filter_rect(const void* in, int64_t in_pitch, void* out, int64_t out_
 
 /* ---- NEW hydrology stages (not in the reference, SURVEY.md 8a N2 / N3) ----------------------------------- */
 /* Sink-fill: Planchon-Darboux fixed point with eps = 0, 8-connectivity; frame cells and NaN cells are outlets.
- * z, w: F32.  Default (max_sweeps <= 0): persistent worklist kernels with a multigrid start (coarse DEMs of 8x8 block
- * maxima are filled first: their fill is an upper bound of the answer and replaces +inf as the starting surface;
- * the result is the same unique fixed point); asynchronous and capturable in a CUDA graph unless sweeps_out is
- * given (then the stream is synchronised once and *sweeps_out = tile visits of the finest level).  max_sweeps > 0 or HD_FILL_MODE=sweep:
- * level-synchronous tile sweeps, the stream is synchronised every few sweeps, *sweeps_out = sweeps executed. */
+ * z, w: F32.  Persistent worklist kernels with a multigrid start (coarse DEMs of 8x8 block maxima are filled first:
+ * their fill is an upper bound of the answer and replaces +inf as the starting surface; the result is the same unique
+ * fixed point); asynchronous and capturable in a CUDA graph unless visits_out is given (then the stream is
+ * synchronised once and *visits_out = tile visits of the finest level). */
 int64_t hd_pdfill_workspace_bytes(int64_t ny, int64_t nx);
 int hd_pdfill(const void* z, int64_t z_pitch, void* w, int64_t w_pitch, int64_t ny, int64_t nx, void* workspace,
-              int64_t workspace_bytes, int max_sweeps, int* sweeps_out, void* stream);
-/* Row-band variant for one band of a sharded mosaic (hydrodem_b200/sharding.py): the raster passed in is
- * [halo row | band | halo row].  flags: 1 = W is already initialised (continue after a halo exchange; only the
- * tile rows next to the halo rows are re-seeded), 2 / 4 = the top / bottom row is a neighbour's halo row, not
- * raster frame.  Nodata cells stay at -inf until hd_pdfill_finish restores NaN.  *visits_out = tile visits. */
+              int64_t workspace_bytes, int* visits_out, void* stream);
+/* Next round of the row-band fill of one band of a sharded mosaic (hydrodem_b200/sharding.py), after a halo exchange:
+ * the raster passed in is [halo row | band | halo row] and W holds the previous round's result (the first round is
+ * hd_pdfill_band_start); only the tile rows next to the halo rows are re-seeded.  flags: 2 / 4 = the top / bottom row
+ * is a neighbour's halo row, not raster frame; any other bit is HD_ERR_ARG.  Nodata cells stay at -inf until
+ * hd_pdfill_finish_d8 restores NaN.  *visits_out (may be NULL) = tile visits, synchronises once. */
 int hd_pdfill_band(const void* z, int64_t z_pitch, void* w, int64_t w_pitch, int64_t ny, int64_t nx, void* workspace,
                    int64_t workspace_bytes, int flags, int* visits_out, void* stream);
 /* Fill + D8 fused: the fill, then ONE pass that restores NaN at the nodata cells and writes the D8 codes (W is not
@@ -375,7 +375,6 @@ int hd_pdfill_coarse(const void* zc, void* wc, int64_t c_pitch, int64_t nyc, int
 int hd_pdfill_band_start(const void* z, int64_t z_pitch, void* w, int64_t w_pitch, int64_t ny, int64_t nx, void* workspace,
                          int64_t workspace_bytes, int flags, const void* wc_global, int64_t c_pitch, int64_t y_origin,
                          void* stream);
-int hd_pdfill_finish(const void* z, int64_t z_pitch, void* w, int64_t w_pitch, int64_t ny, int64_t nx, void* stream);
 /* D8 flow direction on a (filled) F32 surface -> U8 ESRI codes (E=1, SE=2, S=4, SW=8, W=16, NW=32, N=64, NE=128);
  * steepest positive drop, diagonals scaled by 0.70710678f, ties -> first in that order, frame / NaN / flat -> 0. */
 int hd_d8(const void* w, int64_t w_pitch, void* out, int64_t out_pitch, int64_t ny, int64_t nx, void* stream);

@@ -61,6 +61,24 @@ def test_argument_errors_need_no_gpu(lib):
         _lib.check(_lib.HD_ERR_ARG)
 
 
+def test_fill_argument_errors_need_no_gpu(lib):
+    """The fill family rejects bad arguments before it touches the device."""
+    p = ctypes.c_void_p(1 << 20)
+    need = lib.hd_pdfill_workspace_bytes(300, 400)
+    assert lib.hd_pdfill(None, 400, p, 400, 300, 400, p, need, None, None) == _lib.HD_ERR_NULL
+    assert lib.hd_pdfill(p, 400, p, 400, 300, 400, None, need, None, None) == _lib.HD_ERR_NULL
+    assert lib.hd_pdfill(p, 399, p, 400, 300, 400, p, need, None, None) == _lib.HD_ERR_ARG
+    assert lib.hd_pdfill(p, 400, p, 400, 0, 400, p, need, None, None) == _lib.HD_ERR_ARG
+    assert lib.hd_pdfill(p, 400, p, 400, 300, 400, p, need - 1, None, None) == _lib.HD_ERR_WORKSPACE
+    # a later round continues after a halo exchange; the first round is hd_pdfill_band_start
+    for flags in (1, 3, 7, 8):
+        assert lib.hd_pdfill_band(p, 400, p, 400, 300, 400, p, need, flags, None, None) == _lib.HD_ERR_ARG
+    assert lib.hd_pdfill_band(p, 400, p, 400, 300, 400, p, need - 1, 6, None, None) == _lib.HD_ERR_WORKSPACE
+    assert lib.hd_pdfill_band_start(p, 400, p, 400, 300, 400, p, need, 1, p, 64, 0, None) == _lib.HD_ERR_ARG
+    assert lib.hd_fill_pool_band(p, 400, 300, 400, p, p, 64, 1, p, None) == _lib.HD_ERR_ARG
+    assert lib.hd_pdfill_d8(p, 400, p, 400, p, 400, 300, 400, p, need - 1, None, None) == _lib.HD_ERR_WORKSPACE
+
+
 @pytest.mark.skipif(torch.cuda.is_available(), reason="checks the no-GPU behaviour")
 def test_no_cpu_fallback(lib):
     """Without a device the product path must raise, never compute on the host."""

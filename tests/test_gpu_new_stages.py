@@ -63,13 +63,43 @@ def test_sinkfill_d8_vs_oracle(shape):
     eq(nf.SinkFill().apply(w), w)
 
 
-@pytest.mark.parametrize("mode", ["sweep", "async"])
-def test_sinkfill_modes_agree(mode, monkeypatch):
-    """Both schedules (level-synchronous sweeps, asynchronous worklist) reach the same unique fixed point."""
-    if mode == "sweep":
-        monkeypatch.setenv("HD_FILL_MODE", "sweep")
-    else:
-        monkeypatch.delenv("HD_FILL_MODE", raising=False)
+def _d8_ties(ny, nx, seed):
+    """A surface whose D8 decisions hit every special case: exact ties between a straight and a diagonal drop
+    (c = 1, straight neighbour 1 - q, diagonal neighbour 0 with q = float32(0.70710678): both drops are q), ties
+    among straight and among diagonal drops, +-0.0, NaN, +inf and -inf cells, flats with no positive drop."""
+    q = np.float32(0.70710678)
+    vals = np.array([0.0, -0.0, 1.0, 2.0, np.float32(1) - q, np.float32(2) - 2 * q, 2 * q, q], dtype=np.float32)
+    rng = np.random.default_rng(seed)
+    w = vals[rng.integers(0, len(vals), (ny, nx))]
+    special = rng.random((ny, nx))
+    w[special < 0.03] = np.nan
+    w[(special >= 0.03) & (special < 0.05)] = np.inf
+    w[(special >= 0.05) & (special < 0.07)] = -np.inf
+    return w
+
+
+def test_d8_decision_special_cases():
+    """hd_d8 against the strict-greater loop of the oracle on ties, signed zeros, NaN and infinities."""
+    w = _d8_ties(61, 83, 7)
+    want = hydrology.d8(w)
+    # the input exercises what it claims: some cell's winner ties with a later straight or diagonal direction
+    c = w[1:-1, 1:-1]
+    drops = []
+    with np.errstate(invalid="ignore"):
+        for k, (dy, dx) in enumerate(zip(hydrology.D8_DY, hydrology.D8_DX)):
+            d = (c - w[1 + dy:w.shape[0] - 1 + dy, 1 + dx:w.shape[1] - 1 + dx]).astype(np.float32)
+            drops.append((d * hydrology.INV_SQRT2_F32).astype(np.float32) if k & 1 else d)
+    drops = np.stack(drops)
+    best = np.nanmax(np.where(drops > 0, drops, np.nan), axis=0, initial=0)
+    attains = (drops == best) & (best > 0)
+    assert (attains[0::2].any(axis=0) & attains[1::2].any(axis=0)).sum() > 100      # straight-diagonal ties
+    assert (attains.sum(axis=0) > 1).sum() > 500 and (best == np.inf).sum() > 100
+    assert (want[1:-1, 1:-1] == 0).sum() > 100
+    eq(nf.D8FlowDirection().apply(w), want)
+
+
+def test_sinkfill_modes_agree():
+    """The worklist fill of an odd shape with a nodata block reaches the oracle's unique fixed point."""
     z = _terrain(515, 777, 12)
     z[100:104, 200:230] = np.nan
     eq(nf.SinkFill().apply(z), hydrology.sinkfill(z))
