@@ -18,6 +18,7 @@ HD_ERR_ALIGN, HD_ERR_CUDA, HD_ERR_UNSUPPORTED, HD_ERR_ARG, HD_ERR_WORKSPACE = -4
 U8, F32, F64, I64, C64, C128, I32, I16 = range(8)
 OP_COPY, OP_MUL, OP_ADD, OP_RSUB, OP_LT, OP_GT, OP_ABS, OP_RINT, OP_XOR, OP_TRUNC = range(10)
 MORPH_ERODE, MORPH_DILATE, MORPH_CLOSE, MORPH_OPEN = range(4)
+WARP_NEAREST, WARP_BILINEAR = range(2)
 HD_SCATTER_MAX_SEGS = 16
 
 _p, _i, _i64, _d = ctypes.c_void_p, ctypes.c_int, ctypes.c_int64, ctypes.c_double
@@ -100,6 +101,9 @@ SIGNATURES = {
     "hd_binary_morph_struct": (_i, [_p, _i, _i64, _p, _i64, _i64, _i64, _i, _i, ctypes.POINTER(_i), ctypes.POINTER(_i),
                                     _i, _p, _p]),
     "hd_max_filter_rect": (_i, [_p, _i64, _p, _i64, _i, _i64, _i64, _i, _i, _p, _i64, _p]),
+    "hd_warp": (_i, [_p, _i, _i64, _i64, _i64, ctypes.POINTER(_d), _i, _d, _p, _i64, _i64, _i64, ctypes.POINTER(_d), _i64,
+                     ctypes.POINTER(_d), _i, _p]),
+    "hd_host_tm_inverse": (_i, [ctypes.POINTER(_d), _p, _p, _i64, _p, _p]),
 }
 
 

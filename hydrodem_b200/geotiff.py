@@ -93,6 +93,28 @@ class GeoTiffInfo:
         i, j, _, x, y, _ = tie[:6]
         return (x - i * scale[0], scale[0], 0.0, y + j * scale[1], 0.0, -scale[1])
 
+    def geo_keys(self):
+        """The GeoKeyDirectory (tag 34735) as {key id: value}: a SHORT, a float / tuple of floats from GeoDoubleParams
+        (34736) or a str from GeoAsciiParams (34737, without the trailing '|').  {} when the file has no directory."""
+        d = self.values(34735)
+        if not d or len(d) < 4:
+            return {}
+        doubles, ascii_ = self.values(34736) or (), self.values(34737) or ""
+        keys = {}
+        for k in range(min(d[3], (len(d) - 4) // 4)):
+            key, loc, count, off = d[4 + 4 * k:8 + 4 * k]
+            if loc == 0:
+                keys[key] = off
+            elif loc == 34736:
+                v = tuple(doubles[off:off + count])
+                keys[key] = v[0] if count == 1 and v else v
+            elif loc == 34737:
+                keys[key] = ascii_[off:off + count].rstrip("|")
+            elif loc == 34735:
+                v = tuple(d[off:off + count])
+                keys[key] = v[0] if count == 1 and v else v
+        return keys
+
 
 def read_info(path):
     """Parse the header and the first IFD of ``path``."""
@@ -467,16 +489,38 @@ def array2raster(new_rasterfn, array, rasterfn=None):
     write_geotiff(new_rasterfn, array, like=rasterfn, dtype=np.float32)
 
 
-def process_geotiffs(srtm_tif, groves_tif, hsheds_tif, final_tif, rivers_tif=None, chain=None):
+def process_geotiffs(srtm_tif, groves_tif, hsheds_tif, final_tif, rivers_tif=None, chain=None, envelope=None):
     """HydroDEMProcess.start between its reads and its write (hydro_dem_process.py:122-153): three (four) GeoTIFFs in,
     the conditioned DEM out as a float32 GeoTIFF georeferenced like the SRTM raster.  Returns the chain's host results
-    (``final`` float64, ``filled``, ``d8``)."""
+    (``final`` float64, ``filled``, ``d8``).
+
+    ``envelope``: an ESRI shapefile of the area of interest, or a ``warp.Grid``.  The inputs (raw downloads, geographic
+    WGS84 or EPSG:22184) are then first reprojected onto the envelope's EPSG:22184 90 m grid on the device
+    (``warp.warp_to_device``, nearest neighbour: the reference's ``resample_and_cut`` step), go through the chain without
+    leaving the device, and the DEM is written with that grid's georeference."""
     from .pipeline import ConditioningChain
     chain = chain or ConditioningChain()
+    if envelope is not None:
+        return _process_on_grid(chain, srtm_tif, groves_tif, hsheds_tif, final_tif, rivers_tif, envelope)
     srtm = read_array(srtm_tif)
     groves = read_array(groves_tif)
     hsheds = read_array(hsheds_tif)
     rivers = read_array(rivers_tif) if rivers_tif else None
     out = chain.apply_to_host(srtm, groves, hsheds, rivers)
     array2raster(final_tif, out["final"], srtm_tif)
+    return out
+
+
+def _process_on_grid(chain, srtm_tif, groves_tif, hsheds_tif, final_tif, rivers_tif, envelope):
+    from . import warp
+    from .exceptions import DeviceError
+    grid = warp.as_grid(envelope)
+    paths = (srtm_tif, groves_tif, hsheds_tif) + ((rivers_tif,) if rivers_tif else ())
+    rasters = [warp.warp_to_device(p, grid) for p in paths]
+    res = chain.run_device(*rasters)
+    out = {k: res.host(k) for k in ("final", "filled", "d8") if k in res.rasters}
+    fill = res.info.get("fill")
+    if fill is not None and fill.status() != 0:
+        raise DeviceError(f"sink-fill did not reach its fixed point (status {fill.status()}): filled / d8 are invalid")
+    write_geotiff(final_tif, out["final"], dtype=np.float32, geo_tags=grid.geo_tags())
     return out

@@ -379,6 +379,25 @@ int hd_pdfill_band_start(const void* z, int64_t z_pitch, void* w, int64_t w_pitc
  * steepest positive drop, diagonals scaled by 0.70710678f, ties -> first in that order, frame / NaN / flat -> 0. */
 int hd_d8(const void* w, int64_t w_pitch, void* out, int64_t out_pitch, int64_t ny, int64_t nx, void* stream);
 
+/* ---- reprojection onto the EPSG:22184 grid: utils_dem.resample_and_cut, utils_dem.py:65-84 (gdal.Warp) ------------ */
+typedef enum { HD_WARP_NEAREST = 0, HD_WARP_BILINEAR = 1 } hd_warp_resample;
+/* Fill the F32 destination raster dst (dst_ny x dst_nx, rows dst_row0 ... of the grid dst_geo describes) from src
+ * (U8 / I16 / F32).  Grids: HOST double[4] (x0, dx, y0, dy) of the top-left pixel corner, north up, dx, dy > 0.
+ * Per destination cell: centre (x0 + (i + 1/2) dx, y0 - (dst_row0 + j + 1/2) dy); if tm (HOST double[7] a, f, lat0,
+ * lon0, k0, FE, FN; degrees and metres) is not NULL, inverse Transverse Mercator (Krueger series to n^6, float64) to
+ * (lon, lat) degrees; NULL: the source is in the destination CRS.  Source pixel coordinates u = (lon - sx0) / sdx,
+ * v = (sy0 - lat) / sdy.  Nearest: the cell (floor u, floor v).  Bilinear: taps floor(u - 1/2), floor(v - 1/2) and their
+ * +1 neighbours; taps outside the source or equal to nodata are dropped and the remaining weights renormalised.  A cell
+ * with no valid sample gets nodata (has_nodata) or 0.  Allocates nothing; asynchronous and capturable.  Empty grids,
+ * pitches below a row, dst_row0 < 0, non-positive pixel sizes, an unknown resampling code or a tm block that describes no
+ * ellipsoid -> HD_ERR_ARG. */
+int hd_warp(const void* src, int src_dtype, int64_t src_pitch, int64_t src_ny, int64_t src_nx, const double* src_geo,
+            int has_nodata, double nodata, void* dst, int64_t dst_pitch, int64_t dst_ny, int64_t dst_nx, const double* dst_geo,
+            int64_t dst_row0, const double* tm, int resample, void* stream);
+/* HOST: the same inverse Transverse Mercator as hd_warp, on n points (x, y metres -> lon, lat degrees); the host API uses it
+ * to check that a destination grid overlaps its source before any device work. */
+int hd_host_tm_inverse(const double* tm, const double* x, const double* y, int64_t n, double* lon, double* lat);
+
 #ifdef __cplusplus
 }
 #endif
