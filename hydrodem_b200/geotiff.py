@@ -513,14 +513,14 @@ def process_geotiffs(srtm_tif, groves_tif, hsheds_tif, final_tif, rivers_tif=Non
 
 def _process_on_grid(chain, srtm_tif, groves_tif, hsheds_tif, final_tif, rivers_tif, envelope):
     from . import warp
-    from .exceptions import DeviceError
+    from .pipeline import check_fill_status
     grid = warp.as_grid(envelope)
     paths = (srtm_tif, groves_tif, hsheds_tif) + ((rivers_tif,) if rivers_tif else ())
     rasters = [warp.warp_to_device(p, grid) for p in paths]
     res = chain.run_device(*rasters)
     out = {k: res.host(k) for k in ("final", "filled", "d8") if k in res.rasters}
     fill = res.info.get("fill")
-    if fill is not None and fill.status() != 0:
-        raise DeviceError(f"sink-fill did not reach its fixed point (status {fill.status()}): filled / d8 are invalid")
+    if fill is not None:
+        check_fill_status(fill.status())
     write_geotiff(final_tif, out["final"], dtype=np.float32, geo_tags=grid.geo_tags())
     return out

@@ -63,6 +63,32 @@ class CapturedChain:
         return self.result
 
 
+def copy_streams(owner):
+    """The (upload, download) copy streams of ``owner`` (a chain or a band), created on first use and kept on it."""
+    streams = owner.__dict__.get("_copy_streams")
+    if streams is None:
+        import torch
+        streams = owner._copy_streams = (torch.cuda.Stream(), torch.cuda.Stream())
+    return streams
+
+
+def host_threads():
+    """Host threads that widen int16 results: the cores this process may use, shared by the ranks of the box."""
+    local = int(os.environ.get("LOCAL_WORLD_SIZE", "1") or 1)
+    return max(1, min(16, len(os.sched_getaffinity(0)) // max(local, 1)))
+
+
+def narrow_final_default():
+    """Whether the eager host calls send the final DEM (integer metres) down as int16 (HD_NARROW_FINAL=0: float64)."""
+    return os.environ.get("HD_NARROW_FINAL", "1") != "0"
+
+
+def check_fill_status(status):
+    """Raise DeviceError unless ``status`` (the sink-fill's sticky status word) says the fixed point was reached."""
+    if status != 0:
+        raise DeviceError(f"sink-fill did not reach its fixed point (status {status}): filled / d8 are invalid")
+
+
 class _StreamSlot:
     """One pipeline slot of ConditioningChain.stream: static input rasters, the chain captured as CUDA-graph
     segments (split where an input is first needed / an output is complete) and the events that order the three
@@ -75,9 +101,7 @@ class _StreamSlot:
         lib = _lib.load()
         self.chain = chain
         self.cur = torch.cuda.current_stream()
-        if not hasattr(chain, "_streams"):
-            chain._streams = (torch.cuda.Stream(), torch.cuda.Stream())
-        self.up, self.down = chain._streams
+        self.up, self.down = copy_streams(chain)
         self.names = [n for n in self.ORDER if n in arrays]
         self.inputs = {n: dev.empty(*arrays[n].shape, dev.hd_dtype_of(arrays[n].dtype), arrays[n].dtype)
                        for n in self.names}
@@ -134,10 +158,7 @@ class _StreamSlot:
                 self.flags[src] = torch.zeros(1, dtype=torch.int32, device=r.buf.device)
         size = lambda t: t.numel() * t.element_size()
         self.transfer_bytes = (sum(size(t) for t in self.dense_in.values()), sum(size(t) for t in self.dense_out.values()))
-        local = int(os.environ.get("LOCAL_WORLD_SIZE", "1") or 1)
-        self.host_threads = max(1, min(16, len(os.sched_getaffinity(0)) // max(local, 1)))
-        if os.environ.get("HD_HOST_THREADS"):
-            self.host_threads = max(1, int(os.environ["HD_HOST_THREADS"]))
+        self.host_threads = host_threads()
         self.ev_compute = self.ev_down = None
         self.keep = None
 
@@ -249,7 +270,7 @@ class _StreamSlot:
                     # not int16-representable: fetch the float32 raster itself (still intact: the slot is not reused
                     # before this tile has been collected)
                     arr = dev.download(raster.with_ref(np_dtype))
-                elif arr.dtype != np_dtype and not os.environ.get("HD_STREAM_NO_WIDEN"):   # int16 -> float32 / float64 on host threads (the switch is for bandwidth experiments only)
+                elif arr.dtype != np_dtype:                          # int16 -> float32 / float64 on host threads
                     wide = dev.pinned_empty(arr.shape, np_dtype)
                     _lib.check(lib.hd_host_widen_i16(ctypes.c_void_p(wide.ctypes.data), dev.hd_dtype_of(np_dtype),
                                                      ctypes.c_void_p(arr.ctypes.data), arr.size, self.host_threads))
@@ -265,7 +286,7 @@ class NarrowDownload:
     cores as it lands -- underneath the sink-fill and the download of the filled DEM.  hd_pack_i16 raises a device flag
     if any value is not an int16 integer; ``result()`` fetches the float64 raster itself then.  Same bits either way."""
 
-    def __init__(self, raster, cur, down, threads=None, chunks=8):
+    def __init__(self, raster, cur, down, chunks=8):
         import threading
         import torch
         lib = _lib.load()
@@ -301,9 +322,7 @@ class NarrowDownload:
         self._last_copy, self._host16 = parts[-1][2], host16
         self.state = state = {"inexact": False, "error": None}
         device_index = torch.cuda.current_device()
-        if threads is None:
-            local = int(os.environ.get("LOCAL_WORLD_SIZE", "1") or 1)
-            threads = max(1, min(16, len(os.sched_getaffinity(0)) // max(local, 1)))
+        threads = host_threads()
 
         def widen():
             try:
@@ -332,6 +351,52 @@ class NarrowDownload:
         return self.wide
 
 
+def overlapped_to_host(streams, inputs, run, narrow_final):
+    """The eager ``apply_to_host`` of ConditioningChain and of Band: host arrays in and out, the PCIe traffic underneath
+    the kernels.  ``inputs``: ``(name, host ndarray, destination raster or None)`` in the order the chain first needs
+    them, uploaded on ``streams[0]`` (into a new raster without a destination).  ``run(rasters, ready, on_ready)``
+    enqueues the chain (waiting for ``ready[name]`` where an input is first used, calling ``on_ready(name, raster)``
+    when an output is enqueued) and returns a function that reads the sink-fill's status word, or None.  Outputs go down
+    on ``streams[1]`` at once, the final DEM as int16 when ``narrow_final``.  Returns the ndarrays and the (H2D, D2H)
+    bytes."""
+    import torch
+    cur = torch.cuda.current_stream()
+    up, down = streams
+    up.wait_stream(cur)                                   # recycled blocks: earlier work on them is over
+    rasters, ready = {}, {}
+    for name, host, into in inputs:
+        if into is None:
+            rasters[name], ready[name] = dev.upload_async(host, up)
+        else:
+            rasters[name], ready[name] = into, dev.upload_into(into, host, up)
+        if not dev._is_pinned(host):
+            up.synchronize()                              # a pageable source may be released by the caller
+    pending, narrow = {}, {}
+
+    def on_ready(name, raster):
+        if narrow_final and raster.dtype == _lib.F32 and raster.ref_dtype == np.float64:
+            narrow[name] = NarrowDownload(raster, cur, down)
+            return
+        conv = dev.convert(raster, dev.hd_dtype_of(raster.ref_dtype))
+        ev = torch.cuda.Event()
+        ev.record(cur)
+        down.wait_event(ev)
+        pending[name] = dev.download_async(conv, down) + (conv,)
+
+    fill_status = run(rasters, ready, on_ready)
+    out = {}
+    for name, (host, ev, _conv) in pending.items():
+        ev.synchronize()
+        out[name] = host
+    for name, nd in narrow.items():
+        out[name] = nd.result()
+    if fill_status is not None:
+        check_fill_status(fill_status())
+    transfer = (sum(host.nbytes for _, host, _ in inputs),
+                sum(out[name].nbytes for name in pending) + sum(nd.nbytes + nd.extra_bytes for nd in narrow.values()))
+    return {k: out[k] for k in ("final", "filled", "d8") if k in out}, transfer
+
+
 class ConditioningChain:
     """Run the whole chain on the GPU.
 
@@ -345,7 +410,7 @@ class ConditioningChain:
         # apply_to_host: rasters of at least this many cells run eagerly on three streams instead of captured slots
         self.eager_cells = int(os.environ.get("HD_EAGER_CELLS", str(64 << 20)))
         # ... and send the final DEM (integer metres) down as int16, widened to float64 by host threads as it lands
-        self.narrow_final = os.environ.get("HD_NARROW_FINAL", "1") != "0"
+        self.narrow_final = narrow_final_default()
         self.sparse_groves = sparse_groves    # False: every groves iteration rewrites the whole raster (tests compare both)
         self.keep_complete = keep_complete    # also return / keep the float64 sum of the final terms ("dem_complete")
         self.fused_combine = fused_combine    # False: hd_final_terms + hd_convolve3 as two kernels (tests compare both)
@@ -586,11 +651,7 @@ class ConditioningChain:
 
     # ---- host API ---------------------------------------------------------------------------------
     def upload_inputs(self, srtm_raw, groves_class_raw, hsheds, rivers=None):
-        for a in (srtm_raw, groves_class_raw, hsheds) + ((rivers,) if rivers is not None else ()):
-            if not isinstance(a, np.ndarray):
-                raise NumpyArrayExpectedError(a)
-        if not (srtm_raw.shape == groves_class_raw.shape == hsheds.shape):
-            raise ValueError("srtm, groves_class and hsheds must have the same shape")
+        self._check_inputs(srtm_raw, groves_class_raw, hsheds, rivers)
         return (dev.upload(srtm_raw), dev.upload(groves_class_raw), dev.upload(hsheds),
                 dev.upload(rivers) if rivers is not None else None)
 
@@ -617,50 +678,14 @@ class ConditioningChain:
         nothing against 160 ms of kernels.  Timeline at 36000^2 on PCIe 5: SRTM up (94 ms) | Fourier stage under the
         HydroSHEDS upload (94 ms) | lagoon branch under the groves upload (24 ms) | groves, final terms | final DEM
         down as int16 (47 ms) over the sink-fill, widened on the host underneath | filled DEM + D8 down (118 ms)."""
-        import torch
-        cur = torch.cuda.current_stream()
-        if not hasattr(self, "_streams"):
-            self._streams = (torch.cuda.Stream(), torch.cuda.Stream())
-        up, down = self._streams
-        up.wait_stream(cur)                                   # recycled blocks: earlier work on them is over
-        rasters, ready, keep = {}, {}, []
-        for name in ("srtm", "hsheds", "groves", "rivers"):   # the order run_device first needs them in
-            if name not in arrays:
-                continue
-            host = np.ascontiguousarray(arrays[name])
-            rasters[name], ready[name] = dev.upload_async(host, up)
-            if not dev._is_pinned(host):
-                up.synchronize()                              # a pageable source may be released by the caller
-            keep.append(host)
-        pending, narrow = {}, {}
-        lib = _lib.load()
-        d2h_bytes = [0]
+        order = ("srtm", "hsheds", "groves", "rivers")                # the order run_device first needs them in
+        inputs = [(n, np.ascontiguousarray(arrays[n]), None) for n in order if n in arrays]
 
-        def send(name, raster):
-            if self.narrow_final and raster.dtype == _lib.F32 and raster.ref_dtype == np.float64:
-                return send_narrow(name, raster)
-            conv = dev.convert(raster, dev.hd_dtype_of(raster.ref_dtype))
-            ev = torch.cuda.Event()
-            ev.record(cur)
-            down.wait_event(ev)
-            pending[name] = dev.download_async(conv, down) + (conv,)
-            d2h_bytes[0] += pending[name][0].nbytes
+        def run(rasters, ready, on_ready):
+            res = self.run_device(rasters["srtm"], rasters["groves"], rasters["hsheds"], rasters.get("rivers"),
+                                  ready=ready, on_ready=on_ready)
+            fill = res.info.get("fill")
+            return fill.status if fill is not None else None
 
-        def send_narrow(name, raster):
-            narrow[name] = NarrowDownload(raster, cur, down)
-            d2h_bytes[0] += narrow[name].nbytes
-
-        res = self.run_device(rasters["srtm"], rasters["groves"], rasters["hsheds"], rasters.get("rivers"), ready=ready,
-                              on_ready=send)
-        out = {}
-        for name, (host, ev, _conv) in pending.items():
-            ev.synchronize()
-            out[name] = host
-        for name, nd in narrow.items():
-            out[name] = nd.result()
-            d2h_bytes[0] += nd.extra_bytes
-        fill = res.info.get("fill")
-        if fill is not None and fill.status() != 0:
-            raise DeviceError(f"sink-fill did not reach its fixed point (status {fill.status()}): filled / d8 are invalid")
-        self.last_transfer_bytes = (sum(h.nbytes for h in keep), d2h_bytes[0])
-        return {k: out[k] for k in ("final", "filled", "d8") if k in out}
+        out, self.last_transfer_bytes = overlapped_to_host(copy_streams(self), inputs, run, self.narrow_final)
+        return out

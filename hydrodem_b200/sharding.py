@@ -396,7 +396,8 @@ class Band:
             raise ValueError(f"{ny} rows over {comm.world} ranks leave bands thinner than the {self.halo}-row halo")
         import os
         self.fill_overlap = max(8, int(os.environ.get("HD_FILL_OVERLAP", "64")) // 8 * 8)
-        self.narrow_final = os.environ.get("HD_NARROW_FINAL", "1") != "0"   # apply_to_host: final DEM down as int16
+        from .pipeline import narrow_final_default
+        self.narrow_final = narrow_final_default()                       # apply_to_host: final DEM down as int16
         if comm.world > 1 and min(b - a for a, b in self.bounds) < 2 * self.fill_overlap:
             self.fill_overlap = max(8, min(b - a for a, b in self.bounds) // 16 * 8)
         self.up, self.down = self._margins(comm.rank)
@@ -819,60 +820,24 @@ class Band:
         """The banded chain through host buffers: this rank's rows of the three input mosaics (ndarrays: float32,
         uint8 / bool, float32; pinned memory is copied asynchronously) -> {"final" float64, "filled" float32, "d8" uint8}
         ndarrays of the same rows.  What bench.py's e2e measures at N > 1."""
-        import torch
+        from .pipeline import copy_streams, overlapped_to_host
         for a in (srtm_rows, groves_rows, hsheds_rows):
             if not isinstance(a, np.ndarray):
                 from .exceptions import NumpyArrayExpectedError
                 raise NumpyArrayExpectedError(a)
             if a.shape != (self.rows, self.nx):
                 raise ValueError(f"expected this rank's rows {(self.rows, self.nx)}, got {a.shape}")
-        # three streams: the SRTM rows go up first, groves + HydroSHEDS follow underneath the Fourier stage, and the
-        # final DEM travels down while the sink-fill rounds run (what ConditioningChain.apply_to_host does on one GPU)
-        cur = torch.cuda.current_stream()
-        if not hasattr(self, "_copy_streams"):
-            self._copy_streams = (torch.cuda.Stream(), torch.cuda.Stream())
-        up, down = self._copy_streams
+        # the SRTM rows go up first, HydroSHEDS + groves follow underneath the Fourier stage, straight into the owned rows
+        # of their extended rasters, and the final DEM travels down while the sink-fill rounds run
         g_ext, h_ext = self.alloc_ext(_lib.U8, np.uint8), self.alloc_ext(_lib.F32, np.float32)
-        up.wait_stream(cur)
-        ready, keep = {}, []
-
-        def send_up(name, host, into=None):
-            if into is None:
-                r, ready[name] = dev.upload_async(host, up)
-            else:
-                r, ready[name] = into, dev.upload_into(into, host, up)
-            if not dev._is_pinned(host):
-                up.synchronize()                              # a pageable source may be released by the caller
-            keep.append(host)
-            return r
-
-        srtm = send_up("srtm", np.ascontiguousarray(srtm_rows, dtype=np.float32))
-        send_up("hsheds", np.ascontiguousarray(hsheds_rows, dtype=np.float32), h_ext.owned())
         g = np.ascontiguousarray(groves_rows)
-        send_up("groves", g.view(np.uint8) if g.dtype == np.bool_ else g.astype(np.uint8, copy=False), g_ext.owned())
-        pending = {}
+        inputs = [("srtm", np.ascontiguousarray(srtm_rows, dtype=np.float32), None),
+                  ("hsheds", np.ascontiguousarray(hsheds_rows, dtype=np.float32), h_ext.owned()),
+                  ("groves", g.view(np.uint8) if g.dtype == np.bool_ else g.astype(np.uint8, copy=False), g_ext.owned())]
 
-        narrow = {}
+        def run(rasters, ready, on_ready):
+            self.conditioning_chain(rasters["srtm"], g_ext, h_ext, ready=ready, on_ready=on_ready)
+            return self.fill_status
 
-        def send_down(name, raster):
-            if self.narrow_final and raster.dtype == _lib.F32 and raster.ref_dtype == np.float64:
-                from .pipeline import NarrowDownload
-                narrow[name] = NarrowDownload(raster, cur, down)        # int16 over PCIe, widened on host threads
-                return
-            conv = dev.convert(raster, dev.hd_dtype_of(raster.ref_dtype))
-            ev = torch.cuda.Event()
-            ev.record(cur)
-            down.wait_event(ev)
-            pending[name] = dev.download_async(conv, down) + (conv,)
-
-        self.conditioning_chain(srtm, g_ext, h_ext, ready=ready, on_ready=send_down)
-        out = {}
-        for name, (host, ev, _conv) in pending.items():
-            ev.synchronize()
-            out[name] = host
-        for name, nd in narrow.items():
-            out[name] = nd.result()
-        self.last_transfer_bytes = (sum(h.nbytes for h in keep),
-                                    sum(h.nbytes for h, _e, _c in pending.values())
-                                    + sum(nd.nbytes + nd.extra_bytes for nd in narrow.values()))
-        return {k: out[k] for k in ("final", "filled", "d8")}
+        out, self.last_transfer_bytes = overlapped_to_host(copy_streams(self), inputs, run, self.narrow_final)
+        return out

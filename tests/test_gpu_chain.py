@@ -165,6 +165,19 @@ def test_apply_to_host_matches_lazy_path():
     assert chain.last_transfer_bytes[1] == 8 * srtm.size + 4 * srtm.size + srtm.size
 
 
+def test_apply_to_host_raises_on_a_stalled_fill(monkeypatch):
+    """The eager host call raises DeviceError when the sink-fill did not reach its fixed point.  The status word is
+    faked on the host: no fill is made to stall."""
+    from hydrodem_b200.exceptions import DeviceError
+    from hydrodem_b200.filters import new_filters as nf
+    sc = SynthScene(200, 260, 6)
+    chain = ConditioningChain()
+    chain.eager_cells = 0
+    monkeypatch.setattr(nf.SinkFillD8, "status", lambda self: 1)
+    with pytest.raises(DeviceError, match="fixed point"):
+        chain.apply_to_host(sc.srtm(), sc.groves(), sc.hsheds())
+
+
 def test_captured_graph_matches_eager():
     """Replaying the captured CUDA graph gives the same bits as eager launches, also after the inputs changed."""
     from hydrodem_b200 import device as dev

@@ -118,11 +118,17 @@ def test_banded_chain_is_bit_identical(world, shape, direct, monkeypatch):
 @pytest.mark.parametrize("world", [2, 3])
 def test_banded_apply_to_host_is_bit_identical(world):
     """Band.apply_to_host (copies on their own streams, underneath the kernels) returns the single-GPU bits; pageable and
-    pinned inputs, called twice (recycled buffers)."""
+    pinned inputs, called twice (recycled buffers), the final DEM sent as int16 and as float64, and a final DEM outside
+    int16 (the device flag makes the int16 transport fetch the float64 raster after all).  Every rank counts the PCIe
+    bytes of its rows: the three inputs up; the final DEM (int16 + a 4-byte flag, or float64), filled (float32), d8
+    down."""
     from hydrodem_b200.pipeline import ConditioningChain
     sc = SynthScene(420, 333, 83)
     srtm, groves, hsheds = sc.srtm(), sc.groves(), sc.hsheds()
     ref = ConditioningChain().apply(srtm, groves, hsheds.copy())
+    srtm_hi, hsheds_hi = srtm + np.float32(40000), hsheds + np.float32(40000)
+    ref_hi = ConditioningChain().apply(srtm_hi, groves, hsheds_hi.copy())
+    assert ref_hi.final.max() > 32767
 
     def fn(comm):
         band = sharding.Band(comm, *srtm.shape)
@@ -132,15 +138,44 @@ def test_banded_apply_to_host_is_bit_identical(world):
             p = dev.pinned_empty(a.shape, a.dtype)
             p[...] = a
             pinned.append(p)
-        a = band.apply_to_host(*rows)
-        b = band.apply_to_host(*pinned)
-        b = {k: v.copy() for k, v in band.apply_to_host(*pinned).items()}
-        return a, b
+        out, sent = {}, {}
+        out["pageable"] = band.apply_to_host(*rows)
+        sent["pageable"] = band.last_transfer_bytes
+        band.apply_to_host(*pinned)
+        out["pinned"] = {k: v.copy() for k, v in band.apply_to_host(*pinned).items()}
+        sent["pinned"] = band.last_transfer_bytes
+        out["high"] = band.apply_to_host(band.take(srtm_hi), rows[1], band.take(hsheds_hi))
+        sent["high"] = band.last_transfer_bytes
+        band.narrow_final = False
+        out["float64"] = band.apply_to_host(*pinned)
+        sent["float64"] = band.last_transfer_bytes
+        return out, sent, sum(a.nbytes for a in rows), band.rows * band.nx
 
     res = sharding.ThreadComm.run(world, fn)
-    for which in (0, 1):
-        got = {k: np.concatenate([r[which][k] for r in res]) for k in ("final", "filled", "d8")}
+    for which, want in (("pageable", ref), ("pinned", ref), ("high", ref_hi), ("float64", ref)):
+        got = {k: np.concatenate([r[0][which][k] for r in res]) for k in ("final", "filled", "d8")}
         assert got["final"].dtype == np.float64 and got["filled"].dtype == np.float32 and got["d8"].dtype == np.uint8
-        np.testing.assert_array_equal(got["final"], ref.final)
-        np.testing.assert_array_equal(got["filled"], ref.filled)
-        np.testing.assert_array_equal(got["d8"], ref.d8)
+        np.testing.assert_array_equal(got["final"], want.final)
+        np.testing.assert_array_equal(got["filled"], want.filled)
+        np.testing.assert_array_equal(got["d8"], want.d8)
+    for _, sent, h2d, cells in res:
+        assert sent["pageable"] == sent["pinned"] == (h2d, 2 * cells + 4 + 4 * cells + cells)
+        assert sent["high"] == (h2d, 2 * cells + 4 + 8 * cells + 4 * cells + cells)     # int16 + flag, then float64
+        assert sent["float64"] == (h2d, 8 * cells + 4 * cells + cells)
+
+
+def test_banded_apply_to_host_raises_on_a_stalled_fill(monkeypatch):
+    """A banded run whose sink-fill did not reach its fixed point raises DeviceError on every rank instead of returning
+    the poisoned surface.  The status word is faked on the host: no fill is made to stall."""
+    from hydrodem_b200.exceptions import DeviceError
+    sc = SynthScene(420, 333, 83)
+    srtm, groves, hsheds = sc.srtm(), sc.groves(), sc.hsheds()
+    monkeypatch.setattr(sharding.Band, "fill_status", lambda self: 1)
+
+    def fn(comm):
+        band = sharding.Band(comm, *srtm.shape)
+        with pytest.raises(DeviceError, match="fixed point"):
+            band.apply_to_host(band.take(srtm), band.take(groves), band.take(hsheds))
+        return True
+
+    assert sharding.ThreadComm.run(2, fn) == [True, True]
