@@ -104,6 +104,10 @@ SIGNATURES = {
     "hd_warp": (_i, [_p, _i, _i64, _i64, _i64, ctypes.POINTER(_d), _i, _d, _p, _i64, _i64, _i64, ctypes.POINTER(_d), _i64,
                      ctypes.POINTER(_d), _i, _p]),
     "hd_host_tm_inverse": (_i, [ctypes.POINTER(_d), _p, _p, _i64, _p, _p]),
+    "hd_host_tm_forward": (_i, [ctypes.POINTER(_d), _p, _p, _i64, _p, _p]),
+    "hd_rasterize_workspace_bytes": (_i64, [_i64]),
+    "hd_rasterize_lines": (_i, [_p, _p, _i64, _p, _p, _i64, _p, _i64, _p, _i64, _i64, _i64, ctypes.POINTER(_d), _i64,
+                                ctypes.POINTER(_d), _p, _i64, _p]),
 }
 
 

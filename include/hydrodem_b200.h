@@ -397,6 +397,30 @@ int hd_warp(const void* src, int src_dtype, int64_t src_pitch, int64_t src_ny, i
 /* HOST: the same inverse Transverse Mercator as hd_warp, on n points (x, y metres -> lon, lat degrees); the host API uses it
  * to check that a destination grid overlaps its source before any device work. */
 int hd_host_tm_inverse(const double* tm, const double* x, const double* y, int64_t n, double* lon, double* lat);
+/* HOST: the forward Transverse Mercator hd_rasterize_lines applies to geographic vertices, on n points (lon, lat degrees ->
+ * x, y metres): the Krueger series to n^6, summed by the same Clenshaw routine as the inverse. */
+int hd_host_tm_forward(const double* tm, const double* lon, const double* lat, int64_t n, double* x, double* y);
+
+/* ---- line rasterization onto the EPSG:22184 grid: rasterize_rivers, utils_dem.py:183-191 (gdal.RasterizeLayer) ------ */
+/* DEVICE workspace bytes hd_rasterize_lines needs for n_vertices vertices (0 for n_vertices < 0 or above 2^38). */
+int64_t hd_rasterize_workspace_bytes(int64_t n_vertices);
+/* Burn polylines into the F32 destination dst (dst_ny x dst_nx, rows dst_row0 ... of the grid dst_geo describes; HOST
+ * double[4] (x0, dx, y0, dy) as for hd_warp).  DEVICE inputs: vx, vy (double[n_vertices]; lon / lat degrees when tm, a
+ * HOST double[7] as for hd_warp, is not NULL, else EPSG:22184 metres), part_start (int64[n_parts + 1], non-decreasing;
+ * part p is vertices [part_start[p], part_start[p + 1])), part_feature (int32[n_parts], the feature of each part) and
+ * values (float[n_features]).  A vertex has pixel (floor((X - x0) / dx), floor((y0 - Y) / dy)), rows in the full grid's
+ * frame; a non-finite vertex, one with |latitude| > 90, or one whose pixel coordinate is 2^29 or more in magnitude burns no
+ * segment.  Each segment of a part is walked by GDAL's integer Bresenham (GDALdllImageLine: major axis x when
+ * |dx| >= |dy|, max(|dx|, |dy|) + 1 pixels, both ends burned, minor offset after k steps
+ * floor((2 k |d_minor| + |d_major| - 1) / (2 |d_major|))); pixels outside dst are dropped.  A cell takes the value of the
+ * last feature (largest index) whose walk touches it, 0 when none does.  Allocates nothing, never synchronises, capturable.
+ * Workspace: hd_rasterize_workspace_bytes(n_vertices).  Counts < 0, n_vertices > 2^38, n_features > 2^31 - 1, an empty
+ * grid, a pitch below a row, dst_row0 < 0, columns or rows at or beyond 2^29, non-positive pixel sizes or a tm block that
+ * describes no ellipsoid -> HD_ERR_ARG. */
+int hd_rasterize_lines(const void* vx, const void* vy, int64_t n_vertices, const void* part_start, const void* part_feature,
+                       int64_t n_parts, const void* values, int64_t n_features, void* dst, int64_t dst_pitch, int64_t dst_ny,
+                       int64_t dst_nx, const double* dst_geo, int64_t dst_row0, const double* tm, void* workspace,
+                       int64_t workspace_bytes, void* stream);
 
 #ifdef __cplusplus
 }
