@@ -15,7 +15,7 @@ LIB_PATH = os.path.join(_HERE, "libhydrodem_b200.so")
 # hd_status / hd_dtype / op codes (mirrors of the header enums)
 HD_OK, HD_ERR_NULL, HD_ERR_WINDOW_HIGH, HD_ERR_WINDOW_EVEN = 0, -1, -2, -3
 HD_ERR_ALIGN, HD_ERR_CUDA, HD_ERR_UNSUPPORTED, HD_ERR_ARG, HD_ERR_WORKSPACE = -4, -5, -6, -7, -8
-U8, F32, F64, I64, C64, C128, I32, I16 = range(8)
+U8, F32, F64, I64, C64, C128, I32, I16, BOOL = range(9)
 OP_COPY, OP_MUL, OP_ADD, OP_RSUB, OP_LT, OP_GT, OP_ABS, OP_RINT, OP_XOR, OP_TRUNC = range(10)
 MORPH_ERODE, MORPH_DILATE, MORPH_CLOSE, MORPH_OPEN = range(4)
 WARP_NEAREST, WARP_BILINEAR = range(2)
@@ -43,7 +43,7 @@ SIGNATURES = {
     "hd_host_lzw_decode": (_i64, [_p, _i64, _p, _i64]),
     "hd_confusion_counts": (_i, [_p, _i, _i64, _p, _i, _i64, _i64, _i64, ctypes.c_double, _p, _p]),
     "hd_pack_i16": (_i, [_p, _i64, _p, _i64, _i64, _p, _p]),
-    "hd_elementwise": (_i, [_i, _p, _i, _i64, _p, _i, _i64, _d, _p, _i, _i64, _i64, _i64, _p]),
+    "hd_elementwise": (_i, [_i, _p, _i, _i64, _p, _i, _i64, _p, _i, _p, _i, _i64, _i64, _i64, _p]),
     "hd_final_terms": (_i, [_p, _i, _i64, _p, _i64, _p, _i64, _p, _i64, _p, _i, _i64, _i64, _i64, _p]),
     "hd_final_mean3": (_i, [_p, _i64, _p, _i64, _p, _i64, _p, _i64, _p, _i64, _i64, _i64, _p]),
     "hd_expand": (_i, [_p, _i, _i64, _p, _i, _i64, _i64, _i64, _i, _p]),

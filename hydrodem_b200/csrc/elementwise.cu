@@ -2,112 +2,234 @@
 // dtype-generic kernel.  These are HBM-bound streaming ops; inside the fused chain they never run alone
 // (they are folded into the neighbouring stencil kernels) -- this entry point exists so that each
 // reference class has a device implementation behind the same Filter.apply() API.
+#include <cstring>
+#include <type_traits>
+
 #include "common.cuh"
 #include "tile_common.cuh"
 
 namespace {
 
-struct cplx { double re, im; };
+// Every op is evaluated in the dtype of NumPy's ufunc loop (the compute type C): both operands are converted to C
+// as ndarray.astype would, the op runs in C with NumPy's semantics, and the result is converted to out_dtype.
+struct cf { float re, im; };
+struct cd { double re, im; };
+template <typename T> constexpr bool is_cplx = std::is_same_v<T, cf> || std::is_same_v<T, cd>;
+template <typename T> using part_t = std::conditional_t<std::is_same_v<T, cf>, float, double>;
+// integer arithmetic wraps: done on unsigned words at least as wide as int, so no promotion overflows
+template <typename T> using word_t = std::conditional_t<sizeof(T) == 8, uint64_t, uint32_t>;
 
-__device__ __forceinline__ cplx load_as(const void* p, int dtype, int64_t idx)
+template <typename S> __device__ __forceinline__ bool nonzero(S v)
 {
-    switch (dtype) {
-        case HD_U8: return {(double)((const uint8_t*)p)[idx], 0.0};
-        case HD_F32: return {(double)((const float*)p)[idx], 0.0};
-        case HD_F64: return {((const double*)p)[idx], 0.0};
-        case HD_I64: return {(double)((const int64_t*)p)[idx], 0.0};
-        case HD_I32: return {(double)((const int32_t*)p)[idx], 0.0};
-        case HD_I16: return {(double)((const int16_t*)p)[idx], 0.0};
-        case HD_C64: { float2 v = ((const float2*)p)[idx]; return {(double)v.x, (double)v.y}; }
-        default: { double2 v = ((const double2*)p)[idx]; return {v.x, v.y}; }
-    }
-}
-__device__ __forceinline__ int64_t load_int(const void* p, int dtype, int64_t idx)
-{
-    switch (dtype) {
-        case HD_U8: return ((const uint8_t*)p)[idx];
-        case HD_I32: return ((const int32_t*)p)[idx];
-        case HD_I16: return ((const int16_t*)p)[idx];
-        default: return ((const int64_t*)p)[idx];
-    }
-}
-__device__ __forceinline__ void store_as(void* p, int dtype, int64_t idx, cplx v)
-{
-    switch (dtype) {
-        case HD_U8: ((uint8_t*)p)[idx] = (uint8_t)v.re; break;
-        case HD_F32: ((float*)p)[idx] = (float)v.re; break;
-        case HD_F64: ((double*)p)[idx] = v.re; break;
-        case HD_I64: ((int64_t*)p)[idx] = (int64_t)v.re; break;
-        case HD_I32: ((int32_t*)p)[idx] = (int32_t)v.re; break;
-        case HD_I16: ((int16_t*)p)[idx] = (int16_t)(int32_t)v.re; break;
-        case HD_C64: ((float2*)p)[idx] = make_float2((float)v.re, (float)v.im); break;
-        default: ((double2*)p)[idx] = make_double2(v.re, v.im); break;
-    }
+    if constexpr (is_cplx<S>) return v.re != 0 || v.im != 0;
+    else return v != 0;                                               // NaN is non-zero
 }
 
-__global__ void __launch_bounds__(256) elementwise_kernel(int op, const void* __restrict__ a, int a_dtype,
-                                                          int64_t a_pitch, const void* __restrict__ b, int b_dtype,
-                                                          int64_t b_pitch, double b_scalar, void* __restrict__ out,
-                                                          int out_dtype, int64_t out_pitch, int64_t ny, int64_t nx)
+// ndarray.astype(T): round to nearest between floats and from integers, truncate a float toward zero into an
+// integer (then wrap into a narrower one), `!= 0` into bool, drop the imaginary part into a real type
+template <typename T, typename S> __device__ __forceinline__ T cvt(S v)
 {
-    for (CellIter it(nx); it.y < ny; it.next()) {
-        const int64_t y = (int64_t)it.y, x = (int64_t)it.x;
-        const int64_t ia = y * a_pitch + x, io = y * out_pitch + x;
-        if (op == HD_OP_XOR) {
-            const int64_t va = load_int(a, a_dtype, ia);
-            const int64_t vb = b ? load_int(b, b_dtype, y * b_pitch + x) : (int64_t)b_scalar;
-            const int64_t r = va ^ vb;
-            if (out_dtype == HD_U8) ((uint8_t*)out)[io] = (uint8_t)r;
-            else if (out_dtype == HD_I32) ((int32_t*)out)[io] = (int32_t)r;
-            else if (out_dtype == HD_I16) ((int16_t*)out)[io] = (int16_t)r;
-            else ((int64_t*)out)[io] = r;
-            continue;
-        }
-        const cplx va = load_as(a, a_dtype, ia);
-        const cplx vb = b ? load_as(b, b_dtype, y * b_pitch + x) : cplx{b_scalar, 0.0};
-        cplx r{0.0, 0.0};
+    if constexpr (std::is_same_v<T, S>) return v;
+    else if constexpr (std::is_same_v<T, bool>) return nonzero(v);
+    else if constexpr (is_cplx<T> && is_cplx<S>) return T{(part_t<T>)v.re, (part_t<T>)v.im};
+    else if constexpr (is_cplx<T>) return T{cvt<part_t<T>>(v), part_t<T>(0)};
+    else if constexpr (is_cplx<S>) return cvt<T>(v.re);
+    else if constexpr (std::is_integral_v<T> && std::is_floating_point_v<S>) return (T)(int64_t)v;
+    else return (T)v;
+}
+
+template <typename C> __device__ __forceinline__ C load(const void* p, int dtype, int64_t i)
+{
+    switch (dtype) {
+        case HD_BOOL: return cvt<C>(((const uint8_t*)p)[i] != 0);
+        case HD_U8: return cvt<C>(((const uint8_t*)p)[i]);
+        case HD_I16: return cvt<C>(((const int16_t*)p)[i]);
+        case HD_I32: return cvt<C>(((const int32_t*)p)[i]);
+        case HD_I64: return cvt<C>(((const int64_t*)p)[i]);
+        case HD_F32: return cvt<C>(((const float*)p)[i]);
+        case HD_F64: return cvt<C>(((const double*)p)[i]);
+        case HD_C64: { const float2 v = ((const float2*)p)[i]; return cvt<C>(cf{v.x, v.y}); }
+        default: { const double2 v = ((const double2*)p)[i]; return cvt<C>(cd{v.x, v.y}); }
+    }
+}
+
+template <typename C> __device__ __forceinline__ void store(void* p, int dtype, int64_t i, C v)
+{
+    switch (dtype) {
+        case HD_BOOL: ((uint8_t*)p)[i] = cvt<bool>(v); break;
+        case HD_U8: ((uint8_t*)p)[i] = cvt<uint8_t>(v); break;
+        case HD_I16: ((int16_t*)p)[i] = cvt<int16_t>(v); break;
+        case HD_I32: ((int32_t*)p)[i] = cvt<int32_t>(v); break;
+        case HD_I64: ((int64_t*)p)[i] = cvt<int64_t>(v); break;
+        case HD_F32: ((float*)p)[i] = cvt<float>(v); break;
+        case HD_F64: ((double*)p)[i] = cvt<double>(v); break;
+        case HD_C64: { const cf c = cvt<cf>(v); ((float2*)p)[i] = make_float2(c.re, c.im); break; }
+        default: { const cd c = cvt<cd>(v); ((double2*)p)[i] = make_double2(c.re, c.im); break; }
+    }
+}
+
+// correctly rounded float ops of the part type, so that nothing is contracted or widened
+__device__ __forceinline__ float add_rn(float x, float y) { return __fadd_rn(x, y); }
+__device__ __forceinline__ double add_rn(double x, double y) { return __dadd_rn(x, y); }
+__device__ __forceinline__ float sub_rn(float x, float y) { return __fsub_rn(x, y); }
+__device__ __forceinline__ double sub_rn(double x, double y) { return __dsub_rn(x, y); }
+__device__ __forceinline__ float mul_rn(float x, float y) { return __fmul_rn(x, y); }
+__device__ __forceinline__ double mul_rn(double x, double y) { return __dmul_rn(x, y); }
+__device__ __forceinline__ float div_rn(float x, float y) { return __fdiv_rn(x, y); }
+__device__ __forceinline__ double div_rn(double x, double y) { return __ddiv_rn(x, y); }
+__device__ __forceinline__ float fma_rn(float x, float y, float z) { return __fmaf_rn(x, y, z); }
+__device__ __forceinline__ double fma_rn(double x, double y, double z) { return __fma_rn(x, y, z); }
+__device__ __forceinline__ float sqrt_rn(float x) { return __fsqrt_rn(x); }
+__device__ __forceinline__ double sqrt_rn(double x) { return __dsqrt_rn(x); }
+
+// NumPy's complex loops (pinned against the host's NumPy in tests/test_gpu_elementwise.py):
+//   x * y: re = fma(xr, yr, -(xi * yi)), im = fma(xr, yi, xi * yr)
+//   |z|:   hi * sqrt(fma(r, r, 1)) with r = lo / hi (hi, lo = the larger and smaller of |re|, |im|);
+//          inf if a part is infinite, else NaN if a part is NaN, and 0 when hi is 0
+template <typename T> __device__ __forceinline__ T cmul(T x, T y)
+{
+    return T{fma_rn(x.re, y.re, -mul_rn(x.im, y.im)), fma_rn(x.re, y.im, mul_rn(x.im, y.re))};
+}
+template <typename T> __device__ __forceinline__ part_t<T> cabs(T z)
+{
+    using R = part_t<T>;
+    const R a = fabs(z.re), b = fabs(z.im);
+    if (isinf(a) || isinf(b)) return R(INFINITY);
+    if (isnan(a) || isnan(b)) return R(NAN);
+    const R hi = fmax(a, b), lo = fmin(a, b);
+    if (hi == R(0)) return R(0);
+    const R r = div_rn(lo, hi);
+    return mul_rn(hi, sqrt_rn(fma_rn(r, r, R(1))));
+}
+// NumPy's complex ordering: by real part, then by imaginary part; a NaN part makes the real-part test false
+template <typename T> __device__ __forceinline__ bool clt(T x, T y)
+{
+    return (x.re < y.re && x.im == x.im && y.im == y.im) || (x.re == y.re && x.im < y.im);
+}
+
+template <typename C> __device__ __forceinline__ C apply(int op, C a, C b)
+{
+    if constexpr (is_cplx<C>) {
+        using R = part_t<C>;
         switch (op) {
-            case HD_OP_COPY: r = va; break;
-            case HD_OP_MUL:
-                r.re = __dsub_rn(__dmul_rn(vb.re, va.re), __dmul_rn(vb.im, va.im));
-                r.im = __dadd_rn(__dmul_rn(vb.re, va.im), __dmul_rn(vb.im, va.re));
-                break;
-            case HD_OP_ADD: r = {vb.re + va.re, vb.im + va.im}; break;
-            case HD_OP_RSUB: r = {vb.re - va.re, vb.im - va.im}; break;
-            case HD_OP_LT: r.re = va.re < vb.re ? 1.0 : 0.0; break;
-            case HD_OP_GT: r.re = va.re > vb.re ? 1.0 : 0.0; break;
-            case HD_OP_ABS: r.re = (va.im == 0.0) ? fabs(va.re) : hypot(va.re, va.im); break;
-            case HD_OP_RINT: r.re = rint(va.re); break;
-            case HD_OP_TRUNC: r.re = (va.re == va.re) ? trunc(va.re) : 0.0; break;
-            default: break;
+            case HD_OP_MUL: return cmul(b, a);
+            case HD_OP_ADD: return C{add_rn(b.re, a.re), add_rn(b.im, a.im)};
+            case HD_OP_RSUB: return C{sub_rn(b.re, a.re), sub_rn(b.im, a.im)};
+            case HD_OP_LT: return cvt<C>(clt(a, b));
+            case HD_OP_GT: return cvt<C>(clt(b, a));
+            case HD_OP_ABS: return C{cabs(a), R(0)};
+            case HD_OP_RINT: return C{rint(a.re), rint(a.im)};
+            default: return a;                                        // COPY
         }
-        store_as(out, out_dtype, io, r);
+    } else if constexpr (std::is_floating_point_v<C>) {
+        switch (op) {
+            case HD_OP_MUL: return mul_rn(b, a);
+            case HD_OP_ADD: return add_rn(b, a);
+            case HD_OP_RSUB: return sub_rn(b, a);
+            case HD_OP_LT: return a < b;
+            case HD_OP_GT: return a > b;
+            case HD_OP_ABS: return fabs(a);
+            case HD_OP_RINT: return rint(a);                          // half to even
+            case HD_OP_TRUNC: return a == a ? trunc(a) : C(0);
+            default: return a;
+        }
+    } else if constexpr (std::is_same_v<C, bool>) {
+        switch (op) {
+            case HD_OP_MUL: return a && b;
+            case HD_OP_ADD: return a || b;
+            case HD_OP_LT: return !a && b;
+            case HD_OP_GT: return a && !b;
+            case HD_OP_XOR: return a != b;
+            default: return a;                                        // COPY, ABS, RINT, TRUNC
+        }
+    } else {
+        using W = word_t<C>;
+        switch (op) {
+            case HD_OP_MUL: return (C)(W)((W)b * (W)a);
+            case HD_OP_ADD: return (C)(W)((W)b + (W)a);
+            case HD_OP_RSUB: return (C)(W)((W)b - (W)a);
+            case HD_OP_LT: return a < b;
+            case HD_OP_GT: return a > b;
+            case HD_OP_ABS:                                           // the minimum stays the minimum
+                if constexpr (std::is_signed_v<C>) return a < 0 ? (C)(W)(W(0) - (W)a) : a;
+                else return a;
+            case HD_OP_XOR: return a ^ b;
+            default: return a;                                        // COPY, RINT, TRUNC
+        }
     }
+}
+
+template <typename C>
+__global__ void __launch_bounds__(256) elementwise_kernel(int op, const void* a, int a_dtype, int64_t a_pitch,
+                                                          const void* b, int b_dtype, int64_t b_pitch, C b_scalar,
+                                                          void* out, int out_dtype, int64_t out_pitch, int64_t ny,
+                                                          int64_t nx)
+{
+    // `a` may be `out` (in-place TRUNC): each cell is read before it is written, by the same thread
+    for (CellIter it(nx); it.y < ny; it.next()) {
+        const int64_t y = it.y, x = it.x;
+        const C va = load<C>(a, a_dtype, y * a_pitch + x);
+        const C vb = b ? load<C>(b, b_dtype, y * b_pitch + x) : b_scalar;
+        store(out, out_dtype, y * out_pitch + x, apply(op, va, vb));
+    }
+}
+
+size_t dtype_size(int dtype) { return dtype == HD_BOOL ? 1 : hd_dtype_size(dtype); }
+
+template <typename C>
+int launch(int op, const void* a, int a_dtype, int64_t a_pitch, const void* b, int b_dtype, int64_t b_pitch,
+           const void* b_scalar, void* out, int out_dtype, int64_t out_pitch, int64_t ny, int64_t nx, cudaStream_t s)
+{
+    C scalar{};
+    if (b_scalar) {                                                   // read before the call returns
+        if constexpr (std::is_same_v<C, bool>) scalar = *(const uint8_t*)b_scalar != 0;
+        else memcpy(&scalar, b_scalar, sizeof(C));
+    }
+    const int64_t total = ny * nx;
+    const int blocks = (int)((total + 255) / 256 < (int64_t)hd_num_sms() * 16 ? (total + 255) / 256 : hd_num_sms() * 16);
+    hd_prof_begin("elementwise_kernel", s);
+    elementwise_kernel<C><<<blocks, 256, 0, s>>>(op, a, a_dtype, a_pitch, b, b_dtype, b_pitch, scalar, out, out_dtype,
+                                                 out_pitch, ny, nx);
+    HD_LAUNCH_CHECK();
+    hd_count_launch();
+    return HD_OK;
 }
 
 }  // namespace
 
 extern "C" int hd_elementwise(int op, const void* a, int a_dtype, int64_t a_pitch, const void* b, int b_dtype,
-                              int64_t b_pitch, double b_scalar, void* out, int out_dtype, int64_t out_pitch, int64_t ny,
-                              int64_t nx, void* stream)
+                              int64_t b_pitch, const void* b_scalar, int compute_dtype, void* out, int out_dtype,
+                              int64_t out_pitch, int64_t ny, int64_t nx, void* stream)
 {
     if (!a || !out) return HD_ERR_NULL;
     if (op < HD_OP_COPY || op > HD_OP_TRUNC) return HD_ERR_ARG;
-    if (!hd_dtype_size(a_dtype) || !hd_dtype_size(out_dtype) || (b && !hd_dtype_size(b_dtype))) return HD_ERR_ARG;
+    if (!dtype_size(a_dtype) || !dtype_size(out_dtype) || !dtype_size(compute_dtype) || (b && !dtype_size(b_dtype)))
+        return HD_ERR_ARG;
+    const bool binary = op >= HD_OP_MUL && op <= HD_OP_GT || op == HD_OP_XOR;
+    if (binary && !b && !b_scalar) return HD_ERR_NULL;
     if (ny < 0 || nx < 0 || a_pitch < nx || out_pitch < nx || (b && b_pitch < nx)) return HD_ERR_ARG;
-    if (op == HD_OP_XOR) {
-        auto is_int = [](int d) { return d == HD_U8 || d == HD_I64 || d == HD_I32 || d == HD_I16; };
-        if (!is_int(a_dtype) || (b && !is_int(b_dtype)) || !is_int(out_dtype)) return HD_ERR_UNSUPPORTED;
-    }
+    const bool is_float = compute_dtype == HD_F32 || compute_dtype == HD_F64;
+    const bool is_cplx = compute_dtype == HD_C64 || compute_dtype == HD_C128;
+    if ((op == HD_OP_XOR && (is_float || is_cplx)) || (op == HD_OP_RSUB && compute_dtype == HD_BOOL) ||
+        (op == HD_OP_TRUNC && is_cplx))
+        return HD_ERR_UNSUPPORTED;                                    // NumPy has no such loop either
     if (ny == 0 || nx == 0) return HD_OK;
-    const int64_t total = ny * nx;
-    const int blocks = (int)((total + 255) / 256 < (int64_t)hd_num_sms() * 16 ? (total + 255) / 256 : hd_num_sms() * 16);
-    hd_prof_begin("elementwise_kernel", (cudaStream_t)stream);
-    elementwise_kernel<<<blocks, 256, 0, (cudaStream_t)stream>>>(op, a, a_dtype, a_pitch, b, b_dtype, b_pitch, b_scalar,
-                                                                 out, out_dtype, out_pitch, ny, nx);
-    HD_LAUNCH_CHECK();
-    hd_count_launch();
-    return HD_OK;
+    cudaStream_t s = (cudaStream_t)stream;
+    switch (compute_dtype) {
+#define HD_EW(T, TAG) \
+    case TAG: return launch<T>(op, a, a_dtype, a_pitch, b, b_dtype, b_pitch, b_scalar, out, out_dtype, out_pitch, ny, nx, s);
+        HD_EW(bool, HD_BOOL)
+        HD_EW(uint8_t, HD_U8)
+        HD_EW(int16_t, HD_I16)
+        HD_EW(int32_t, HD_I32)
+        HD_EW(int64_t, HD_I64)
+        HD_EW(float, HD_F32)
+        HD_EW(double, HD_F64)
+        HD_EW(cf, HD_C64)
+        HD_EW(cd, HD_C128)
+#undef HD_EW
+        default: return HD_ERR_ARG;
+    }
 }
 
 // ---- HydroDEMProcess._prepare_final_terms + the three-term sum (hydro_dem_process.py:60-91, :148) ----------

@@ -131,19 +131,36 @@ def _is_pinned(host):
 
 
 def convert(src, dtype, ref_dtype=None):
-    """Device-side dtype conversion (HD_OP_COPY)."""
-    if src.dtype == dtype:
+    """Device-side dtype conversion (HD_OP_COPY) with the semantics of ``astype`` (to bool: ``!= 0``)."""
+    to_bool = ref_dtype is not None and np.dtype(ref_dtype) == np.bool_ and src.ref_dtype != np.bool_
+    if src.dtype == dtype and not to_bool:
         return src if ref_dtype is None else src.with_ref(ref_dtype)
     dst = empty(src.ny, src.nx, dtype, ref_dtype if ref_dtype is not None else src.ref_dtype)
-    elementwise(_lib.OP_COPY, src, None, 0.0, dst)
+    elementwise(_lib.OP_COPY, src, None, dst)
     return dst
 
 
-def elementwise(op, a, b, scalar, out):
+def _tag(raster):
+    """hd_dtype of a raster's storage, HD_BOOL for a byte raster that holds a bool reference."""
+    return _lib.BOOL if raster.dtype == _lib.U8 and raster.ref_dtype == np.bool_ else raster.dtype
+
+
+def elementwise(op, a, b, out, compute=None, scalar=None):
+    """out = op(a, b) in ``compute``, the NumPy dtype of the ufunc loop (default: a's storage dtype).  Without a
+    raster ``b``, ``scalar`` is the second operand: a Python scalar, NumPy scalar or 0-d array, cast to ``compute``
+    as NumPy casts an operand into the loop."""
     lib = _lib.load()
-    bp, bd, bpitch = (b.ptr, b.dtype, b.pitch) if b is not None else (None, 0, 0)
-    _lib.check(lib.hd_elementwise(op, a.ptr, a.dtype, a.pitch, bp, bd, bpitch, float(scalar), out.ptr, out.dtype,
-                                  out.pitch, a.ny, a.nx, stream_ptr()))
+    cdt = np.dtype(compute) if compute is not None else _HD2NP[a.dtype]
+    ctag = _lib.BOOL if cdt == np.bool_ else hd_dtype_of(cdt)
+    bp, bd, bpitch = (b.ptr, _tag(b), b.pitch) if b is not None else (None, 0, 0)
+    host = None
+    if b is None and scalar is not None:
+        with np.errstate(all="ignore"):
+            host = np.asarray(scalar, dtype=cdt) if isinstance(scalar, (bool, int, float, complex)) \
+                else np.asarray(scalar).astype(cdt)
+    sp = ctypes.c_void_p(host.ctypes.data) if host is not None else None
+    _lib.check(lib.hd_elementwise(op, a.ptr, _tag(a), a.pitch, bp, bd, bpitch, sp, ctag, out.ptr, _tag(out), out.pitch,
+                                  a.ny, a.nx, stream_ptr()))
     return out
 
 

@@ -100,7 +100,7 @@ class _InPlace3(WindowFilter):
         if np.dtype(raster.ref_dtype).kind in "iu":
             # the reference writes the float32 result into the caller's INTEGER array (dem[center] = mean, :316):
             # NumPy truncates toward zero on assignment, and the next stage (MajorityFilter) counts those integers
-            dev.elementwise(_lib.OP_TRUNC, out, None, 0.0, out)
+            dev.elementwise(_lib.OP_TRUNC, out, None, out)
         return out
 
     def apply(self, image_to_filter):
@@ -149,7 +149,7 @@ class RouteRivers(WindowFilter):
         check_window(dem.shape, self.window_size)
         # the working copy the reference mutates: dem_sliding.grid = dem.astype('float32') (sliding_window.py:132)
         g = dev.empty(dem.ny, dem.nx, _lib.F32, np.float32)
-        dev.elementwise(_lib.OP_COPY, dem, None, 0.0, g)
+        dev.elementwise(_lib.OP_COPY, dem, None, g)
         mask = as_f32(raster)
         out = dev.empty(raster.ny, raster.nx, _lib.U8, np.float64)
         nbytes = raster.ny * 4
@@ -535,7 +535,7 @@ class FourierProcessQuarters(Filter):
         q1 = fabs.sub(0, qh, 0, qw)                                          # [:my-m, :mx-m]          (:942-943)
         x0 = self._mid_x + m + self._x_odd
         q2 = dev.empty(qh, qw, _lib.F32)                                     # [:my-m, mx+m+x_odd:nx]  (:945-947)
-        dev.elementwise(_lib.OP_COPY, fabs.sub(0, qh, x0, self._nx), None, 0.0, q2)
+        dev.elementwise(_lib.OP_COPY, fabs.sub(0, qh, x0, self._nx), None, q2)
         mask_fn = mask_fn or MaskFourier().run_device
         m1 = mask_fn(q1)
         m2 = mask_fn(q2)

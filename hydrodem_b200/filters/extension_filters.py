@@ -14,7 +14,7 @@ import numpy as np
 from . import DeviceFilter, Filter
 from .. import _lib, device as dev
 from ..exceptions import DeviceError
-from .simple_filters import _operand
+from .simple_filters import binary_op
 
 
 class BitwiseXOR(DeviceFilter):
@@ -24,13 +24,7 @@ class BitwiseXOR(DeviceFilter):
         self.operand = operand if isinstance(operand, dev.DeviceRaster) else copy.deepcopy(operand)
 
     def run_device(self, raster):
-        b, scalar, proto = _operand(self.operand, raster)
-        ref = np.bitwise_xor(proto, np.zeros(0, dtype=raster.ref_dtype)).dtype
-        a = dev.convert(raster, dev.hd_dtype_of(raster.ref_dtype))
-        if b is not None:
-            b = dev.convert(b, dev.hd_dtype_of(b.ref_dtype))
-        out = dev.empty(raster.ny, raster.nx, dev.hd_dtype_of(ref), ref)
-        return dev.elementwise(_lib.OP_XOR, a, b, scalar, out)
+        return binary_op(_lib.OP_XOR, raster, self.operand, np.bitwise_xor)
 
 
 class AbsoluteValues(DeviceFilter):
@@ -38,20 +32,19 @@ class AbsoluteValues(DeviceFilter):
 
     def run_device(self, raster):
         ref = np.abs(np.zeros(0, dtype=raster.ref_dtype)).dtype
-        src = raster
         if np.dtype(raster.ref_dtype).kind == "c" and raster.dtype not in (_lib.C64, _lib.C128):
             raise DeviceError("complex raster stored as a real dtype")
         out = dev.empty(raster.ny, raster.nx, dev.hd_dtype_of(ref), ref)
-        return dev.elementwise(_lib.OP_ABS, src, None, 0.0, out)
+        return dev.elementwise(_lib.OP_ABS, raster, None, out, raster.ref_dtype)
 
 
 class Around(DeviceFilter):
-    """``np.around(image)`` -- round half to even (extension_filters.py:98-130)."""
+    """``np.around(image)`` -- round half to even, both parts of a complex (extension_filters.py:98-130)."""
 
     def run_device(self, raster):
         ref = np.around(np.zeros(0, dtype=raster.ref_dtype)).dtype
         out = dev.empty(raster.ny, raster.nx, dev.hd_dtype_of(ref), ref)
-        return dev.elementwise(_lib.OP_RINT, raster, None, 0.0, out)
+        return dev.elementwise(_lib.OP_RINT, raster, None, out, raster.ref_dtype)
 
 
 # ---- general footprints: host-side plans --------------------------------------------------------------------------
@@ -231,7 +224,7 @@ class BinaryClosing(_CheckedFilter):
         if path == "morph3":
             return _morph(raster, _lib.MORPH_CLOSE, self.structure, 1)
         dil, ero = taps
-        src = raster if raster.dtype in (_lib.U8, _lib.F32) else _nonzero_u8(raster)
+        src = raster if raster.dtype in (_lib.U8, _lib.F32) else dev.convert(raster, _lib.U8, np.bool_)
         return _morph_struct(_morph_struct(src, 1, dil, 1), 0, ero, 1)
 
 
@@ -252,7 +245,7 @@ def _erode_until_stable(raster):
     import torch
     taps = _offsets(_CROSS, reversed_=False)
     flags = torch.zeros(STABLE_LAUNCHES_PER_READ, dtype=torch.int32, device=dev.device())
-    cur = raster if raster.dtype in (_lib.U8, _lib.F32) else _nonzero_u8(raster)
+    cur = raster if raster.dtype in (_lib.U8, _lib.F32) else dev.convert(raster, _lib.U8, np.bool_)
     while True:
         for i in range(STABLE_LAUNCHES_PER_READ):
             cur = _morph_struct(cur, 0, taps, STABLE_STEPS_PER_LAUNCH, ctypes.c_void_p(flags.data_ptr() + 4 * i))
@@ -272,20 +265,11 @@ def _morph(raster, op, structure, iterations):
             full = 0
         else:
             raise DeviceError("binary morphology: only the 3x3 cross and the 3x3 square are implemented on the device")
-    src = raster if raster.dtype in (_lib.U8, _lib.F32) else _nonzero_u8(raster)
+    src = raster if raster.dtype in (_lib.U8, _lib.F32) else dev.convert(raster, _lib.U8, np.bool_)
     out = dev.empty(raster.ny, raster.nx, _lib.U8, np.bool_)
     _lib.check(_lib.load().hd_binary_morph(src.ptr, src.dtype, src.pitch, out.ptr, out.pitch, src.ny, src.nx, op, full,
                                            int(iterations), dev.stream_ptr()))
     return out
-
-
-def _nonzero_u8(raster):
-    """(raster != 0) as uint8 for dtypes the morphology kernel does not stage directly."""
-    lt = dev.empty(raster.ny, raster.nx, _lib.U8, np.bool_)
-    gt = dev.empty(raster.ny, raster.nx, _lib.U8, np.bool_)
-    dev.elementwise(_lib.OP_LT, raster, None, 0.0, lt)
-    dev.elementwise(_lib.OP_GT, raster, None, 0.0, gt)
-    return dev.elementwise(_lib.OP_ADD, lt, gt, 0.0, dev.empty(raster.ny, raster.nx, _lib.U8, np.bool_))
 
 
 class GreyDilation(_CheckedFilter):

@@ -37,7 +37,7 @@ class MedianFilter(WindowFilter):
             ny, nx = raster.shape
             for (y0, y1, x0, x1) in ((0, h, 0, nx), (ny - h, ny, 0, nx), (h, ny - h, 0, h), (h, ny - h, nx - h, nx)):
                 if y1 > y0 and x1 > x0:
-                    dev.elementwise(_lib.OP_COPY, raster.sub(y0, y1, x0, x1), None, 0.0, wide.sub(y0, y1, x0, x1))
+                    dev.elementwise(_lib.OP_COPY, raster.sub(y0, y1, x0, x1), None, wide.sub(y0, y1, x0, x1))
             return wide
         return out
 

@@ -13,24 +13,36 @@ from .. import _lib, device as dev
 
 
 def _operand(value, like):
-    """-> (DeviceRaster | None, scalar, numpy dtype-or-python-scalar for promotion)."""
+    """-> (DeviceRaster | None, scalar | None, prototype of the operand for NumPy's promotion).  Python scalars stay
+    Python scalars (weak under NEP 50); NumPy scalars and 0-d arrays keep their dtype."""
     if isinstance(value, dev.DeviceRaster):
-        return value, 0.0, np.zeros(0, dtype=value.ref_dtype)
-    if isinstance(value, np.ndarray):
-        if value.ndim == 0:
-            return None, value.item(), value
+        return value, None, np.zeros(0, dtype=value.ref_dtype)
+    if isinstance(value, np.ndarray) and value.ndim:
         if value.shape != like.shape:
             raise ValueError(f"operand shape {value.shape} does not match raster shape {like.shape}")
-        return dev.upload(value), 0.0, np.zeros(0, dtype=value.dtype)
+        return dev.upload(value), None, np.zeros(0, dtype=value.dtype)
     return None, value, value
 
 
 def binary_op(op, raster, operand, np_func):
-    """out = np_func(operand, raster) on the device, in NumPy's result dtype."""
+    """out = np_func(operand, raster) on the device, in NumPy's result dtype, which is also the dtype of its loop.
+    Raises what NumPy raises (TypeError for a missing loop, OverflowError for a Python int out of range)."""
     b, scalar, proto = _operand(operand, raster)
     ref = np_func(proto, np.zeros(0, dtype=raster.ref_dtype)).dtype
     out = dev.empty(raster.ny, raster.nx, dev.hd_dtype_of(ref), ref)
-    return dev.elementwise(op, raster, b, scalar, out)
+    return dev.elementwise(op, raster, b, out, ref, scalar)
+
+
+def compare(op, raster, value):
+    """image < value / image > value -> bool, in the dtype NumPy compares in.  NumPy compares a Python int outside
+    the range of an integer loop exactly (np.less(uint8, 300) is all True); against an integer raster that int acts
+    like an infinity of its sign, so it is compared as one, in float64."""
+    b, scalar, proto = _operand(value, raster)
+    loop = np.result_type(raster.ref_dtype, proto)
+    if type(scalar) is int and loop.kind in "iu" and not np.iinfo(loop).min <= scalar <= np.iinfo(loop).max:
+        loop, scalar = np.dtype(np.float64), np.inf if scalar > 0 else -np.inf
+    out = dev.empty(raster.ny, raster.nx, _lib.U8, np.bool_)
+    return dev.elementwise(op, raster, b, out, loop, scalar)
 
 
 class LowerThan(DeviceFilter):
@@ -40,9 +52,7 @@ class LowerThan(DeviceFilter):
         self.value = value
 
     def run_device(self, raster):
-        out = dev.empty(raster.ny, raster.nx, _lib.U8, np.bool_)
-        b, scalar, _ = _operand(self.value, raster)
-        return dev.elementwise(_lib.OP_LT, raster, b, scalar, out)
+        return compare(_lib.OP_LT, raster, self.value)
 
 
 class GreaterThan(DeviceFilter):
@@ -52,9 +62,7 @@ class GreaterThan(DeviceFilter):
         self.value = value
 
     def run_device(self, raster):
-        out = dev.empty(raster.ny, raster.nx, _lib.U8, np.bool_)
-        b, scalar, _ = _operand(self.value, raster)
-        return dev.elementwise(_lib.OP_GT, raster, b, scalar, out)
+        return compare(_lib.OP_GT, raster, self.value)
 
 
 class BooleanToInteger(DeviceFilter):

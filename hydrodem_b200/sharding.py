@@ -625,7 +625,7 @@ class Band:
             own = self._dense(s1 - s0, qw, _lib.U8)
             if hi > lo:
                 q = dev.empty(hi - lo, qw, _lib.F32)
-                dev.elementwise(_lib.OP_COPY, slab.sub(0, hi - lo, xa, xb), None, 0.0, q)
+                dev.elementwise(_lib.OP_COPY, slab.sub(0, hi - lo, xa, xb), None, q)
                 mk = dev.convert(cf.MaskFourier().run_device(q), _lib.U8)
                 own.tensor().copy_(mk.tensor()[s0 - lo:s1 - lo])
             masks.append(own)

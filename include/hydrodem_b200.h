@@ -46,7 +46,9 @@ typedef enum {
     HD_C64 = 4,  /* interleaved float re, im  */
     HD_C128 = 5, /* interleaved double re, im */
     HD_I32 = 6,
-    HD_I16 = 7   /* SRTM / HydroSHEDS on disk: what gdal ReadAsArray hands the reference (image_srtm.py:125, image_hsheds.py:133) */
+    HD_I16 = 7,  /* SRTM / HydroSHEDS on disk: what gdal ReadAsArray hands the reference (image_srtm.py:125, image_hsheds.py:133) */
+    HD_BOOL = 8  /* numpy bool, stored as one byte 0 / 1 like HD_U8; a dtype of hd_elementwise only, where it selects
+                  * bool semantics: `!= 0` on conversion, OR / AND for add / multiply */
 } hd_dtype;
 
 /* ---- runtime --------------------------------------------------------------------------------- */
@@ -90,7 +92,7 @@ int64_t hd_host_lzw_decode(const uint8_t* src, int64_t nsrc, uint8_t* dst, int64
 
 /* ---- elementwise filters (filters/simple_filters.py, extension_filters.py:12-130) -------------- */
 typedef enum {
-    HD_OP_COPY = 0, /* out = (out_dtype) a                      -- dtype conversion                        */
+    HD_OP_COPY = 0, /* out = a          -- dtype conversion (ndarray.astype)                                   */
     HD_OP_MUL = 1,  /* out = b * a      ProductFilter.apply      simple_filters.py:165-180                 */
     HD_OP_ADD = 2,  /* out = b + a      AdditionFilter.apply     simple_filters.py:214-229                 */
     HD_OP_RSUB = 3, /* out = b - a      SubtractionFilter.apply  simple_filters.py:261-275 (b = minuend)   */
@@ -98,14 +100,21 @@ typedef enum {
     HD_OP_GT = 5,   /* out = a > b      GreaterThan.apply        simple_filters.py:81-96                   */
     HD_OP_ABS = 6,  /* out = |a|        AbsoluteValues.apply     extension_filters.py:78-95 (C64 -> F32)   */
     HD_OP_RINT = 7, /* out = around(a)  Around.apply             extension_filters.py:113-130 (half-even)  */
-    HD_OP_XOR = 8,  /* out = b ^ a      BitwiseXOR.apply         extension_filters.py:43-60 (U8/I64)       */
+    HD_OP_XOR = 8,  /* out = b ^ a      BitwiseXOR.apply         extension_filters.py:43-60                */
     HD_OP_TRUNC = 9 /* out = trunc(a), NaN -> 0: what NumPy's assignment of a float into an integer array does
                      * (CorrectNANValues on the int16 HydroSHEDS raster, custom_filters.py:316) */
 } hd_elementwise_op;
-/* `b` may be NULL: then the scalar `b_scalar` is the second operand.  Arithmetic is done in double and
- * rounded once to out_dtype (innocuous double rounding: identical to native float32 arithmetic). */
+/* Each op runs in `compute_dtype`, the dtype of NumPy's ufunc loop: `a` and `b` are converted to it as
+ * ndarray.astype converts (round to nearest; a float truncated toward zero into an integer, then wrapped; `!= 0`
+ * into HD_BOOL; the imaginary part dropped into a real dtype), the op is evaluated in it with NumPy's semantics
+ * (integers wrap, float32 is not widened, complex multiply, |z| and ordering use NumPy's formulas, around rounds
+ * both parts of a complex), and the result is converted the same way to `out_dtype`.  Comparisons give 0 / 1.
+ * `b` may be NULL: then `b_scalar`, a host pointer to one value of compute_dtype (HD_BOOL: one byte), is the second
+ * operand; it is read before the call returns.  `a` may be `out`.  XOR on float or complex, RSUB on HD_BOOL and
+ * TRUNC on complex return HD_ERR_UNSUPPORTED, as NumPy has no such loop. */
 int hd_elementwise(int op, const void* a, int a_dtype, int64_t a_pitch, const void* b, int b_dtype, int64_t b_pitch,
-                   double b_scalar, void* out, int out_dtype, int64_t out_pitch, int64_t ny, int64_t nx, void* stream);
+                   const void* b_scalar, int compute_dtype, void* out, int out_dtype, int64_t out_pitch, int64_t ny,
+                   int64_t nx, void* stream);
 
 /* HydroDEMProcess._prepare_final_terms and the three-term sum, hydro_dem_process.py:60-91, :148, fused:
  * out = srtm * (1 - ((lagoon_values > 0) + rivers)) + lagoon_values + hsheds_fixed * rivers, in float64
