@@ -85,7 +85,7 @@ SIGNATURES = {
     "hd_pdfill": (_i, [_p, _i64, _p, _i64, _i64, _i64, _p, _i64, ctypes.POINTER(_i), _p]),
     "hd_pdfill_band": (_i, [_p, _i64, _p, _i64, _i64, _i64, _p, _i64, _i, ctypes.POINTER(_i), _p]),
     "hd_pdfill_d8": (_i, [_p, _i64, _p, _i64, _p, _i64, _i64, _i64, _p, _i64, ctypes.POINTER(_i), _p]),
-    "hd_pdfill_finish_d8": (_i, [_p, _i64, _p, _i64, _i64, _i64, _p, _p]),
+    "hd_pdfill_finish_d8": (_i, [_p, _i64, _p, _i64, _p, _i64, _i64, _i64, _p, _p]),
     "hd_pdfill_status": (_i, [_p, ctypes.POINTER(_i), _p]),
     "hd_halo_min_flag": (_i, [_p, _p, _i64, _p, _p]),
     "hd_fill_pool_band": (_i, [_p, _i64, _i64, _i64, _p, _p, _i64, _i, _p, _p]),

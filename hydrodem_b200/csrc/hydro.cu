@@ -34,10 +34,11 @@ constexpr int WS_STRIDE = FT + 3;         // 67: odd stride -> row marches are b
 __global__ void __launch_bounds__(256) fill_init_kernel(const float* __restrict__ z, int64_t z_pitch, float* __restrict__ w,
                                                         int64_t w_pitch, int64_t ny, int64_t nx, int top_is_halo = 0,
                                                         int bottom_is_halo = 0, int* __restrict__ tile_has_nodata = nullptr,
-                                                        int tiles_x = 0, int* __restrict__ any_nodata = nullptr,
+                                                        int tiles_x = 0, int* __restrict__ seen = nullptr,
                                                         const float* __restrict__ wc = nullptr, int64_t c_pitch = 0,
                                                         int64_t wc_y0 = 0)
 {
+    // seen[0] = 1: z holds a nodata cell, seen[1] = 1: z holds a -0.0 (what fill_finish_kernel has to rewrite)
     const int64_t nxq = (nx + 3) / 4;                                            // four consecutive cells per thread
     for (CellIter it(nxq); it.y < ny; it.next()) {
         const int64_t y = it.y, x0 = 4 * it.x;
@@ -49,7 +50,7 @@ __global__ void __launch_bounds__(256) fill_init_kernel(const float* __restrict_
         // looks up the GLOBAL coarse fill)
         const float start = wc ? __ldg(wc + ((y + wc_y0) / CB) * c_pitch + x0 / CB) : __int_as_float(0x7f800000);
         const bool yframe = (y == 0 && !top_is_halo) || (y == ny - 1 && !bottom_is_halo);
-        bool nodata = false;
+        bool nodata = false, negzero = false;
 #pragma unroll
         for (int j = 0; j < 4; ++j) {
             const int64_t x = x0 + j;
@@ -61,31 +62,43 @@ __global__ void __launch_bounds__(256) fill_init_kernel(const float* __restrict_
             }
             else if (yframe || x == 0 || x == nx - 1)
                 r = v;                                                           // frame: W = z (a band's halo rows are not frame)
+            negzero |= __float_as_uint(v) == 0x80000000u;                        // (cells past the row end read +0)
             r4[j] = r;
         }
-        if (nodata) {
-            if (tile_has_nodata) tile_has_nodata[(y / FT) * tiles_x + (x0 / FT)] = 1;   // benign race: every writer stores 1
-            if (any_nodata) *any_nodata = 1;
+        if (nodata) {                                                            // benign races: every writer stores 1
+            if (tile_has_nodata) tile_has_nodata[(y / FT) * tiles_x + (x0 / FT)] = 1;
+            if (seen) seen[0] = 1;
         }
+        if (negzero && seen) seen[1] = 1;
         store4<float>(w, w_pitch, y, x0, nx, r4);
     }
 }
 
 __global__ void __launch_bounds__(256) fill_finish_kernel(const float* __restrict__ z, int64_t z_pitch,
                                                           float* __restrict__ w, int64_t w_pitch, int64_t ny, int64_t nx,
-                                                          const int* __restrict__ any_nodata = nullptr,
+                                                          const int* __restrict__ seen = nullptr,
                                                           const int* __restrict__ status = nullptr,
                                                           const int* __restrict__ pending = nullptr)
 {
-    // a fill that stalled must not pass for a result: poison the first cell (see STATUS_OFF)
+    // Every zero of the result is +0.0: the racy update order decides which signed zero of z a cell takes first (a
+    // candidate that only differs in the sign of zero never replaces it), so the sign is rewritten here.  W only ever
+    // holds values of z and +-inf, so without a -0.0 in z (seen[1], fill_init_kernel) there is none to rewrite.
+    const bool nodata = !seen || seen[0], negzero = !seen || seen[1];
+    if (nodata || negzero) {
+        for (CellIter it(nx); it.y < ny; it.next()) {
+            const int64_t y = (int64_t)it.y, x = (int64_t)it.x;
+            float* p = w + y * w_pitch + x;
+            if (nodata) {
+                const float v = z[y * z_pitch + x];
+                if (v != v) { *p = v; continue; }                                // nodata stays nodata
+            }
+            if (negzero && __float_as_uint(*p) == 0x80000000u) *p = 0.f;
+        }
+    }
+    // a fill that stalled must not pass for a result: poison the first cell (see STATUS_OFF) -- after the pass above,
+    // in which this same thread handled that cell
     if (blockIdx.x == 0 && threadIdx.x == 0 && ((status && *status != 0) || (pending && *pending != 0)))
         w[0] = __int_as_float(0x7fc00000);
-    if (any_nodata && *any_nodata == 0) return;          // fill_init_kernel saw no nodata cell: nothing to restore
-    for (CellIter it(nx); it.y < ny; it.next()) {
-        const int64_t y = (int64_t)it.y, x = (int64_t)it.x;
-        const float v = z[y * z_pitch + x];
-        if (v != v) w[y * w_pitch + x] = v;                                      // nodata stays nodata
-    }
 }
 
 // ---- asynchronous worklist ----------------------------------------------------------------------------------------------
@@ -130,7 +143,7 @@ __global__ void __launch_bounds__(256) fill_finish_kernel(const float* __restric
 struct FillCtl {
     int head, tail, pending, error;
     unsigned long long visits, changed_visits, iterations;
-    int qcap, any_nodata, pad_[2];
+    int qcap, seen[2], pad_;          // seen: fill_init_kernel found a nodata cell / a -0.0 in z
     unsigned long long cycles[6];     // per-phase SM cycles of thread 0, summed over visits (HD_FILL_TRACE)
 };
 constexpr int SLOT_EMPTY = -1;
@@ -592,7 +605,10 @@ __global__ void __launch_bounds__(256) d8_kernel(const float* __restrict__ w, in
 // every cell's flow direction is written in the same sweep over W -- 4 B read + 1 B written per cell, W is not read
 // a second time by a separate D8 launch.  A fill that stalled (status word set, see FILL_*) poisons W[0][0] and the
 // first code with NaN / 255 so that it cannot pass for a result.
-__global__ void __launch_bounds__(256) fill_finish_d8_kernel(float* __restrict__ w, int64_t w_pitch, uint8_t* __restrict__ out,
+// W = -inf does not make a cell nodata: a cell whose own z is -inf keeps -inf when it drains to an outlet at -inf.
+// Only a window that holds a -inf reads z, and only at its -inf cells.
+__global__ void __launch_bounds__(256) fill_finish_d8_kernel(const float* __restrict__ z, int64_t z_pitch,
+                                                             float* __restrict__ w, int64_t w_pitch, uint8_t* __restrict__ out,
                                                              int64_t out_pitch, int64_t ny, int64_t nx,
                                                              const FillCtl* __restrict__ ctl, const int* __restrict__ status)
 {
@@ -623,7 +639,7 @@ __global__ void __launch_bounds__(256) fill_finish_d8_kernel(float* __restrict__
             win[dy][1] = q[0]; win[dy][2] = q[1]; win[dy][3] = q[2]; win[dy][4] = q[3];
             win[dy][5] = x0 + 4 < nx ? __ldcg(p + 4) : 0.f;
         }
-        // nodata cells are -inf here: only a window that holds one needs the NaN conversion (and the restore below)
+        // nodata cells are -inf here: only a window that holds a -inf needs the NaN conversion (and the restore below)
         float lowest = win[0][0];
 #pragma unroll
         for (int dy = 0; dy < 3; ++dy)
@@ -632,9 +648,19 @@ __global__ void __launch_bounds__(256) fill_finish_d8_kernel(float* __restrict__
         const bool has_nodata = lowest == ninf;
         if (has_nodata) {
 #pragma unroll
-            for (int dy = 0; dy < 3; ++dy)
+            for (int dy = 0; dy < 3; ++dy) {
+                const int64_t yy = y + dy - 1;                           // (cells outside the raster hold 0, never -inf)
+                const float* p = z + yy * z_pitch + x0;
+                if (win[dy][1] == ninf || win[dy][2] == ninf || win[dy][3] == ninf || win[dy][4] == ninf) {
+                    float zq[4];
+                    gload4(p, x0, nx, zq);
 #pragma unroll
-                for (int j = 0; j < 6; ++j) win[dy][j] = win[dy][j] == ninf ? qnan : win[dy][j];
+                    for (int j = 0; j < 4; ++j)
+                        if (win[dy][j + 1] == ninf && zq[j] != zq[j]) win[dy][j + 1] = qnan;
+                }
+                if (win[dy][0] == ninf && __ldg(p - 1) != __ldg(p - 1)) win[dy][0] = qnan;
+                if (win[dy][5] == ninf && __ldg(p + 4) != __ldg(p + 4)) win[dy][5] = qnan;
+            }
         }
         uint8_t codes[4] = {0, 0, 0, 0};
         bool restore = false;
@@ -642,14 +668,18 @@ __global__ void __launch_bounds__(256) fill_finish_d8_kernel(float* __restrict__
         for (int j = 0; j < 4; ++j) {
             const int64_t x = x0 + j;
             const float c = win[1][j + 1];
-            restore |= has_nodata && (c != c) && x < nx;
+            // nodata cells get NaN back; every zero becomes +0.0 (see fill_finish_kernel).  No D8 decision depends on the
+            // sign of a zero: a drop between two zeros is a zero, never positive
+            restore |= ((has_nodata && c != c) || __float_as_uint(c) == 0x80000000u) && x < nx;
             if (y == 0 || y >= ny - 1 || x == 0 || x >= nx - 1) continue;
             codes[j] = d8_code(win, j);
         }
-        if (restore) {                                                    // rare: rewrite the quad with NaN at the nodata cells
+        if (restore) {                                                    // rare: rewrite the quad's nodata cells and -0.0
 #pragma unroll
-            for (int j = 0; j < 4; ++j)
-                if (x0 + j < nx && win[1][j + 1] != win[1][j + 1]) w[y * w_pitch + x0 + j] = qnan;
+            for (int j = 0; j < 4; ++j) {
+                const float c = win[1][j + 1];
+                if (x0 + j < nx && (c != c || __float_as_uint(c) == 0x80000000u)) w[y * w_pitch + x0 + j] = c != c ? qnan : 0.f;
+            }
         }
         if (bad && y == 0 && x0 == 0) { w[0] = qnan; codes[0] = 255; }
         store4v<uint8_t>(out, out_pitch, y, x0, nx, codes);
@@ -689,14 +719,14 @@ struct FillOpts {
     int* status = nullptr;        // sticky status word of the whole fill (root workspace + STATUS_OFF)
 };
 
-static int launch_finish_d8(void* w, int64_t w_pitch, void* d8, int64_t d8_pitch, int64_t ny, int64_t nx, const void* workspace,
-                            cudaStream_t s)
+static int launch_finish_d8(const void* z, int64_t z_pitch, void* w, int64_t w_pitch, void* d8, int64_t d8_pitch, int64_t ny,
+                            int64_t nx, const void* workspace, cudaStream_t s)
 {
     const FillCtl* ctl = (const FillCtl*)workspace;
     const int* status = workspace ? (const int*)((const char*)workspace + STATUS_OFF) : nullptr;
     hd_prof_begin("fill_finish_d8_kernel", s);
-    fill_finish_d8_kernel<<<stream_grid(ny * ((nx + 3) / 4)), 256, 0, s>>>((float*)w, w_pitch, (uint8_t*)d8, d8_pitch, ny, nx, ctl,
-                                                                          status);
+    fill_finish_d8_kernel<<<stream_grid(ny * ((nx + 3) / 4)), 256, 0, s>>>((const float*)z, z_pitch, (float*)w, w_pitch, (uint8_t*)d8,
+                                                                          d8_pitch, ny, nx, ctl, status);
     HD_LAUNCH_CHECK(); hd_count_launch();
     return HD_OK;
 }
@@ -729,7 +759,7 @@ static int pdfill_async(const void* z, int64_t z_pitch, void* w, int64_t w_pitch
     if (!(flags & 1) && !opt.preinit) {
         hd_prof_begin("fill_init_kernel", s);
         fill_init_kernel<<<stream_grid(ny * ((nx + 3) / 4)), 256, 0, s>>>((const float*)z, z_pitch, (float*)w, w_pitch, ny, nx, flags & 2,
-                                                             flags & 4, queued, tiles_x, &ctl->any_nodata, opt.wc, opt.c_pitch,
+                                                             flags & 4, queued, tiles_x, ctl->seen, opt.wc, opt.c_pitch,
                                                              opt.wc_y0);
         HD_LAUNCH_CHECK(); hd_count_launch();
     }
@@ -744,7 +774,7 @@ static int pdfill_async(const void* z, int64_t z_pitch, void* w, int64_t w_pitch
     if (finish) {
         hd_prof_begin("fill_finish_kernel", s);
         fill_finish_kernel<<<stream_grid(ny * nx), 256, 0, s>>>((const float*)z, z_pitch, (float*)w, w_pitch, ny, nx,
-                                                               (flags & 1) ? nullptr : &ctl->any_nodata, opt.status,
+                                                               (flags & 1) ? nullptr : ctl->seen, opt.status,
                                                                &ctl->pending);
         HD_LAUNCH_CHECK(); hd_count_launch();
     }
@@ -900,16 +930,16 @@ extern "C" int hd_pdfill_d8(const void* z, int64_t z_pitch, void* w, int64_t w_p
     cudaStream_t s = (cudaStream_t)stream;
     HD_CUDA_OK(cudaMemsetAsync((char*)workspace + STATUS_OFF, 0, sizeof(int), s));
     if (int e = pdfill_multilevel(z, z_pitch, w, w_pitch, ny, nx, workspace, visits_out, s, false)) return e;
-    return launch_finish_d8(w, w_pitch, d8, d8_pitch, ny, nx, workspace, s);
+    return launch_finish_d8(z, z_pitch, w, w_pitch, d8, d8_pitch, ny, nx, workspace, s);
 }
 
 // The fused last pass on its own (row-band fill: after the last round and the final halo refresh).
-extern "C" int hd_pdfill_finish_d8(void* w, int64_t w_pitch, void* d8, int64_t d8_pitch, int64_t ny, int64_t nx,
-                                   const void* workspace, void* stream)
+extern "C" int hd_pdfill_finish_d8(const void* z, int64_t z_pitch, void* w, int64_t w_pitch, void* d8, int64_t d8_pitch,
+                                   int64_t ny, int64_t nx, const void* workspace, void* stream)
 {
-    if (!w || !d8) return HD_ERR_NULL;
-    if (ny < 1 || nx < 1 || w_pitch < nx || d8_pitch < nx) return HD_ERR_ARG;
-    return launch_finish_d8(w, w_pitch, d8, d8_pitch, ny, nx, workspace, (cudaStream_t)stream);
+    if (!z || !w || !d8) return HD_ERR_NULL;
+    if (ny < 1 || nx < 1 || z_pitch < nx || w_pitch < nx || d8_pitch < nx) return HD_ERR_ARG;
+    return launch_finish_d8(z, z_pitch, w, w_pitch, d8, d8_pitch, ny, nx, workspace, (cudaStream_t)stream);
 }
 
 // Sticky status of the last fill that used this workspace (synchronises the stream): 0 = reached the fixed point.

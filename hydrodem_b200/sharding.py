@@ -804,7 +804,8 @@ class Band:
         self.fill_rounds = rounds
         # at the fixed point a halo row equals the neighbour's owned row, so D8 needs no further exchange; NaN
         # restoration and the flow directions are one fused pass
-        _lib.check(lib.hd_pdfill_finish_d8(w.ptr, w.pitch, d8.ptr, d8.pitch, zv.ny, nx, wp, dev.stream_ptr()))
+        _lib.check(lib.hd_pdfill_finish_d8(zv.ptr, zv.pitch, w.ptr, w.pitch, d8.ptr, d8.pitch, zv.ny, nx, wp,
+                                           dev.stream_ptr()))
         self._fill_work = work
         return w.sub(n_up, n_up + rows, 0, nx), d8.sub(n_up, n_up + rows, 0, nx)
 

@@ -363,9 +363,10 @@ int hd_pdfill_band(const void* z, int64_t z_pitch, void* w, int64_t w_pitch, int
  * re-read by a separate D8 launch).  Asynchronous and capturable; *visits_out (may be NULL) synchronises once. */
 int hd_pdfill_d8(const void* z, int64_t z_pitch, void* w, int64_t w_pitch, void* d8, int64_t d8_pitch, int64_t ny,
                  int64_t nx, void* workspace, int64_t workspace_bytes, int* visits_out, void* stream);
-/* The fused last pass alone (row-band fill: after the last round).  workspace: the fill's (status word), may be NULL. */
-int hd_pdfill_finish_d8(void* w, int64_t w_pitch, void* d8, int64_t d8_pitch, int64_t ny, int64_t nx,
-                        const void* workspace, void* stream);
+/* The fused last pass alone (row-band fill: after the last round), on the raster the fill ran on: z tells a nodata
+ * cell (NaN) from a cell of height -inf, both -inf in W.  workspace: the fill's (status word), may be NULL. */
+int hd_pdfill_finish_d8(const void* z, int64_t z_pitch, void* w, int64_t w_pitch, void* d8, int64_t d8_pitch, int64_t ny,
+                        int64_t nx, const void* workspace, void* stream);
 /* Sticky status of the last fill run with this workspace (0 = fixed point reached; 1 worklist stalled, 2 in-tile
  * iteration cap, 4 work left).  The finish passes also poison W[0][0] = NaN when it is non-zero.  Synchronises. */
 int hd_pdfill_status(const void* workspace, int* status_out, void* stream);
