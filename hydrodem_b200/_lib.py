@@ -103,6 +103,8 @@ SIGNATURES = {
     "hd_max_filter_rect": (_i, [_p, _i64, _p, _i64, _i, _i64, _i64, _i, _i, _p, _i64, _p]),
     "hd_warp": (_i, [_p, _i, _i64, _i64, _i64, ctypes.POINTER(_d), _i, _d, _p, _i64, _i64, _i64, ctypes.POINTER(_d), _i64,
                      ctypes.POINTER(_d), _i, _p]),
+    "hd_warp_mosaic": (_i, [_p, _i64, _p, _p, ctypes.POINTER(_i64), _i, ctypes.POINTER(_d), _i, _d, _p, _i64, _i64, _i64,
+                            ctypes.POINTER(_d), _i64, ctypes.POINTER(_d), _i, _p]),
     "hd_host_tm_inverse": (_i, [ctypes.POINTER(_d), _p, _p, _i64, _p, _p]),
     "hd_host_tm_forward": (_i, [ctypes.POINTER(_d), _p, _p, _i64, _p, _p]),
     "hd_rasterize_workspace_bytes": (_i64, [_i64]),

@@ -422,7 +422,7 @@ def write_geotiff(path, array, like=None, dtype=None, geo_tags=None, nodata=None
     for t, v in (geo_tags or {}).items():
         tags[t] = v
     if nodata is not None:
-        s = (repr(float(nodata)) if float(nodata) != int(nodata) else str(int(nodata))).encode() + b"\0"
+        s = (str(int(nodata)) if float(nodata).is_integer() else repr(float(nodata))).encode() + b"\0"    # NaN: "nan"
         tags[GDAL_NODATA] = (2, len(s), s)
     row_bytes = nx * dt.itemsize
     rps = max(1, min(ny, strip_bytes // max(row_bytes, 1)))
@@ -497,11 +497,17 @@ def process_geotiffs(srtm_tif, groves_tif, hsheds_tif, final_tif, rivers_tif=Non
     ``envelope``: an ESRI shapefile of the area of interest, or a ``warp.Grid``.  The inputs (raw downloads, geographic
     WGS84 or EPSG:22184) are then first reprojected onto the envelope's EPSG:22184 90 m grid on the device
     (``warp.warp_to_device``, nearest neighbour: the reference's ``resample_and_cut`` step), go through the chain without
-    leaving the device, and the DEM is written with that grid's georeference."""
+    leaving the device, and the DEM is written with that grid's georeference.  Each input may then also be a list of
+    tile paths, mosaicked onto the grid as one virtual raster (``warp.warp_to_device``); without an envelope there is
+    no grid to mosaic onto, and a list raises GeoTiffError."""
     from .pipeline import ConditioningChain
     chain = chain or ConditioningChain()
     if envelope is not None:
         return _process_on_grid(chain, srtm_tif, groves_tif, hsheds_tif, final_tif, rivers_tif, envelope)
+    for name, p in (("srtm_tif", srtm_tif), ("groves_tif", groves_tif), ("hsheds_tif", hsheds_tif),
+                    ("rivers_tif", rivers_tif)):
+        if isinstance(p, (list, tuple)):
+            raise GeoTiffError(f"{name}: a list of tiles needs an envelope (or a warp.Grid) to mosaic onto")
     srtm = read_array(srtm_tif)
     groves = read_array(groves_tif)
     hsheds = read_array(hsheds_tif)

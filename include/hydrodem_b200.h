@@ -404,6 +404,20 @@ typedef enum { HD_WARP_NEAREST = 0, HD_WARP_BILINEAR = 1 } hd_warp_resample;
 int hd_warp(const void* src, int src_dtype, int64_t src_pitch, int64_t src_ny, int64_t src_nx, const double* src_geo,
             int has_nodata, double nodata, void* dst, int64_t dst_pitch, int64_t dst_ny, int64_t dst_nx, const double* dst_geo,
             int64_t dst_row0, const double* tm, int resample, void* stream);
+/* hd_warp over a mosaic of sources sampled as one virtual raster (DESIGN §9c).  frame: HOST double[4] (x0, dx, y0, dy) of
+ * the first listed source, the virtual raster's corner; u and v are computed from it exactly as in hd_warp.  Virtual pixel
+ * (U, V) holds the value of the last listed source that contains it with a value that is not nodata; else it has no
+ * sample, which nearest and bilinear treat as hd_warp treats a pixel outside its source.  DEVICE index built on the host:
+ * sources = int64[n_sources][6] (device pointer, pitch in elements, U, V, ny, nx: the source's pixel (0, 0) is virtual
+ * pixel (U, V)); bins = HOST int64[6] (iu0, iv0, bw, bh, nbu, nbv): a grid of nbu x nbv bins of bw x bh pixels from
+ * (iu0, iv0); bin_start = int64[nbu * nbv + 1] and bin_list (int64) are the CSR lists, bin (bu, bv) = bv * nbu + bu, of
+ * the sources whose rectangle meets the bin, in descending list order.  Every source has sample type src_dtype (U8 / I16
+ * / F32).  Allocates nothing; asynchronous and capturable.  The checks of hd_warp, n_sources < 1, a bin size or count
+ * below 1 or a bin grid beyond 2^52 pixels -> HD_ERR_ARG, before any device work. */
+int hd_warp_mosaic(const int64_t* sources, int64_t n_sources, const int64_t* bin_start, const int64_t* bin_list,
+                   const int64_t* bins, int src_dtype, const double* frame, int has_nodata, double nodata, void* dst,
+                   int64_t dst_pitch, int64_t dst_ny, int64_t dst_nx, const double* dst_geo, int64_t dst_row0,
+                   const double* tm, int resample, void* stream);
 /* HOST: the same inverse Transverse Mercator as hd_warp, on n points (x, y metres -> lon, lat degrees); the host API uses it
  * to check that a destination grid overlaps its source before any device work. */
 int hd_host_tm_inverse(const double* tm, const double* x, const double* y, int64_t n, double* lon, double* lat);
