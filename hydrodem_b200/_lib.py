@@ -41,6 +41,8 @@ SIGNATURES = {
     "hd_host_widen_f32_f64": (_i, [_p, _p, _i64, _i]),
     "hd_host_widen_i16": (_i, [_p, _i, _p, _i64, _i]),
     "hd_host_lzw_decode": (_i64, [_p, _i64, _p, _i64]),
+    "hd_host_inflate": (_i64, [_p, _i64, _p, _i64]),
+    "hd_host_tiff_lzw": (_i64, [_p, _i64, _p, _i64]),
     "hd_confusion_counts": (_i, [_p, _i, _i64, _p, _i, _i64, _i64, _i64, ctypes.c_double, _p, _p]),
     "hd_pack_i16": (_i, [_p, _i64, _p, _i64, _i64, _p, _p]),
     "hd_elementwise": (_i, [_i, _p, _i, _i64, _p, _i, _i64, _p, _i, _p, _i, _i64, _i64, _i64, _p]),
@@ -110,6 +112,8 @@ SIGNATURES = {
     "hd_rasterize_workspace_bytes": (_i64, [_i64]),
     "hd_rasterize_lines": (_i, [_p, _p, _i64, _p, _p, _i64, _p, _i64, _p, _i64, _i64, _i64, ctypes.POINTER(_d), _i64,
                                 ctypes.POINTER(_d), _p, _i64, _p]),
+    "hd_tiff_decode_workspace_bytes": (_i64, [_i64, _i64, _i64, _i]),
+    "hd_tiff_decode": (_i, [_p, _i64, _p, _i64, _i, _i, _i, _i, _p, _i64, _i64, _i64, _i64, _i64, _p, _p, _i64, _p]),
 }
 
 

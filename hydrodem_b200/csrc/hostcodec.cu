@@ -73,3 +73,26 @@ extern "C" int64_t hd_host_lzw_decode(const uint8_t* src, int64_t nsrc, uint8_t*
     }
     return op;
 }
+
+// ---- the GPU decoder's core on the host (csrc/tiffcodec.cuh), for tests against zlib and hd_host_lzw_decode ------------
+#include "tiffcodec.cuh"
+
+extern "C" int64_t hd_host_inflate(const uint8_t* src, int64_t nsrc, uint8_t* dst, int64_t cap)
+{
+    if (!src || !dst) return HD_ERR_NULL;
+    if (nsrc < 0 || cap < 0) return HD_ERR_ARG;
+    tiffcodec::InflateTables t;
+    int64_t n = 0;
+    const int st = tiffcodec::inflate(src, nsrc, tiffcodec::HostEmit{dst}, cap, t, &n);
+    return st == tiffcodec::OK ? n : st == tiffcodec::HOST ? (int64_t)HD_ERR_WORKSPACE : (int64_t)HD_ERR_ARG;
+}
+
+extern "C" int64_t hd_host_tiff_lzw(const uint8_t* src, int64_t nsrc, uint8_t* dst, int64_t cap)
+{
+    if (!src || !dst) return HD_ERR_NULL;
+    if (nsrc < 0 || cap < 0) return HD_ERR_ARG;
+    static thread_local tiffcodec::LzwTable t;
+    int64_t n = 0;
+    const int st = tiffcodec::lzw(src, nsrc, tiffcodec::HostEmit{dst}, cap, t, &n);
+    return st == tiffcodec::OK ? n : (int64_t)HD_ERR_ARG;
+}

@@ -12,7 +12,8 @@ minimal replacement for exactly those two calls:
   uncompressed striped file whose strips are contiguous (what GDAL and ``array2raster`` write) is ONE ``readinto``
   straight into a pinned host array -- the array the upload DMA reads from, no intermediate copy.
 * ``read_to_device(path)``      the same file -> ``DeviceRaster``, row chunks read into two pinned staging buffers and
-  uploaded on a copy stream while the next chunk is being read (int16 rasters cross PCIe as int16).
+  uploaded on a copy stream while the next chunk is being read (int16 rasters cross PCIe as int16); Deflate and LZW
+  files cross PCIe compressed and their blocks are decoded on the GPU (``hd_tiff_decode``, DESIGN §9d).
 * ``array2raster(new, array, rasterfn)``  same signature and meaning as the reference's: float32, georeference tags
   (ModelPixelScale / ModelTiepoint / GeoKeyDirectory / GeoDoubleParams / GeoAsciiParams, i.e. geotransform + projection)
   copied from ``rasterfn``.  BigTIFF automatically above 4 GB.
@@ -348,8 +349,9 @@ def read_array(path, pinned=True, info=None):
 
 def read_to_device(path, chunk_bytes=64 << 20):
     """The first band of ``path`` as a DeviceRaster in the file's sample type.  Contiguous uncompressed files are read in
-    row chunks into two pinned staging buffers; chunk k uploads on a copy stream while chunk k+1 is read.  Other
-    layouts go through ``read_array`` (pinned) and one upload."""
+    row chunks into two pinned staging buffers; chunk k uploads on a copy stream while chunk k+1 is read.  LZW and
+    Deflate files cross PCIe compressed and are decoded on the device (``_read_compressed_to_device``, DESIGN §9d).
+    Other layouts go through ``read_array`` (pinned) and one upload."""
     import ctypes
     import torch
     from . import _lib, device as dev
@@ -357,6 +359,8 @@ def read_to_device(path, chunk_bytes=64 << 20):
     info = read_info(path)
     native = info.dtype.newbyteorder("=")
     swap = info.dtype.byteorder == ">" or (info.dtype.byteorder == "=" and not np.little_endian)
+    if info.compression in (5, 8, 32946):
+        return _read_compressed_to_device(path, info, chunk_bytes)
     if not _contiguous(info) or swap:
         return dev.upload(read_array(path, pinned=True, info=info))
     ny, nx = info.shape
@@ -387,6 +391,144 @@ def read_to_device(path, chunk_bytes=64 << 20):
     for ev in events:
         if ev is not None:
             ev.synchronize()                                    # the staging buffers go out of scope
+    return raster
+
+
+_DECODE_CORRUPT, _DECODE_HOST = 1, 2                           # hd_tiff_decode's status words (0 = stored)
+
+
+def _block_table(path, info):
+    """(TIFF block index, file offset, byte count, y0, x0, rows) of every block inside the raster, as read_array walks
+    them: strips hold min(block_h, height - y0) rows, tiles always block_h; blocks past the height are skipped."""
+    n = len(info.offsets)
+    k = np.arange(n, dtype=np.int64)
+    across = -(-info.width // info.block_w)
+    by, bx = (k // across, k % across) if info.tiled else (k, np.zeros_like(k))
+    y0, x0 = by * info.block_h, bx * info.block_w
+    keep = y0 < info.height
+    if len(info.bytecounts) < n:
+        raise GeoTiffError(f"{path}: fewer byte counts than blocks")
+    rows = np.full(n, info.block_h, dtype=np.int64) if info.tiled else np.minimum(info.block_h, info.height - y0)
+    tbl = np.stack([k, info.offsets, info.bytecounts[:n], y0, x0, rows], axis=1)[keep]
+    empty = tbl[tbl[:, 2] <= 0]
+    if len(empty):
+        raise GeoTiffError(f"{path}: block {int(empty[0, 0])} has no data (sparse files are not read)")
+    return tbl
+
+
+def _read_compressed_to_device(path, info, chunk_bytes):
+    """LZW / Deflate blocks -> DeviceRaster, bit for bit what ``dev.upload(read_array(path))`` gives.  The compressed
+    bytes of a batch of blocks (about ``chunk_bytes``) are pread on the I/O threads into one of two pinned staging
+    buffers and uploaded on a copy stream while the next batch is read; each batch is decoded on the current stream by
+    ``hd_tiff_decode``.  The per-block status words are read once at the end: a corrupt block raises GeoTiffError
+    naming it; a Deflate block that decodes to more than the block holds (legal: the surplus is ignored) is decoded
+    again on the host by ``_decode_block`` and uploaded into its place."""
+    import ctypes
+    import os
+    import torch
+    from . import _lib, device as dev
+    native = info.dtype.newbyteorder("=")
+    hd = dev.hd_dtype_of(native)
+    if info.predictor == 2 and info.dtype.kind == "f":
+        raise GeoTiffError("horizontal predictor on floating-point samples")
+    ny, nx = info.shape
+    bh, bw, es = info.block_h, info.block_w, native.itemsize
+    tbl = _block_table(path, info)
+    with open(path, "rb", buffering=0) as f:
+        fd = f.fileno()
+        size = os.fstat(fd).st_size
+        if len(tbl) and int((tbl[:, 1] + tbl[:, 2]).max()) > size:
+            raise GeoTiffError(f"{path}: truncated pixel data")
+        raster = dev.empty(ny, nx, hd, native)
+        if not len(tbl):
+            return raster
+        # batches: consecutive blocks up to chunk_bytes compressed (and 4 * chunk_bytes decoded), at least one block
+        slot = _lib.load().hd_tiff_decode_workspace_bytes(1, bh, bw, hd)
+        if slot <= 0:
+            raise GeoTiffError(f"{path}: blocks of {bh} x {bw} samples are too large")
+        starts, comp, dec = [0], 0, 0
+        for i, nb in enumerate(tbl[:, 2].tolist()):
+            if i > starts[-1] and (comp + nb > chunk_bytes or dec + slot > 4 * chunk_bytes):
+                starts.append(i)
+                comp = dec = 0
+            comp += nb
+            dec += slot
+        starts.append(len(tbl))
+        src_off = np.zeros(len(tbl), dtype=np.int64)            # offset of each block inside its batch
+        batch_bytes = []
+        for a, b in zip(starts[:-1], starts[1:]):
+            c = np.cumsum(tbl[a:b, 2])
+            src_off[a:b] = c - tbl[a:b, 2]
+            batch_bytes.append(int(c[-1]))
+        max_blocks = max(b - a for a, b in zip(starts[:-1], starts[1:]))
+        stage_bytes = max(batch_bytes)
+        lib = _lib.load()
+        device = dev.device()
+        dtbl = torch.from_numpy(np.ascontiguousarray(np.stack([src_off, tbl[:, 2], tbl[:, 3], tbl[:, 4], tbl[:, 5]], 1))
+                                ).to(device)
+        status = torch.zeros(len(tbl), dtype=torch.int32, device=device)
+        ws_bytes = lib.hd_tiff_decode_workspace_bytes(max_blocks, bh, bw, hd)
+        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=device)
+        host = [dev.pinned_empty((stage_bytes,), np.uint8) for _ in range(2)]
+        dsrc = [torch.empty(stage_bytes, dtype=torch.uint8, device=device) for _ in range(2)]
+        uploaded, decoded = [None, None], [None, None]
+        cur = torch.cuda.current_stream()
+        copy = torch.cuda.Stream()
+        copy.wait_stream(cur)
+
+        def read_batch(buf, a, b):
+            def one(i):
+                got = os.preadv(fd, [memoryview(buf)[src_off[i]:src_off[i] + tbl[i, 2]]], int(tbl[i, 1]))
+                if got < tbl[i, 2]:
+                    raise GeoTiffError(f"{path}: truncated pixel data")
+            if b - a > 1 and _io_threads() > 1:
+                list(_pool().map(one, range(a, b)))
+            else:
+                for i in range(a, b):
+                    one(i)
+
+        for j, (a, b) in enumerate(zip(starts[:-1], starts[1:])):
+            s = j & 1
+            if uploaded[s] is not None:
+                uploaded[s].synchronize()                       # the upload of batch j - 2 has left host[s]
+            read_batch(host[s], a, b)
+            with torch.cuda.stream(copy):
+                if decoded[s] is not None:
+                    copy.wait_event(decoded[s])                 # batch j - 2 is decoded: dsrc[s] is free
+                _lib.check(lib.hd_memcpy2d_h2d(ctypes.c_void_p(dsrc[s].data_ptr()), batch_bytes[j],
+                                               ctypes.c_void_p(host[s].ctypes.data), batch_bytes[j], batch_bytes[j], 1,
+                                               ctypes.c_void_p(copy.cuda_stream)))
+                uploaded[s] = torch.cuda.Event()
+                uploaded[s].record(copy)
+            cur.wait_event(uploaded[s])
+            _lib.check(lib.hd_tiff_decode(ctypes.c_void_p(dsrc[s].data_ptr()), batch_bytes[j],
+                                          ctypes.c_void_p(dtbl[a].data_ptr()), b - a, info.compression, info.predictor,
+                                          hd, int(info.dtype.byteorder == ">"), raster.ptr, raster.pitch, ny, nx, bh, bw,
+                                          ctypes.c_void_p(status[a].data_ptr()), ctypes.c_void_p(ws.data_ptr()), ws_bytes,
+                                          dev.stream_ptr()))
+            decoded[s] = torch.cuda.Event()
+            decoded[s].record(cur)
+        for d in dsrc:
+            d.record_stream(copy)
+        st = status.cpu().numpy()                               # the one synchronisation of the decode
+        for ev in uploaded:
+            if ev is not None:
+                ev.synchronize()                                # the staging buffers go out of scope
+        bad = np.flatnonzero(st == _DECODE_CORRUPT)
+        if len(bad):
+            raise GeoTiffError(f"{path}: corrupt compressed block {int(tbl[bad[0], 0])}")
+        for i in np.flatnonzero(st == _DECODE_HOST).tolist():
+            k, off, nb, y0, x0, rows = (int(v) for v in tbl[i])
+            try:
+                blk = _decode_block(os.pread(fd, nb, off), info, rows, bw)
+            except (zlib.error, ValueError) as e:
+                raise GeoTiffError(f"{path}: corrupt compressed block {k} ({e})") from None
+            ys, xs = min(bh, ny - y0), min(bw, nx - x0)
+            host_blk = np.ascontiguousarray(blk[:ys, :xs], dtype=native)
+            sub = raster.sub(y0, y0 + ys, x0, x0 + xs)
+            _lib.check(lib.hd_memcpy2d_h2d(sub.ptr, sub.pitch * es, ctypes.c_void_p(host_blk.ctypes.data), xs * es,
+                                           xs * es, ys, dev.stream_ptr()))
+            _lib.check(lib.hd_stream_synchronize(dev.stream_ptr()))     # host_blk is pageable
     return raster
 
 

@@ -89,6 +89,13 @@ int hd_host_widen_i16(void* dst, int dst_dtype, const int16_t* src, int64_t n, i
 /* HOST helper of the GeoTIFF reader (hydrodem_b200/geotiff.py): TIFF 6.0 LZW (MSB-first codes, 9..12 bits, early change).
  * Returns the number of bytes written to dst (at most cap) or a negative hd_status for a corrupt stream. */
 int64_t hd_host_lzw_decode(const uint8_t* src, int64_t nsrc, uint8_t* dst, int64_t cap);
+/* HOST entries of the GPU block decoder's core (csrc/tiffcodec.cuh), for tests: hd_host_inflate decodes a zlib stream
+ * (RFC 1950 header without preset dictionary, RFC 1951 blocks, Adler-32 verified, bytes after the stream ignored);
+ * hd_host_tiff_lzw decodes TIFF LZW exactly as hd_host_lzw_decode.  Both return the number of bytes written to dst or a
+ * negative hd_status: HD_ERR_ARG for a corrupt stream, and for hd_host_inflate HD_ERR_WORKSPACE when the stream decodes to
+ * more than cap bytes. */
+int64_t hd_host_inflate(const uint8_t* src, int64_t nsrc, uint8_t* dst, int64_t cap);
+int64_t hd_host_tiff_lzw(const uint8_t* src, int64_t nsrc, uint8_t* dst, int64_t cap);
 
 /* ---- elementwise filters (filters/simple_filters.py, extension_filters.py:12-130) -------------- */
 typedef enum {
@@ -445,6 +452,28 @@ int hd_rasterize_lines(const void* vx, const void* vy, int64_t n_vertices, const
                        int64_t n_parts, const void* values, int64_t n_features, void* dst, int64_t dst_pitch, int64_t dst_ny,
                        int64_t dst_nx, const double* dst_geo, int64_t dst_row0, const double* tm, void* workspace,
                        int64_t workspace_bytes, void* stream);
+
+/* ---- GeoTIFF block decode: geotiff.read_to_device of Deflate / LZW rasters (DESIGN §9d) ------------------------------ */
+/* DEVICE workspace bytes hd_tiff_decode needs: one 16-byte aligned slot of block_h * block_w samples per block (0 for
+ * invalid arguments, a block above 2 GB or more than 2^40 blocks). */
+int64_t hd_tiff_decode_workspace_bytes(int64_t n_blocks, int64_t block_h, int64_t block_w, int sample_dtype);
+/* Decode n_blocks compressed strips / tiles of one single-band TIFF into the pitched raster out (ny x nx, sample_dtype
+ * U8 / I16 / I32 / I64 / F32 / F64, pitch in elements), as geotiff.read_array decodes them on the host.  DEVICE inputs:
+ * src (src_bytes bytes of compressed data) and blocks = int64[n_blocks][5] (offset in src, byte count, y0, x0, rows): the
+ * block decodes to rows x block_w samples (rows <= block_h; strips: min(block_h, ny - y0), tiles: block_h) and its
+ * top-left sample is cell (y0, x0); what falls outside the raster is cropped.  compression 5 = TIFF LZW (short output is
+ * zero-padded, output beyond the block is dropped), 8 / 32946 = zlib Deflate (Adler-32 verified; output shorter than the
+ * block is corrupt).  predictor 1, 2 (horizontal, integer samples: a row-wise prefix sum modulo 2^bits after the byte
+ * swap) or 3 (floating point, TIFF TN3: byte-wise prefix sum per row, planes most significant first); big_endian: the
+ * file's byte order.  status = DEVICE int32[n_blocks], written per block: 0 decoded and stored, 1 corrupt (or a table
+ * entry outside src or the raster), 2 a legal Deflate stream longer than the block: not stored, the caller re-decodes it
+ * on the host.  One warp per block, persistent; no waiting between warps or CTAs.  Allocates nothing; asynchronous and
+ * capturable.  Bad codes, a predictor the sample type does not allow, empty rasters or blocks, pitch < nx -> HD_ERR_ARG;
+ * out or its row stride not 16-byte aligned -> HD_ERR_ALIGN; workspace below hd_tiff_decode_workspace_bytes ->
+ * HD_ERR_WORKSPACE; all before any device work. */
+int hd_tiff_decode(const void* src, int64_t src_bytes, const void* blocks, int64_t n_blocks, int compression, int predictor,
+                   int sample_dtype, int big_endian, void* out, int64_t out_pitch, int64_t ny, int64_t nx, int64_t block_h,
+                   int64_t block_w, void* status, void* workspace, int64_t workspace_bytes, void* stream);
 
 #ifdef __cplusplus
 }
